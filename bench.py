@@ -21,11 +21,16 @@ front-end over the rank's shard, chained per utterance as the reference's caller
 
 `--impl reference` times the reference front-end on all host cores instead (same config, bounded sample per step).
 `--workload mfcc` is the MFCC-only line of BASELINE configs[1] (4096 x 2 s, fused K1 kernel).
+`--dump-outputs DIR` writes what the last timed step returned as DIR/<name>.npy (DIR/rank<r>/ when N > 1), at most 64 MB over
+all ranks; the inputs are seeded, so two builds run with the same arguments can be compared output for output.  It covers the
+GPU workloads only: the reference arm's pool workers hand back no outputs, and returning them would change what it times.
 Launch: python bench.py [--gpus N --steps K --warmup W]; for N > 1 via torch.distributed.run (one rank per GPU).
 """
 import argparse
+import atexit
 import json
 import os
+import signal
 import subprocess
 import sys
 import tempfile
@@ -70,6 +75,56 @@ def peaks():
         with open(path) as f:
             return float(json.load(f)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
     return 6650.0, "fallback (B200_PROFILING.md)"
+
+
+DUMP_BYTES = 64 * 10**6            # all ranks together
+
+
+def dump_outputs(d, per_utt, ragged, budget):
+    """Writes the outputs of one call as d/<name>.npy: float32 stays float32, every other type becomes float64 (exact for
+    the int32 / int64 outputs).  `per_utt` maps a name to an output with one row per utterance; `ragged` maps the name of a
+    frame-offset output [U+1] to (those offsets as a NumPy array, {name: per-frame rows}).  When all of it does not fit in
+    `budget` bytes, a fixed seeded sample of utterances is written instead, the same utterances in every array, and each
+    offset array is rebuilt to index the rows written (what the call returns for those utterances alone).
+    d/utterances.npy lists the utterances written, in order."""
+    import torch
+    os.makedirs(d, exist_ok=True)
+    width = lambda t: int(np.prod(t.shape[1:])) * (4 if t.dtype == torch.float32 else 8)
+    n_utt = len(next(iter(ragged.values()))[0]) - 1
+    files = 1 + len(per_utt) + sum(1 + len(rows) for _, rows in ragged.values())
+    fixed = 1024 * files + 8 * len(ragged)                    # .npy headers, the leading zero of each offset array
+    cost = 8 + sum(width(t) for t in per_utt.values()) + sum(8 + np.diff(fo) * sum(width(r) for r in rows.values())
+                                                             for fo, rows in ragged.values())
+    keep = np.arange(n_utt)
+    if fixed + int(np.sum(cost)) > budget:
+        order = np.random.default_rng(0).permutation(n_utt)
+        keep = np.sort(order[: int(np.searchsorted(np.cumsum(cost[order]), budget - fixed, side="right"))])
+
+    written = []
+
+    def save(name, a):
+        path = os.path.join(d, name + ".npy")
+        np.save(path, np.ascontiguousarray(a, dtype=np.float32 if a.dtype == np.float32 else np.float64))
+        written.append(os.path.getsize(path))
+
+    save("utterances", keep)
+    sel = torch.from_numpy(keep)
+    for k, t in per_utt.items():
+        save(k, t[sel.to(t.device)].cpu().numpy())
+    for k, (fo, rows) in ragged.items():
+        n = np.diff(fo)[keep]
+        off = np.concatenate([[0], np.cumsum(n)])
+        save(k, off)
+        idx = torch.from_numpy(np.arange(off[-1], dtype=np.int64) + np.repeat(fo[keep] - off[:-1], n))
+        for name, r in rows.items():
+            save(name, r[idx.to(r.device)].cpu().numpy())
+    assert sum(written) <= budget, written
+
+
+def dump(args, rank, world, per_utt, ragged):
+    """--dump-outputs: rank r of N > 1 writes to DIR/rank<r>/, each with a 1/N share of DUMP_BYTES."""
+    d = args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}")
+    dump_outputs(d, per_utt, ragged, DUMP_BYTES // world)
 
 
 def recorded_traffic(kernel):
@@ -269,6 +324,7 @@ class ClockSampler:
         try:
             self.p = subprocess.Popen(["nvidia-smi", "-i", str(gpu_index), f"--query-gpu={self.Q}",
                                        "--format=csv,noheader,nounits", "-lms", "20"], stdout=self.f, stderr=subprocess.DEVNULL)
+            atexit.register(self.p.kill)         # the sampler must not outlive bench.py when a step fails before stop()
         except OSError:
             self.p = None
 
@@ -393,6 +449,8 @@ def run_frontend(args, rank, world, local_rank):
     ms_total = ev0.elapsed_time(ev1)
     launches = dspfe.launch_count() - n_launch0
     rows, fcep, facr = tot[0]
+    # the last timed step's outputs, copied on the device now and written after the clock sampling (later steps reuse `out`)
+    last = {k: v.clone() for k, v in out.items()} if args.dump_outputs else None
 
     # per-kernel device times of the same step: CUDA events on the launching stream around every kernel (3 steps, mean)
     acc = {}
@@ -404,6 +462,12 @@ def run_frontend(args, rank, world, local_rank):
                 acc.setdefault(path, {}).setdefault(k, []).append(v)
     kern = {path: {k: float(np.mean(v)) for k, v in ks.items()} for path, ks in acc.items()}
     clocks = sample_clocks_under(sampler, step, torch) if sampler else None
+    if last:
+        fo = {k: last[k].cpu().numpy() for k in ("mfcc_frame_off", "cep_frame_off", "acr_frame_off")}
+        dump(args, rank, world, {"lr": last["lr"], "cep_feat": last["cep_feat"]},
+             {"mfcc_frame_off": (fo["mfcc_frame_off"], {"mfcc": last["mfcc"][:rows]}),
+              "cep_frame_off": (fo["cep_frame_off"], {"cep_pitch": last["cep_pitch"][:fcep], "cep_lag": last["cep_lag"][:fcep]}),
+              "acr_frame_off": (fo["acr_frame_off"], {"acr_pitch": last["acr_pitch"][:facr], "acr_lag": last["acr_lag"][:facr]})})
 
     # end to end through the host-buffer call: pinned host PCM in, pinned host outputs back, every step
     h_pcm = torch.empty(total, dtype=torch.int16).pin_memory()
@@ -584,11 +648,14 @@ def run_mfcc(args, rank, world, local_rank):
     ev1.record()
     barrier()
     ms_total = ev0.elapsed_time(ev1)
+    last = (out[:rows].clone(), fo.clone()) if args.dump_outputs else None     # written after the clock sampling
     dspfe.timing_begin()
     for _ in range(args.steps):
         step()
     k_ms = float(np.median([ms for name, ms in dspfe.timing_end() if name == "mfcc_delta_kernel"]))
     clocks = sample_clocks_under(sampler, step, torch) if sampler else None
+    if last:
+        dump(args, rank, world, {}, {"mfcc_frame_off": (last[1].cpu().numpy(), {"mfcc": last[0]})})
     t = torch.tensor([ms_total, k_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -623,7 +690,14 @@ def main():
     ap.add_argument("--workload", default="frontend", choices=["frontend", "mfcc"],
                     help="frontend = the metric's workload (default); mfcc = the MFCC-only line of BASELINE configs[1]")
     ap.add_argument("--utterances", type=int, default=UTT_PER_GPU, help="utterances per GPU of the frontend workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    # SIGTERM (torch.distributed.run stopping the ranks when one fails) leaves through sys.exit, so the atexit hooks run
+    signal.signal(signal.SIGTERM, lambda *_: sys.exit(128 + signal.SIGTERM))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm keeps no outputs")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
