@@ -119,46 +119,28 @@ MfccConfig to_config(const dspfe_mfcc_params& q) {
 
 // Per-stream scratch for one in-flight batch.
 struct Workspace {
-    int64_t cap_utt = 0, cap_tiles = 0, cap_cep = 0;
-    float* cep = nullptr;       // K1L: static cepstra [rows, numcep] between the two kernels
-    int ensure_cep(int64_t floats) {
-        if (floats > cap_cep) { cudaFree(cep); cep = nullptr; cap_cep = 0; CUDA_TRY(cudaMalloc(&cep, floats * sizeof(float))); cap_cep = floats; }
-        return DSPFE_OK;
-    }
-    int64_t* seg_start = nullptr; int32_t* seg_len = nullptr; int64_t* frame_off = nullptr;
-    int32_t* tile_off = nullptr; Tile* tiles = nullptr; int32_t* ntiles = nullptr;
+    DeviceArray<float> cep;     // K1L: static cepstra [rows, numcep] between the two kernels
+    DeviceArray<int64_t> seg_start; DeviceArray<int32_t> seg_len; DeviceArray<int64_t> frame_off;
+    DeviceArray<int32_t> tile_off; DeviceArray<Tile> tiles; DeviceArray<int32_t> ntiles;
     int ensure(int64_t n_utt, int64_t n_tiles) {
-        if (n_utt > cap_utt) {
-            cudaFree(seg_start); cudaFree(seg_len); cudaFree(frame_off); cudaFree(tile_off);
-            seg_start = nullptr; seg_len = nullptr; frame_off = nullptr; tile_off = nullptr; cap_utt = 0;
-            CUDA_TRY(cudaMalloc(&seg_start, (n_utt + 1) * sizeof(int64_t)));
-            CUDA_TRY(cudaMalloc(&seg_len, (n_utt + 1) * sizeof(int32_t)));
-            CUDA_TRY(cudaMalloc(&frame_off, (n_utt + 1) * sizeof(int64_t)));
-            CUDA_TRY(cudaMalloc(&tile_off, (n_utt + 1) * sizeof(int32_t)));
-            cap_utt = n_utt;
-        }
-        if (n_tiles > cap_tiles) {
-            cudaFree(tiles); tiles = nullptr; cap_tiles = 0;
-            CUDA_TRY(cudaMalloc(&tiles, n_tiles * sizeof(Tile)));
-            cap_tiles = n_tiles;
-        }
-        if (!ntiles) CUDA_TRY(cudaMalloc(&ntiles, sizeof(int32_t)));
-        return DSPFE_OK;
-    }
-    void release() {
-        cudaFree(seg_start); cudaFree(seg_len); cudaFree(frame_off); cudaFree(tile_off); cudaFree(tiles); cudaFree(ntiles); cudaFree(cep);
-        *this = Workspace();
+        int rc = seg_start.reserve(n_utt + 1);
+        if (!rc) rc = seg_len.reserve(n_utt + 1);
+        if (!rc) rc = frame_off.reserve(n_utt + 1);
+        if (!rc) rc = tile_off.reserve(n_utt + 1);
+        if (!rc) rc = tiles.reserve(n_tiles);
+        if (!rc) rc = ntiles.reserve(1);
+        return rc;
     }
 };
 
 constexpr int kSlots = 3;
 struct HostSlot {
-    cudaStream_t stream = nullptr;
+    Stream stream;
     Workspace ws;
-    int16_t* d_pcm = nullptr; int64_t cap_samples = 0;
-    int64_t* d_off = nullptr; int64_t* h_off = nullptr; int64_t cap_utt = 0;  // h_off pinned
-    float* d_out = nullptr; int64_t cap_rows = 0;
-    int64_t* d_frame_off = nullptr;
+    DeviceArray<int16_t> d_pcm;
+    DeviceArray<int64_t> d_off; PinnedArray<int64_t> h_off;
+    DeviceArray<float> d_out;
+    DeviceArray<int64_t> d_frame_off;
 };
 
 }  // namespace
@@ -167,14 +149,14 @@ struct dspfe_plan {
     MfccConfig cfg;
     MfccParams layout;          // scalars + offsets filled by build_mfcc_tables; pointers filled per call
     MfccParams layout_f32;      // same for float32 input samples (larger raw staging area)
-    float* d_tables = nullptr;
+    DeviceArray<float> d_tables;
     bool has_win = false;
     mfcc_kernel_t kernel = nullptr, kernel_f32 = nullptr, kernel_fbank = nullptr, kernel_spec = nullptr;
     Workspace ws;
     HostSlot slots[kSlots];
     int width = 0;              // 3 * numcep
     bool is_long = false;       // K1L: nfft other than 512, or nfft = 512 with an odd hop
-    float* d_long_tab = nullptr;
+    DeviceArray<float> d_long_tab;
     std::vector<float> h_long_tab;   // host copy: the mel edges travel as kernel parameters
 };
 
@@ -189,18 +171,18 @@ int launch_mfcc(dspfe_plan* pl, Workspace& ws, const void* d_pcm, bool f32, int6
     PrepParams pp;
     pp.offsets = d_offsets; pp.trim = d_trim; pp.n_utt = n_utt;
     pp.frame_len = pl->cfg.count_len; pp.frame_step = pl->cfg.frame_step; pp.seg_frames = pl->cfg.seg_frames;
-    pp.seg_start = ws.seg_start; pp.seg_len = ws.seg_len; pp.frame_off = d_frame_off ? d_frame_off : ws.frame_off;
-    pp.tile_off = ws.tile_off; pp.tiles = ws.tiles; pp.ntiles = ws.ntiles; pp.max_tiles = (int)max_tiles;
+    pp.seg_start = ws.seg_start.get(); pp.seg_len = ws.seg_len.get(); pp.frame_off = d_frame_off ? d_frame_off : ws.frame_off.get();
+    pp.tile_off = ws.tile_off.get(); pp.tiles = ws.tiles.get(); pp.ntiles = ws.ntiles.get(); pp.max_tiles = (int)max_tiles;
     prep_kernel<<<1, kPrepThreads, 0, st>>>(pp);
     LAUNCH_CHECK("prep_kernel", st);
 
-    if (pl->is_long || (mode != 0 && pl->d_long_tab)) {
+    if (pl->is_long || (mode != 0 && pl->d_long_tab.get())) {
         const int64_t rows = dspfe_rows_bound(pl, total_samples, n_utt);
-        if (mode == 0) { rc = ws.ensure_cep(rows * pl->cfg.numcep); if (rc) return rc; }
+        if (mode == 0) { rc = ws.cep.reserve(rows * pl->cfg.numcep); if (rc) return rc; }
         MfccLongParams lp;
-        lp.pcm = d_pcm; lp.in_f32 = f32 ? 1 : 0; lp.seg_start = ws.seg_start; lp.seg_len = ws.seg_len; lp.frame_off = pp.frame_off; lp.n_utt = n_utt;
+        lp.pcm = d_pcm; lp.in_f32 = f32 ? 1 : 0; lp.seg_start = ws.seg_start.get(); lp.seg_len = ws.seg_len.get(); lp.frame_off = pp.frame_off; lp.n_utt = n_utt;
         lp.frame_len = pl->cfg.frame_len; lp.frame_step = pl->cfg.frame_step; lp.nfilt = pl->cfg.nfilt; lp.numcep = pl->cfg.numcep;
-        lp.append_energy = pl->cfg.append_energy; lp.preemph = (float)pl->cfg.preemph; lp.tab = pl->d_long_tab; lp.mfcc = mode == 0 ? ws.cep : d_out; lp.max_frames = rows;
+        lp.append_energy = pl->cfg.append_energy; lp.preemph = (float)pl->cfg.preemph; lp.tab = pl->d_long_tab.get(); lp.mfcc = mode == 0 ? ws.cep.get() : d_out; lp.max_frames = rows;
         long_fill_size_params(lp, pl->cfg.nfft, mode, spec_kind);
         long_fill_mel_params(lp, pl->h_long_tab.data());
         const unsigned lgrid = (unsigned)((rows + 2 * kLongWarps - 1) / (2 * kLongWarps));
@@ -209,14 +191,14 @@ int launch_mfcc(dspfe_plan* pl, Workspace& ws, const void* d_pcm, bool f32, int6
         LAUNCH_CHECK("mfcc_long_kernel", st);
         if (mode != 0) return DSPFE_OK;
         int den = 0; for (int i = 1; i <= pl->cfg.delta_n; ++i) den += i * i;
-        delta_batch_kernel<<<(unsigned)n_utt, 128, 0, st>>>(ws.cep, pp.frame_off, n_utt, pl->cfg.numcep, pl->cfg.delta_n,
+        delta_batch_kernel<<<(unsigned)n_utt, 128, 0, st>>>(ws.cep.get(), pp.frame_off, n_utt, pl->cfg.numcep, pl->cfg.delta_n,
                                                                                           (float)(1.0 / (2.0 * den)), rows, d_out);
         LAUNCH_CHECK("delta_batch_kernel", st);
         return DSPFE_OK;
     }
     MfccParams mp = f32 ? pl->layout_f32 : pl->layout;
-    mp.pcm = d_pcm; mp.total_samples = total_samples; mp.seg_start = ws.seg_start; mp.seg_len = ws.seg_len;
-    mp.frame_off = pp.frame_off; mp.tiles = ws.tiles; mp.ntiles = ws.ntiles; mp.tables = pl->d_tables; mp.out = d_out;
+    mp.pcm = d_pcm; mp.total_samples = total_samples; mp.seg_start = ws.seg_start.get(); mp.seg_len = ws.seg_len.get();
+    mp.frame_off = pp.frame_off; mp.tiles = ws.tiles.get(); mp.ntiles = ws.ntiles.get(); mp.tables = pl->d_tables.get(); mp.out = d_out;
     mp.spec_kind = spec_kind;
     mfcc_kernel_t kern = mode == 1 ? pl->kernel_fbank : mode == 2 ? pl->kernel_spec : (f32 ? pl->kernel_f32 : pl->kernel);
     kern<<<(unsigned)max_tiles, kMfccThreads, mp.sm_total, st>>>(mp);
@@ -283,23 +265,23 @@ int dspfe_plan_create(const dspfe_mfcc_params* p, dspfe_plan** plan) {
         pl->is_long = !tiled; pl->has_win = !pl->cfg.window.empty(); pl->width = 3 * pl->cfg.numcep;
         const std::vector<float> t = build_long_tables(pl->cfg);
         pl->h_long_tab = t;
-        cudaError_t e = cudaMalloc(&pl->d_long_tab, t.size() * sizeof(float));
-        if (e == cudaSuccess) e = cudaMemcpy(pl->d_long_tab, t.data(), t.size() * sizeof(float), cudaMemcpyHostToDevice);
+        if (int rc = pl->d_long_tab.reserve(t.size())) { delete pl; return rc; }
+        cudaError_t e = cudaMemcpy(pl->d_long_tab.get(), t.data(), t.size() * sizeof(float), cudaMemcpyHostToDevice);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(mfcc_long_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, long_cta_smem(kLongMaxNfft));
         if (e == cudaSuccess) e = cudaFuncSetAttribute(mfcc_long_kernel<kLongNfft>, cudaFuncAttributeMaxDynamicSharedMemorySize, long_cta_smem(kLongNfft));
-        if (e != cudaSuccess) { cudaFree(pl->d_long_tab); delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
+        if (e != cudaSuccess) { delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
         if (!tiled) { *plan = pl; return DSPFE_OK; }
     }
     std::vector<float> blob = build_mfcc_tables(pl->cfg, pl->layout, err);
     if (err.empty()) { std::memset(&pl->layout_f32, 0, sizeof(pl->layout_f32)); build_mfcc_tables(pl->cfg, pl->layout_f32, err, true); }
-    if (!err.empty() && pl->d_long_tab) {   // e.g. a chunk of 16 long frames with a long hop does not fit shared memory: the general kernel takes it
+    if (!err.empty() && pl->d_long_tab.get()) {   // e.g. a chunk of 16 long frames with a long hop does not fit shared memory: the general kernel takes it
         pl->is_long = true; *plan = pl; return DSPFE_OK;
     }
     if (!err.empty()) { delete pl; return fail(DSPFE_ERR_UNSUPPORTED, err); }
     pl->has_win = !pl->cfg.window.empty();
     pl->width = 3 * pl->cfg.numcep;
-    cudaError_t e = cudaMalloc(&pl->d_tables, blob.size() * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(pl->d_tables, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice);
+    if (int rc = pl->d_tables.reserve(blob.size())) { delete pl; return rc; }
+    cudaError_t e = cudaMemcpy(pl->d_tables.get(), blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice);
     const bool tri = pl->cfg.nfft == kTriNfft;
     pl->kernel = tri ? pick_tri_kernel(pl->has_win, pl->cfg.frame_len, false) : pick_kernel(pl->has_win, pl->cfg.frame_len, false);
     pl->kernel_f32 = tri ? pick_tri_kernel(pl->has_win, pl->cfg.frame_len, true) : pick_kernel(pl->has_win, pl->cfg.frame_len, true);
@@ -311,7 +293,7 @@ int dspfe_plan_create(const dspfe_mfcc_params* p, dspfe_plan** plan) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(pl->kernel_fbank, cudaFuncAttributeMaxDynamicSharedMemorySize, pl->layout_f32.sm_total);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(pl->kernel_spec, cudaFuncAttributeMaxDynamicSharedMemorySize, pl->layout_f32.sm_total);
     }
-    if (e != cudaSuccess) { cudaFree(pl->d_tables); delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
+    if (e != cudaSuccess) { delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
     *plan = pl;
     return DSPFE_OK;
 }
@@ -323,14 +305,6 @@ int dspfe_plan_reserve(dspfe_plan* pl, int64_t max_utt, int64_t max_total_sample
 
 void dspfe_plan_destroy(dspfe_plan* pl) {
     if (!pl) return;
-    pl->ws.release();
-    for (auto& s : pl->slots) {
-        s.ws.release();
-        cudaFree(s.d_pcm); cudaFree(s.d_off); cudaFree(s.d_out); cudaFree(s.d_frame_off);
-        if (s.h_off) cudaFreeHost(s.h_off);
-        if (s.stream) cudaStreamDestroy(s.stream);
-    }
-    cudaFree(pl->d_tables); cudaFree(pl->d_long_tab);
     delete pl;
 }
 
@@ -429,45 +403,30 @@ int dspfe_mfcc_delta_host(dspfe_plan* pl, const int16_t* h_pcm, const int64_t* h
         }
         const int32_t nu = u_end - u;
         HostSlot& s = pl->slots[slab % kSlots];
-        if (!s.stream) CUDA_TRY(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-        CUDA_TRY(cudaStreamSynchronize(s.stream));  // the slot's previous slab has fully drained
-        if (samples + 8 > s.cap_samples) {
-            cudaFree(s.d_pcm); s.d_pcm = nullptr; s.cap_samples = 0;
-            const int64_t cap = std::max<int64_t>(samples + 8, kSlabSamples + 8);
-            CUDA_TRY(cudaMalloc(&s.d_pcm, cap * sizeof(int16_t)));
-            s.cap_samples = cap;
-        }
-        if (nu + 1 > s.cap_utt) {
-            cudaFree(s.d_off); cudaFree(s.d_frame_off); if (s.h_off) cudaFreeHost(s.h_off);
-            s.d_off = nullptr; s.d_frame_off = nullptr; s.h_off = nullptr; s.cap_utt = 0;
-            const int64_t cap = std::max<int64_t>(nu + 1, 4096);
-            CUDA_TRY(cudaMalloc(&s.d_off, cap * sizeof(int64_t)));
-            CUDA_TRY(cudaMalloc(&s.d_frame_off, cap * sizeof(int64_t)));
-            CUDA_TRY(cudaHostAlloc(&s.h_off, cap * sizeof(int64_t), cudaHostAllocDefault));
-            s.cap_utt = cap;
-        }
-        const int64_t rows_bound = dspfe_rows_bound(pl, samples, nu);
-        if (rows_bound > s.cap_rows) {
-            cudaFree(s.d_out); s.d_out = nullptr; s.cap_rows = 0;
-            const int64_t cap = std::max<int64_t>(rows_bound, kSlabSamples / fstep + 4096);
-            CUDA_TRY(cudaMalloc(&s.d_out, cap * width * sizeof(float)));
-            s.cap_rows = cap;
-        }
-        const int64_t base = h_offsets[u];
-        for (int32_t i = 0; i <= nu; ++i) s.h_off[i] = h_offsets[u + i] - base;
-        if (samples > 0)
-            CUDA_TRY(cudaMemcpyAsync(s.d_pcm, h_pcm + base, samples * sizeof(int16_t), cudaMemcpyHostToDevice, s.stream));
-        CUDA_TRY(cudaMemcpyAsync(s.d_off, s.h_off, (nu + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s.stream));
-        int rc = launch_mfcc(pl, s.ws, s.d_pcm, false, samples, s.d_off, nullptr, nu, s.d_out, s.d_frame_off, s.stream);
+        CUDA_TRY(s.stream.ensure());
+        const cudaStream_t st = s.stream.get();
+        CUDA_TRY(cudaStreamSynchronize(st));  // the slot's previous slab has fully drained
+        int rc = s.d_pcm.reserve(samples + 8, kSlabSamples + 8);
+        if (!rc) rc = s.d_off.reserve(nu + 1, 4096);
+        if (!rc) rc = s.d_frame_off.reserve(nu + 1, 4096);
+        if (!rc) rc = s.h_off.reserve(nu + 1, 4096);
+        if (!rc) rc = s.d_out.reserve(dspfe_rows_bound(pl, samples, nu) * width, (kSlabSamples / fstep + 4096) * width);
         if (rc) return rc;
-        CUDA_TRY(cudaMemcpyAsync(h_out + row * width, s.d_out, rows * width * sizeof(float), cudaMemcpyDeviceToHost, s.stream));
+        const int64_t base = h_offsets[u];
+        for (int32_t i = 0; i <= nu; ++i) s.h_off.get()[i] = h_offsets[u + i] - base;
+        if (samples > 0)
+            CUDA_TRY(cudaMemcpyAsync(s.d_pcm.get(), h_pcm + base, samples * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(s.d_off.get(), s.h_off.get(), (nu + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        rc = launch_mfcc(pl, s.ws, s.d_pcm.get(), false, samples, s.d_off.get(), nullptr, nu, s.d_out.get(), s.d_frame_off.get(), st);
+        if (rc) return rc;
+        CUDA_TRY(cudaMemcpyAsync(h_out + row * width, s.d_out.get(), rows * width * sizeof(float), cudaMemcpyDeviceToHost, st));
         row += rows;
         u = u_end;
         ++slab;
     }
     if (h_frame_off) h_frame_off[n_utt] = row;
     for (auto& s : pl->slots)
-        if (s.stream) CUDA_TRY(cudaStreamSynchronize(s.stream));
+        if (s.stream.get()) CUDA_TRY(cudaStreamSynchronize(s.stream.get()));
     return DSPFE_OK;
 }
 

@@ -12,14 +12,13 @@ struct dspfe_endpoint_plan {
     dspfe_endpoint_params prm;
     EpRule rule;
     int frame_len, frame_step, q, rem;
+    Stream stream;              // host path
     // workspaces
-    int64_t cap_utt = 0, cap_blocks = 0, cap_frames = 0;
-    int64_t *frame_off = nullptr, *block_off = nullptr; int32_t* order = nullptr;
-    int32_t *blk = nullptr, *asum = nullptr, *zcr = nullptr;
+    DeviceArray<int64_t> frame_off, block_off; DeviceArray<int32_t> order;
+    DeviceArray<int32_t> blk, asum, zcr;
     // host-path staging
-    cudaStream_t stream = nullptr;
-    int16_t* d_pcm = nullptr; int64_t cap_samples = 0;
-    int64_t* d_off = nullptr; int32_t* d_lr = nullptr; int64_t cap_hutt = 0;
+    DeviceArray<int16_t> d_pcm;
+    DeviceArray<int64_t> d_off; DeviceArray<int32_t> d_lr;
 };
 
 namespace {
@@ -38,25 +37,13 @@ int fill_rule(const dspfe_endpoint_params& q, EpRule& r, int& frame_len, int& fr
 }
 
 int ensure(dspfe_endpoint_plan* pl, int64_t n_utt, int64_t blocks, int64_t frames) {
-    if (n_utt + 1 > pl->cap_utt) {
-        cudaFree(pl->frame_off); cudaFree(pl->block_off); cudaFree(pl->order); pl->frame_off = pl->block_off = nullptr; pl->order = nullptr; pl->cap_utt = 0;
-        CUDA_TRY(cudaMalloc(&pl->frame_off, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->order, (n_utt + 1) * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->block_off, (n_utt + 1) * sizeof(int64_t)));
-        pl->cap_utt = n_utt + 1;
-    }
-    if (blocks > pl->cap_blocks) {
-        cudaFree(pl->blk); pl->blk = nullptr; pl->cap_blocks = 0;
-        CUDA_TRY(cudaMalloc(&pl->blk, blocks * 6 * sizeof(int32_t)));
-        pl->cap_blocks = blocks;
-    }
-    if (frames > pl->cap_frames) {
-        cudaFree(pl->asum); cudaFree(pl->zcr); pl->asum = pl->zcr = nullptr; pl->cap_frames = 0;
-        CUDA_TRY(cudaMalloc(&pl->asum, frames * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->zcr, frames * sizeof(int32_t)));
-        pl->cap_frames = frames;
-    }
-    return DSPFE_OK;
+    int rc = pl->frame_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->order.reserve(n_utt + 1);
+    if (!rc) rc = pl->block_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->blk.reserve(blocks * 6);
+    if (!rc) rc = pl->asum.reserve(frames);
+    if (!rc) rc = pl->zcr.reserve(frames);
+    return rc;
 }
 
 }  // namespace
@@ -142,9 +129,6 @@ int dspfe_endpoint_create(const dspfe_endpoint_params* p, dspfe_endpoint_plan** 
 
 void dspfe_endpoint_destroy(dspfe_endpoint_plan* pl) {
     if (!pl) return;
-    cudaFree(pl->frame_off); cudaFree(pl->block_off); cudaFree(pl->order); cudaFree(pl->blk); cudaFree(pl->asum); cudaFree(pl->zcr);
-    cudaFree(pl->d_pcm); cudaFree(pl->d_off); cudaFree(pl->d_lr);
-    if (pl->stream) cudaStreamDestroy(pl->stream);
     delete pl;
 }
 
@@ -178,9 +162,9 @@ int dspfe_endpoint(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t total_
     cudaStream_t st = (cudaStream_t)stream;
     EpParams p;
     p.pcm = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = d_frame_off ? d_frame_off : pl->frame_off; p.block_off = pl->block_off;
-    p.blk = pl->blk; p.asum = d_asum ? d_asum : pl->asum; p.zcr = d_zcr ? d_zcr : pl->zcr; p.lr = d_lr;
-    p.max_blocks = blocks_bound; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order;
+    p.q = pl->q; p.rem = pl->rem; p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.block_off = pl->block_off.get();
+    p.blk = pl->blk.get(); p.asum = d_asum ? d_asum : pl->asum.get(); p.zcr = d_zcr ? d_zcr : pl->zcr.get(); p.lr = d_lr;
+    p.max_blocks = blocks_bound; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order.get();
     ep_prep_kernel<<<1, kEpPrepThreads, 0, st>>>(p);
     LAUNCH_CHECK("ep_prep_kernel", st);
     ep_block_kernel<<<(unsigned)((blocks_bound + 127) / 128), 128, 0, st>>>(p);
@@ -205,8 +189,9 @@ int dspfe_endpoint_robust(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t
     const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
     EpParams p;
     p.pcm = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off; p.block_off = pl->block_off; p.blk = pl->blk; p.asum = pl->asum; p.zcr = pl->zcr;
-    p.lr = d_lr; p.max_blocks = 0; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order;
+    p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off.get(); p.block_off = pl->block_off.get(); p.blk = pl->blk.get();
+    p.asum = pl->asum.get(); p.zcr = pl->zcr.get(); p.lr = d_lr; p.max_blocks = 0; p.max_frames = frames_bound; p.rule = pl->rule;
+    p.order = pl->order.get();
     CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
     CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     ep_decide_robust_kernel<<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
@@ -221,10 +206,11 @@ int dspfe_endpoint_robust_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, co
     int rc = dspfe_endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, nullptr, nullptr, nullptr);
     if (rc) return rc;
     const int64_t total = h_offsets[n_utt] - h_offsets[0];
-    rc = dspfe_endpoint_robust(pl, pl->d_pcm, total, pl->d_off, n_utt, pl->d_lr, pl->stream);
+    const cudaStream_t st = pl->stream.get();
+    rc = dspfe_endpoint_robust(pl, pl->d_pcm.get(), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
     if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr, (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, pl->stream));
-    CUDA_TRY(cudaStreamSynchronize(pl->stream));
+    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     return DSPFE_OK;
 }
 
@@ -234,18 +220,11 @@ int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int
     if (n_utt == 0) return DSPFE_OK;
     const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
     if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-    if (!pl->stream) CUDA_TRY(cudaStreamCreateWithFlags(&pl->stream, cudaStreamNonBlocking));
-    if (total + 8 > pl->cap_samples) {
-        cudaFree(pl->d_pcm); pl->d_pcm = nullptr; pl->cap_samples = 0;
-        CUDA_TRY(cudaMalloc(&pl->d_pcm, (total + 8) * sizeof(int16_t)));
-        pl->cap_samples = total + 8;
-    }
-    if (n_utt + 1 > pl->cap_hutt) {
-        cudaFree(pl->d_off); cudaFree(pl->d_lr); pl->d_off = nullptr; pl->d_lr = nullptr; pl->cap_hutt = 0;
-        CUDA_TRY(cudaMalloc(&pl->d_off, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->d_lr, (int64_t)n_utt * 2 * sizeof(int32_t)));
-        pl->cap_hutt = n_utt + 1;
-    }
+    CUDA_TRY(pl->stream.ensure());
+    int rc = pl->d_pcm.reserve(total + 8);
+    if (!rc) rc = pl->d_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->d_lr.reserve((int64_t)n_utt * 2);
+    if (rc) return rc;
     std::vector<int64_t> rel(n_utt + 1);
     int64_t frames = 0;
     for (int32_t u = 0; u <= n_utt; ++u) {
@@ -256,14 +235,14 @@ int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int
         }
     }
     if (h_frame_off) h_frame_off[n_utt] = frames;
-    cudaStream_t st = pl->stream;
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm, h_pcm + base, total * sizeof(int16_t), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(pl->d_off, rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    int rc = dspfe_endpoint(pl, pl->d_pcm, total, pl->d_off, n_utt, pl->d_lr, nullptr, nullptr, nullptr, 0, st);
+    cudaStream_t st = pl->stream.get();
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), h_pcm + base, total * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    rc = dspfe_endpoint(pl, pl->d_pcm.get(), total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
     if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr, (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (h_asum) CUDA_TRY(cudaMemcpyAsync(h_asum, pl->asum, frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (h_zcr) CUDA_TRY(cudaMemcpyAsync(h_zcr, pl->zcr, frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (h_asum) CUDA_TRY(cudaMemcpyAsync(h_asum, pl->asum.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (h_zcr) CUDA_TRY(cudaMemcpyAsync(h_zcr, pl->zcr.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return DSPFE_OK;
 }

@@ -6,6 +6,7 @@
 // only queues kernels and copies.
 #include <algorithm>
 #include <cstring>
+#include <memory>
 #include <vector>
 
 #include "abi_common.h"
@@ -42,65 +43,50 @@ __global__ void fe_finish_kernel(const FeFinish f) {
 }
 
 struct FeSlot {
-    int16_t* d_pcm = nullptr; int64_t cap_samples = 0;
-    int64_t* d_rel = nullptr; int64_t* h_rel = nullptr; int64_t cap_utt = 0;
-    int32_t* d_lr = nullptr; double* d_feat = nullptr; int64_t* d_goff[3] = {nullptr, nullptr, nullptr};
-    float* d_mfcc = nullptr; int64_t cap_rows = 0;
-    double* d_cep = nullptr; int64_t cap_cep = 0;
-    double* d_acr = nullptr; int64_t cap_acr = 0;
-    int32_t* d_cep_lag = nullptr; int64_t cap_cep_lag = 0;
-    int32_t* d_acr_lag = nullptr; int64_t cap_acr_lag = 0;
-    cudaEvent_t h2d_done = nullptr, compute_done = nullptr, d2h_done = nullptr;
+    Event h2d_done, compute_done, d2h_done;
+    DeviceArray<int16_t> d_pcm;
+    DeviceArray<int64_t> d_rel; PinnedArray<int64_t> h_rel;
+    DeviceArray<int32_t> d_lr; DeviceArray<double> d_feat; DeviceArray<int64_t> d_goff[3];
+    DeviceArray<float> d_mfcc;
+    DeviceArray<double> d_cep, d_acr;
+    DeviceArray<int32_t> d_cep_lag, d_acr_lag;
 };
+
+struct SubPlanDelete {
+    void operator()(dspfe_endpoint_plan* p) const { dspfe_endpoint_destroy(p); }
+    void operator()(dspfe_plan* p) const { dspfe_plan_destroy(p); }
+    void operator()(dspfe_pitch_plan* p) const { dspfe_pitch_destroy(p); }
+};
+template <class P> using SubPlan = std::unique_ptr<P, SubPlanDelete>;
 
 }  // namespace
 
 struct FeLane {                       // one slab in flight: the four sub-plans own the workspaces of their kernels
-    dspfe_endpoint_plan* ep = nullptr; dspfe_plan* mf = nullptr; dspfe_pitch_plan* cep = nullptr; dspfe_pitch_plan* acr = nullptr;
-    int64_t* loc_off[3] = {nullptr, nullptr, nullptr}; int64_t cap_utt = 0;      // slab-local row / frame prefix sums
-    int64_t* d_tot = nullptr;                                                    // [3] the slab's totals
-    cudaStream_t stream = nullptr;                                               // host path only
-    cudaEvent_t finish_done = nullptr;
+    Stream stream;                                                               // host path only
+    Event finish_done;
     // the two pitch chains of a slab run beside its MFCC kernels (they only share the endpoints): side streams, fork / join events
-    cudaStream_t side[2] = {nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_join[2] = {nullptr, nullptr};
+    Stream side[2];
+    Event ev_fork, ev_join[2];
+    DeviceArray<int64_t> loc_off[3];                                             // slab-local row / frame prefix sums
+    DeviceArray<int64_t> d_tot;                                                  // [3] the slab's totals
+    SubPlan<dspfe_endpoint_plan> ep; SubPlan<dspfe_plan> mf; SubPlan<dspfe_pitch_plan> cep, acr;
 };
 
 struct dspfe_frontend_plan {
     dspfe_frontend_params prm;
+    Stream s_copy, s_out;
     FeLane lanes[kFeLanes];               // the device path uses lane 0 on the caller's stream
-    int64_t* rel_off = nullptr; int64_t cap_rel = 0;
-    int64_t* d_base = nullptr;            // [2][3] device-side running bases of the host path (ping-pong between consecutive slabs)
-    int64_t* h_tot = nullptr;             // pinned [kFeSlots][3]
-    // scratch for outputs the caller does not want
-    int32_t* s_lr = nullptr; int64_t cap_slr = 0;
-    float* s_mfcc = nullptr; int64_t cap_smfcc = 0;
-    double* s_cep = nullptr; int64_t cap_scep = 0;
-    double* s_acr = nullptr; int64_t cap_sacr = 0;
     FeSlot slots[kFeSlots];
-    cudaStream_t s_copy = nullptr, s_out = nullptr;
+    DeviceArray<int64_t> rel_off;
+    DeviceArray<int64_t> d_base;          // [2][3] device-side running bases of the host path (ping-pong between consecutive slabs)
+    PinnedArray<int64_t> h_tot;           // [kFeSlots][3]
+    // scratch for outputs the caller does not want
+    DeviceArray<int32_t> s_lr;
+    DeviceArray<float> s_mfcc;
+    DeviceArray<double> s_cep, s_acr;
 };
 
 namespace {
-
-template <class T>
-int grow(T*& p, int64_t& cap, int64_t need, int64_t floor_elems = 0) {
-    if (need <= cap) return DSPFE_OK;
-    cudaFree(p); p = nullptr; cap = 0;
-    const int64_t n = std::max(need, floor_elems);
-    CUDA_TRY(cudaMalloc(&p, n * sizeof(T)));
-    cap = n;
-    return DSPFE_OK;
-}
-
-int ensure_utt(FeLane& ln, int64_t n) {
-    if (n <= ln.cap_utt) return DSPFE_OK;
-    for (auto& q : ln.loc_off) { cudaFree(q); q = nullptr; }
-    ln.cap_utt = 0;
-    for (auto& q : ln.loc_off) CUDA_TRY(cudaMalloc(&q, n * sizeof(int64_t)));
-    ln.cap_utt = n;
-    return DSPFE_OK;
-}
 
 int create_lane(FeLane& ln, const dspfe_frontend_params& q) {
     dspfe_endpoint_params eq; dspfe_endpoint_params_default(&eq, q.samplerate);
@@ -111,11 +97,13 @@ int create_lane(FeLane& ln, const dspfe_frontend_params& q) {
     cq.samplerate = q.samplerate; cq.preemph = q.cep_preemph;
     dspfe_pitch_params aq; dspfe_pitch_params_default(&aq, 1);
     aq.samplerate = q.samplerate; aq.frame_len = q.acr_frame_len;
-    int rc = dspfe_endpoint_create(&eq, &ln.ep);
-    if (!rc) rc = dspfe_plan_create(&mq, &ln.mf);
-    if (!rc) rc = dspfe_pitch_create(&cq, &ln.cep);
-    if (!rc) rc = dspfe_pitch_create(&aq, &ln.acr);
-    if (!rc && cudaMalloc(&ln.d_tot, 3 * sizeof(int64_t)) != cudaSuccess) rc = fail(DSPFE_ERR_CUDA, "cudaMalloc failed");
+    dspfe_endpoint_plan* ep = nullptr; dspfe_plan* mf = nullptr; dspfe_pitch_plan *cep = nullptr, *acr = nullptr;
+    int rc = dspfe_endpoint_create(&eq, &ep);
+    if (!rc) rc = dspfe_plan_create(&mq, &mf);
+    if (!rc) rc = dspfe_pitch_create(&cq, &cep);
+    if (!rc) rc = dspfe_pitch_create(&aq, &acr);
+    ln.ep.reset(ep); ln.mf.reset(mf); ln.cep.reset(cep); ln.acr.reset(acr);
+    if (!rc) rc = ln.d_tot.reserve(3);
     return rc;
 }
 
@@ -125,7 +113,7 @@ int run_slab(dspfe_frontend_plan* pl, FeLane& ln, const int16_t* pcm, int64_t to
              float* mfcc, int64_t mfcc_cap, double* cep, int32_t* cep_lag, int64_t cep_cap, double* feat, double* acr, int32_t* acr_lag,
              int64_t acr_cap, int64_t* const glob[3], const int64_t base[3], cudaStream_t st, const int64_t* dbase_in = nullptr,
              int64_t* dbase_out = nullptr, int64_t* h_tot = nullptr, cudaEvent_t wait_prev = nullptr) {
-    int rc = dspfe_endpoint(ln.ep, pcm, total, rel_off, nu, lr, nullptr, nullptr, nullptr, 0, st);
+    int rc = dspfe_endpoint(ln.ep.get(), pcm, total, rel_off, nu, lr, nullptr, nullptr, nullptr, 0, st);
     if (rc) return rc;
     // MFCC, cepstrum pitch and autocorrelation pitch depend on the endpoints only: three branches, so that the single-CTA
     // prefix sums, the latency-bound pitch_feature kernel and the ragged tails of the track kernels of one branch are filled
@@ -134,34 +122,34 @@ int run_slab(dspfe_frontend_plan* pl, FeLane& ln, const int16_t* pcm, int64_t to
     cudaStream_t sa = st, sb = st;
     if (fork) {
         for (int k = 0; k < 2; ++k) {
-            if (!ln.side[k]) CUDA_TRY(cudaStreamCreateWithFlags(&ln.side[k], cudaStreamNonBlocking));
-            if (!ln.ev_join[k]) CUDA_TRY(cudaEventCreateWithFlags(&ln.ev_join[k], cudaEventDisableTiming));
+            CUDA_TRY(ln.side[k].ensure());
+            CUDA_TRY(ln.ev_join[k].ensure());
         }
-        if (!ln.ev_fork) CUDA_TRY(cudaEventCreateWithFlags(&ln.ev_fork, cudaEventDisableTiming));
-        CUDA_TRY(cudaEventRecord(ln.ev_fork, st));
-        sa = ln.side[0]; sb = ln.side[1];
-        CUDA_TRY(cudaStreamWaitEvent(sa, ln.ev_fork, 0));
-        CUDA_TRY(cudaStreamWaitEvent(sb, ln.ev_fork, 0));
+        CUDA_TRY(ln.ev_fork.ensure());
+        CUDA_TRY(cudaEventRecord(ln.ev_fork.get(), st));
+        sa = ln.side[0].get(); sb = ln.side[1].get();
+        CUDA_TRY(cudaStreamWaitEvent(sa, ln.ev_fork.get(), 0));
+        CUDA_TRY(cudaStreamWaitEvent(sb, ln.ev_fork.get(), 0));
     }
-    rc = dspfe_pitch(ln.cep, pcm, 0, total, rel_off, lr, nu, cep, cep_lag, feat, nullptr, ln.loc_off[1], cep_cap, sa);
+    rc = dspfe_pitch(ln.cep.get(), pcm, 0, total, rel_off, lr, nu, cep, cep_lag, feat, nullptr, ln.loc_off[1].get(), cep_cap, sa);
     if (rc) return rc;
-    rc = dspfe_pitch(ln.acr, pcm, 0, total, rel_off, lr, nu, acr, acr_lag, nullptr, nullptr, ln.loc_off[2], acr_cap, sb);
+    rc = dspfe_pitch(ln.acr.get(), pcm, 0, total, rel_off, lr, nu, acr, acr_lag, nullptr, nullptr, ln.loc_off[2].get(), acr_cap, sb);
     if (rc) return rc;
-    rc = dspfe_mfcc_delta(ln.mf, pcm, total, rel_off, lr, nu, mfcc, mfcc_cap, ln.loc_off[0], st);
+    rc = dspfe_mfcc_delta(ln.mf.get(), pcm, total, rel_off, lr, nu, mfcc, mfcc_cap, ln.loc_off[0].get(), st);
     if (rc) return rc;
     if (fork) {
-        CUDA_TRY(cudaEventRecord(ln.ev_join[0], sa));
-        CUDA_TRY(cudaEventRecord(ln.ev_join[1], sb));
-        CUDA_TRY(cudaStreamWaitEvent(st, ln.ev_join[0], 0));
-        CUDA_TRY(cudaStreamWaitEvent(st, ln.ev_join[1], 0));
+        CUDA_TRY(cudaEventRecord(ln.ev_join[0].get(), sa));
+        CUDA_TRY(cudaEventRecord(ln.ev_join[1].get(), sb));
+        CUDA_TRY(cudaStreamWaitEvent(st, ln.ev_join[0].get(), 0));
+        CUDA_TRY(cudaStreamWaitEvent(st, ln.ev_join[1].get(), 0));
     }
     if (wait_prev) CUDA_TRY(cudaStreamWaitEvent(st, wait_prev, 0));
     FeFinish f;
-    for (int k = 0; k < 3; ++k) { f.loc[k] = ln.loc_off[k]; f.glob[k] = glob[k]; f.base[k] = base[k]; }
-    f.tot = ln.d_tot; f.n = nu + 1; f.dbase_in = dbase_in; f.dbase_out = dbase_out;
+    for (int k = 0; k < 3; ++k) { f.loc[k] = ln.loc_off[k].get(); f.glob[k] = glob[k]; f.base[k] = base[k]; }
+    f.tot = ln.d_tot.get(); f.n = nu + 1; f.dbase_in = dbase_in; f.dbase_out = dbase_out;
     fe_finish_kernel<<<(unsigned)((nu + 1 + 255) / 256), 256, 0, st>>>(f);
     LAUNCH_CHECK("fe_finish_kernel", st);
-    CUDA_TRY(cudaMemcpyAsync(h_tot ? h_tot : pl->h_tot, ln.d_tot, 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(h_tot ? h_tot : pl->h_tot.get(), ln.d_tot.get(), 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
     return DSPFE_OK;
 }
 
@@ -184,28 +172,6 @@ void dspfe_frontend_params_default(dspfe_frontend_params* p) {
 
 void dspfe_frontend_destroy(dspfe_frontend_plan* pl) {
     if (!pl) return;
-    for (auto& ln : pl->lanes) {
-        dspfe_endpoint_destroy(ln.ep); dspfe_plan_destroy(ln.mf); dspfe_pitch_destroy(ln.cep); dspfe_pitch_destroy(ln.acr);
-        for (auto q : ln.loc_off) cudaFree(q);
-        cudaFree(ln.d_tot);
-        if (ln.stream) cudaStreamDestroy(ln.stream);
-        if (ln.finish_done) cudaEventDestroy(ln.finish_done);
-        for (auto q : ln.side) if (q) cudaStreamDestroy(q);
-        for (auto q : ln.ev_join) if (q) cudaEventDestroy(q);
-        if (ln.ev_fork) cudaEventDestroy(ln.ev_fork);
-    }
-    cudaFree(pl->rel_off); cudaFree(pl->d_base); if (pl->h_tot) cudaFreeHost(pl->h_tot);
-    cudaFree(pl->s_lr); cudaFree(pl->s_mfcc); cudaFree(pl->s_cep); cudaFree(pl->s_acr);
-    for (auto& s : pl->slots) {
-        cudaFree(s.d_pcm); cudaFree(s.d_rel); if (s.h_rel) cudaFreeHost(s.h_rel);
-        cudaFree(s.d_lr); cudaFree(s.d_feat); for (auto q : s.d_goff) cudaFree(q);
-        cudaFree(s.d_mfcc); cudaFree(s.d_cep); cudaFree(s.d_acr); cudaFree(s.d_cep_lag); cudaFree(s.d_acr_lag);
-        if (s.h2d_done) cudaEventDestroy(s.h2d_done);
-        if (s.compute_done) cudaEventDestroy(s.compute_done);
-        if (s.d2h_done) cudaEventDestroy(s.d2h_done);
-    }
-    if (pl->s_copy) cudaStreamDestroy(pl->s_copy);
-    if (pl->s_out) cudaStreamDestroy(pl->s_out);
     delete pl;
 }
 
@@ -220,9 +186,9 @@ int dspfe_frontend_create(const dspfe_frontend_params* q, dspfe_frontend_plan** 
     if (pl->prm.slab_samples == 0) pl->prm.slab_samples = 256ll << 20;
     if (pl->prm.host_slab_samples == 0) pl->prm.host_slab_samples = 32ll << 20;
     int rc = create_lane(pl->lanes[0], pl->prm);       // the second lane (host path only) is created on first use
-    if (!rc && cudaMalloc(&pl->d_base, 6 * sizeof(int64_t)) != cudaSuccess) rc = fail(DSPFE_ERR_CUDA, "cudaMalloc failed");
-    if (!rc && cudaHostAlloc(&pl->h_tot, kFeSlots * 3 * sizeof(int64_t), cudaHostAllocDefault) != cudaSuccess) rc = fail(DSPFE_ERR_CUDA, "cudaHostAlloc failed");
-    if (rc) { const std::string keep = g_err; dspfe_frontend_destroy(pl); g_err = keep; return rc; }
+    if (!rc) rc = pl->d_base.reserve(6);
+    if (!rc) rc = pl->h_tot.reserve(kFeSlots * 3);
+    if (rc) { const std::string keep = g_err; delete pl; g_err = keep; return rc; }
     *plan = pl;
     return DSPFE_OK;
 }
@@ -233,9 +199,9 @@ int dspfe_frontend_bounds(const dspfe_frontend_plan* pl, int64_t total_samples, 
     const int64_t slabs = total_samples / std::min(pl->prm.slab_samples, pl->prm.host_slab_samples) + 8;   // (+ the host path's short ramp-up / ramp-down slabs)
     const int64_t padded = total_samples + 8 * slabs;
     const FeLane& l0 = pl->lanes[0];
-    caps[0] = dspfe_rows_bound(l0.mf, padded, n_utt);
-    caps[1] = dspfe_pitch_frames_bound(l0.cep, padded, n_utt) + 3 * slabs;
-    caps[2] = dspfe_pitch_frames_bound(l0.acr, padded, n_utt) + 3 * slabs;
+    caps[0] = dspfe_rows_bound(l0.mf.get(), padded, n_utt);
+    caps[1] = dspfe_pitch_frames_bound(l0.cep.get(), padded, n_utt) + 3 * slabs;
+    caps[2] = dspfe_pitch_frames_bound(l0.acr.get(), padded, n_utt) + 3 * slabs;
     return DSPFE_OK;
 }
 
@@ -253,30 +219,30 @@ int dspfe_frontend(dspfe_frontend_plan* pl, const int16_t* d_pcm, const int64_t*
         const int32_t u1 = slab_end(h_off, u0, n_utt, pl->prm.slab_samples), nu = u1 - u0;
         const int64_t a0 = h_off[u0] & ~(int64_t)7, total = h_off[u1] - a0;
         FeLane& ln = pl->lanes[0];
-        int rc = ensure_utt(ln, nu + 1);
+        int rc = DSPFE_OK;
+        for (auto& q : ln.loc_off) if (!rc) rc = q.reserve(nu + 1);
+        if (!rc) rc = pl->rel_off.reserve(nu + 1);
         if (rc) return rc;
-        rc = grow(pl->rel_off, pl->cap_rel, nu + 1);
-        if (rc) return rc;
-        fe_rel_offsets_kernel<<<(unsigned)((nu + 1 + 255) / 256), 256, 0, st>>>(d_offsets + u0, nu + 1, a0, pl->rel_off);
+        fe_rel_offsets_kernel<<<(unsigned)((nu + 1 + 255) / 256), 256, 0, st>>>(d_offsets + u0, nu + 1, a0, pl->rel_off.get());
         LAUNCH_CHECK("fe_rel_offsets_kernel", st);
-        const int64_t need0 = dspfe_rows_bound(ln.mf, total, nu), need1 = dspfe_pitch_frames_bound(ln.cep, total, nu),
-                      need2 = dspfe_pitch_frames_bound(ln.acr, total, nu);
+        const int64_t need0 = dspfe_rows_bound(ln.mf.get(), total, nu), need1 = dspfe_pitch_frames_bound(ln.cep.get(), total, nu),
+                      need2 = dspfe_pitch_frames_bound(ln.acr.get(), total, nu);
         int32_t* lr = o->lr ? o->lr + 2 * (int64_t)u0 : nullptr;
         float* mfcc = o->mfcc ? o->mfcc + base[0] * kFeWidth : nullptr; int64_t cap0 = o->mfcc_cap - base[0];
         double* cep = o->cep_pitch ? o->cep_pitch + base[1] : nullptr; int64_t cap1 = o->cep_cap - base[1];
         double* acr = o->acr_pitch ? o->acr_pitch + base[2] : nullptr; int64_t cap2 = o->acr_cap - base[2];
-        if (!lr) { rc = grow(pl->s_lr, pl->cap_slr, 2 * (int64_t)nu); if (rc) return rc; lr = pl->s_lr; }
-        if (!mfcc) { rc = grow(pl->s_mfcc, pl->cap_smfcc, need0 * kFeWidth); if (rc) return rc; mfcc = pl->s_mfcc; cap0 = need0; }
-        if (!cep) { rc = grow(pl->s_cep, pl->cap_scep, need1); if (rc) return rc; cep = pl->s_cep; cap1 = need1; }
-        if (!acr) { rc = grow(pl->s_acr, pl->cap_sacr, need2); if (rc) return rc; acr = pl->s_acr; cap2 = need2; }
+        if (!lr) { rc = pl->s_lr.reserve(2 * (int64_t)nu); if (rc) return rc; lr = pl->s_lr.get(); }
+        if (!mfcc) { rc = pl->s_mfcc.reserve(need0 * kFeWidth); if (rc) return rc; mfcc = pl->s_mfcc.get(); cap0 = need0; }
+        if (!cep) { rc = pl->s_cep.reserve(need1); if (rc) return rc; cep = pl->s_cep.get(); cap1 = need1; }
+        if (!acr) { rc = pl->s_acr.reserve(need2); if (rc) return rc; acr = pl->s_acr.get(); cap2 = need2; }
         if (cap0 < need0 || cap1 < need1 || cap2 < need2) return fail(DSPFE_ERR_INVALID_ARG, "output capacity is below dspfe_frontend_bounds()");
         int64_t* glob[3] = {o->mfcc_frame_off ? o->mfcc_frame_off + u0 : nullptr, o->cep_frame_off ? o->cep_frame_off + u0 : nullptr,
                             o->acr_frame_off ? o->acr_frame_off + u0 : nullptr};
-        rc = run_slab(pl, ln, d_pcm + a0, total, pl->rel_off, nu, lr, mfcc, cap0, cep, o->cep_lag ? o->cep_lag + base[1] : nullptr, cap1,
+        rc = run_slab(pl, ln, d_pcm + a0, total, pl->rel_off.get(), nu, lr, mfcc, cap0, cep, o->cep_lag ? o->cep_lag + base[1] : nullptr, cap1,
                       o->cep_feat ? o->cep_feat + 5 * (int64_t)u0 : nullptr, acr, o->acr_lag ? o->acr_lag + base[2] : nullptr, cap2, glob, base, st);
         if (rc) return rc;
         CUDA_TRY(cudaStreamSynchronize(st));
-        for (int k = 0; k < 3; ++k) base[k] += pl->h_tot[k];
+        for (int k = 0; k < 3; ++k) base[k] += pl->h_tot.get()[k];
         u0 = u1;
     }
     if (totals) for (int k = 0; k < 3; ++k) totals[k] = base[k];
@@ -290,17 +256,17 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
     if (n_utt == 0) return DSPFE_OK;
     if (!h_pcm && h_off[n_utt] > h_off[0]) return fail(DSPFE_ERR_INVALID_ARG, "h_pcm is null");
     for (int32_t u = 0; u < n_utt; ++u) if (h_off[u + 1] < h_off[u]) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-    if (!pl->s_copy) CUDA_TRY(cudaStreamCreateWithFlags(&pl->s_copy, cudaStreamNonBlocking));
+    CUDA_TRY(pl->s_copy.ensure());
     for (auto& ln : pl->lanes) {
         if (!ln.ep) { int rc = create_lane(ln, pl->prm); if (rc) return rc; }
-        if (!ln.stream) CUDA_TRY(cudaStreamCreateWithFlags(&ln.stream, cudaStreamNonBlocking));
-        if (!ln.finish_done) CUDA_TRY(cudaEventCreateWithFlags(&ln.finish_done, cudaEventDisableTiming));
+        CUDA_TRY(ln.stream.ensure());
+        CUDA_TRY(ln.finish_done.ensure());
     }
-    if (!pl->s_out) CUDA_TRY(cudaStreamCreateWithFlags(&pl->s_out, cudaStreamNonBlocking));
+    CUDA_TRY(pl->s_out.ensure());
     for (auto& s : pl->slots) {
-        if (!s.h2d_done) CUDA_TRY(cudaEventCreateWithFlags(&s.h2d_done, cudaEventDisableTiming));
-        if (!s.compute_done) CUDA_TRY(cudaEventCreateWithFlags(&s.compute_done, cudaEventDisableTiming));
-        if (!s.d2h_done) CUDA_TRY(cudaEventCreateWithFlags(&s.d2h_done, cudaEventDisableTiming));
+        CUDA_TRY(s.h2d_done.ensure());
+        CUDA_TRY(s.compute_done.ensure());
+        CUDA_TRY(s.d2h_done.ensure());
     }
     // the slabs
     std::vector<int32_t> cut{0};                         // short slabs first: the kernels start after a quarter-slab's copy;
@@ -317,27 +283,22 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
         FeSlot& sl = pl->slots[s % kFeSlots];
         const int32_t u0 = cut[s], u1 = cut[s + 1], nu = u1 - u0;
         const int64_t a0 = std::max(h_off[u0] & ~(int64_t)7, base0), total = h_off[u1] - a0;
-        CUDA_TRY(cudaStreamWaitEvent(pl->s_copy, sl.compute_done, 0));            // the slab that used this slot has been processed
-        int rc = grow(sl.d_pcm, sl.cap_samples, total + 16, pl->prm.host_slab_samples + 16);
+        const cudaStream_t scopy = pl->s_copy.get();
+        CUDA_TRY(cudaStreamWaitEvent(scopy, sl.compute_done.get(), 0));            // the slab that used this slot has been processed
+        const int64_t n = nu + 1;
+        int rc = sl.d_pcm.reserve(total + 16, pl->prm.host_slab_samples + 16);
+        if (!rc) rc = sl.d_rel.reserve(n, 1024);
+        if (!rc) rc = sl.d_lr.reserve(2 * n, 2 * 1024);
+        if (!rc) rc = sl.d_feat.reserve(5 * n, 5 * 1024);
+        for (auto& q : sl.d_goff) if (!rc) rc = q.reserve(n, 1024);
+        if (!rc) rc = sl.h_rel.reserve(n, 1024);
         if (rc) return rc;
-        if (nu + 1 > sl.cap_utt) {
-            cudaFree(sl.d_rel); cudaFree(sl.d_lr); cudaFree(sl.d_feat); for (auto& q : sl.d_goff) { cudaFree(q); q = nullptr; }
-            if (sl.h_rel) cudaFreeHost(sl.h_rel);
-            sl.d_rel = nullptr; sl.d_lr = nullptr; sl.d_feat = nullptr; sl.h_rel = nullptr; sl.cap_utt = 0;
-            const int64_t cap = std::max<int64_t>(nu + 1, 1024);
-            CUDA_TRY(cudaMalloc(&sl.d_rel, cap * sizeof(int64_t)));
-            CUDA_TRY(cudaMalloc(&sl.d_lr, cap * 2 * sizeof(int32_t)));
-            CUDA_TRY(cudaMalloc(&sl.d_feat, cap * 5 * sizeof(double)));
-            for (auto& q : sl.d_goff) CUDA_TRY(cudaMalloc(&q, cap * sizeof(int64_t)));
-            CUDA_TRY(cudaHostAlloc(&sl.h_rel, cap * sizeof(int64_t), cudaHostAllocDefault));
-            sl.cap_utt = cap;
-        }
-        CUDA_TRY(cudaEventSynchronize(sl.h2d_done));                               // the slot's previous offsets have left h_rel
-        for (int32_t i = 0; i <= nu; ++i) sl.h_rel[i] = h_off[u0 + i] - a0;
+        CUDA_TRY(cudaEventSynchronize(sl.h2d_done.get()));                         // the slot's previous offsets have left h_rel
+        for (int32_t i = 0; i <= nu; ++i) sl.h_rel.get()[i] = h_off[u0 + i] - a0;
         // (a0 - base0 .. ) may start before h_off[u0]: those samples belong to the previous utterance and exist in h_pcm
-        if (total > 0) CUDA_TRY(cudaMemcpyAsync(sl.d_pcm, h_pcm + a0, total * sizeof(int16_t), cudaMemcpyHostToDevice, pl->s_copy));
-        CUDA_TRY(cudaMemcpyAsync(sl.d_rel, sl.h_rel, (nu + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, pl->s_copy));
-        CUDA_TRY(cudaEventRecord(sl.h2d_done, pl->s_copy));
+        if (total > 0) CUDA_TRY(cudaMemcpyAsync(sl.d_pcm.get(), h_pcm + a0, total * sizeof(int16_t), cudaMemcpyHostToDevice, scopy));
+        CUDA_TRY(cudaMemcpyAsync(sl.d_rel.get(), sl.h_rel.get(), n * sizeof(int64_t), cudaMemcpyHostToDevice, scopy));
+        CUDA_TRY(cudaEventRecord(sl.h2d_done.get(), scopy));
         return DSPFE_OK;
     };
     // The kernels of slab s are queued without waiting for slab s - 1, on the other lane (its own plans and stream: two slabs
@@ -346,31 +307,31 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
     // D2H copies, and drains slab s - 1 after queuing slab s, so the GPU never waits for the host.
     int64_t base[3] = {0, 0, 0};
     const int64_t zero3[3] = {0, 0, 0};
-    CUDA_TRY(cudaMemsetAsync(pl->d_base, 0, 3 * sizeof(int64_t), pl->lanes[0].stream));    // slab 0 runs on lane 0 and reads d_base[0]
+    CUDA_TRY(cudaMemsetAsync(pl->d_base.get(), 0, 3 * sizeof(int64_t), pl->lanes[0].stream.get()));    // slab 0 runs on lane 0 and reads d_base[0]
     auto drain = [&](int s) -> int {
         FeSlot& sl = pl->slots[s % kFeSlots];
         const int32_t u0 = cut[s], nu = cut[s + 1] - u0;
-        CUDA_TRY(cudaEventSynchronize(sl.compute_done));                           // the slab's frame counts are in its h_tot
-        const int64_t* ht = pl->h_tot + 3 * (s % kFeSlots);
+        CUDA_TRY(cudaEventSynchronize(sl.compute_done.get()));                     // the slab's frame counts are in its h_tot
+        const int64_t* ht = pl->h_tot.get() + 3 * (s % kFeSlots);
         const int64_t t0 = ht[0], t1 = ht[1], t2 = ht[2];
-        cudaStream_t so = pl->s_out;
-        CUDA_TRY(cudaStreamWaitEvent(so, sl.compute_done, 0));
-        if (o->lr) CUDA_TRY(cudaMemcpyAsync(o->lr + 2 * (int64_t)u0, sl.d_lr, (int64_t)nu * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
+        cudaStream_t so = pl->s_out.get();
+        CUDA_TRY(cudaStreamWaitEvent(so, sl.compute_done.get(), 0));
+        if (o->lr) CUDA_TRY(cudaMemcpyAsync(o->lr + 2 * (int64_t)u0, sl.d_lr.get(), (int64_t)nu * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
         if (o->mfcc) {
             if (base[0] + t0 > o->mfcc_cap) return fail(DSPFE_ERR_INVALID_ARG, "h_out->mfcc capacity too small");
-            CUDA_TRY(cudaMemcpyAsync(o->mfcc + base[0] * kFeWidth, sl.d_mfcc, t0 * kFeWidth * sizeof(float), cudaMemcpyDeviceToHost, so));
+            CUDA_TRY(cudaMemcpyAsync(o->mfcc + base[0] * kFeWidth, sl.d_mfcc.get(), t0 * kFeWidth * sizeof(float), cudaMemcpyDeviceToHost, so));
         }
         if ((o->cep_pitch || o->cep_lag) && base[1] + t1 > o->cep_cap) return fail(DSPFE_ERR_INVALID_ARG, "h_out cepstrum capacity too small");
         if ((o->acr_pitch || o->acr_lag) && base[2] + t2 > o->acr_cap) return fail(DSPFE_ERR_INVALID_ARG, "h_out autocorrelation capacity too small");
-        if (o->cep_pitch) CUDA_TRY(cudaMemcpyAsync(o->cep_pitch + base[1], sl.d_cep, t1 * sizeof(double), cudaMemcpyDeviceToHost, so));
-        if (o->acr_pitch) CUDA_TRY(cudaMemcpyAsync(o->acr_pitch + base[2], sl.d_acr, t2 * sizeof(double), cudaMemcpyDeviceToHost, so));
-        if (o->cep_lag) CUDA_TRY(cudaMemcpyAsync(o->cep_lag + base[1], sl.d_cep_lag, t1 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
-        if (o->acr_lag) CUDA_TRY(cudaMemcpyAsync(o->acr_lag + base[2], sl.d_acr_lag, t2 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
-        if (o->cep_feat) CUDA_TRY(cudaMemcpyAsync(o->cep_feat + 5 * (int64_t)u0, sl.d_feat, (int64_t)nu * 5 * sizeof(double), cudaMemcpyDeviceToHost, so));
+        if (o->cep_pitch) CUDA_TRY(cudaMemcpyAsync(o->cep_pitch + base[1], sl.d_cep.get(), t1 * sizeof(double), cudaMemcpyDeviceToHost, so));
+        if (o->acr_pitch) CUDA_TRY(cudaMemcpyAsync(o->acr_pitch + base[2], sl.d_acr.get(), t2 * sizeof(double), cudaMemcpyDeviceToHost, so));
+        if (o->cep_lag) CUDA_TRY(cudaMemcpyAsync(o->cep_lag + base[1], sl.d_cep_lag.get(), t1 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
+        if (o->acr_lag) CUDA_TRY(cudaMemcpyAsync(o->acr_lag + base[2], sl.d_acr_lag.get(), t2 * sizeof(int32_t), cudaMemcpyDeviceToHost, so));
+        if (o->cep_feat) CUDA_TRY(cudaMemcpyAsync(o->cep_feat + 5 * (int64_t)u0, sl.d_feat.get(), (int64_t)nu * 5 * sizeof(double), cudaMemcpyDeviceToHost, so));
         int64_t* hg[3] = {o->mfcc_frame_off, o->cep_frame_off, o->acr_frame_off};
         for (int k = 0; k < 3; ++k)
-            if (hg[k]) CUDA_TRY(cudaMemcpyAsync(hg[k] + u0, sl.d_goff[k], (int64_t)(nu + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, so));
-        CUDA_TRY(cudaEventRecord(sl.d2h_done, so));
+            if (hg[k]) CUDA_TRY(cudaMemcpyAsync(hg[k] + u0, sl.d_goff[k].get(), (int64_t)(nu + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost, so));
+        CUDA_TRY(cudaEventRecord(sl.d2h_done.get(), so));
         base[0] += t0; base[1] += t1; base[2] += t2;
         return DSPFE_OK;
     };
@@ -381,29 +342,32 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
         const int32_t u0 = cut[s], u1 = cut[s + 1], nu = u1 - u0;
         const int64_t a0 = std::max(h_off[u0] & ~(int64_t)7, base0), total = h_off[u1] - a0;
         FeLane& ln = pl->lanes[s % kFeLanes];
-        cudaStream_t sc = ln.stream;
-        const int64_t need0 = dspfe_rows_bound(ln.mf, total, nu), need1 = dspfe_pitch_frames_bound(ln.cep, total, nu),
-                      need2 = dspfe_pitch_frames_bound(ln.acr, total, nu);
-        CUDA_TRY(cudaStreamWaitEvent(sc, sl.d2h_done, 0));                        // the slot's previous outputs have left
-        rc = grow(sl.d_mfcc, sl.cap_rows, need0 * kFeWidth); if (rc) return rc;
-        rc = grow(sl.d_cep, sl.cap_cep, need1); if (rc) return rc;
-        rc = grow(sl.d_acr, sl.cap_acr, need2); if (rc) return rc;
-        if (o->cep_lag) { rc = grow(sl.d_cep_lag, sl.cap_cep_lag, need1); if (rc) return rc; }
-        if (o->acr_lag) { rc = grow(sl.d_acr_lag, sl.cap_acr_lag, need2); if (rc) return rc; }
-        rc = ensure_utt(ln, nu + 1); if (rc) return rc;
-        CUDA_TRY(cudaStreamWaitEvent(sc, sl.h2d_done, 0));
-        rc = run_slab(pl, ln, sl.d_pcm, total, sl.d_rel, nu, sl.d_lr, sl.d_mfcc, need0, sl.d_cep, o->cep_lag ? sl.d_cep_lag : nullptr, need1, sl.d_feat, sl.d_acr,
-                      o->acr_lag ? sl.d_acr_lag : nullptr, need2, sl.d_goff, zero3, sc, pl->d_base + 3 * (s & 1), pl->d_base + 3 * ((s + 1) & 1),
-                      pl->h_tot + 3 * (s % kFeSlots), s > 0 ? pl->lanes[(s - 1) % kFeLanes].finish_done : nullptr);
+        cudaStream_t sc = ln.stream.get();
+        const int64_t need0 = dspfe_rows_bound(ln.mf.get(), total, nu), need1 = dspfe_pitch_frames_bound(ln.cep.get(), total, nu),
+                      need2 = dspfe_pitch_frames_bound(ln.acr.get(), total, nu);
+        CUDA_TRY(cudaStreamWaitEvent(sc, sl.d2h_done.get(), 0));                  // the slot's previous outputs have left
+        rc = sl.d_mfcc.reserve(need0 * kFeWidth);
+        if (!rc) rc = sl.d_cep.reserve(need1);
+        if (!rc) rc = sl.d_acr.reserve(need2);
+        if (!rc && o->cep_lag) rc = sl.d_cep_lag.reserve(need1);
+        if (!rc && o->acr_lag) rc = sl.d_acr_lag.reserve(need2);
+        for (auto& q : ln.loc_off) if (!rc) rc = q.reserve(nu + 1);
         if (rc) return rc;
-        CUDA_TRY(cudaEventRecord(ln.finish_done, sc));
-        CUDA_TRY(cudaEventRecord(sl.compute_done, sc));
+        CUDA_TRY(cudaStreamWaitEvent(sc, sl.h2d_done.get(), 0));
+        int64_t* const goff[3] = {sl.d_goff[0].get(), sl.d_goff[1].get(), sl.d_goff[2].get()};
+        rc = run_slab(pl, ln, sl.d_pcm.get(), total, sl.d_rel.get(), nu, sl.d_lr.get(), sl.d_mfcc.get(), need0, sl.d_cep.get(),
+                      o->cep_lag ? sl.d_cep_lag.get() : nullptr, need1, sl.d_feat.get(), sl.d_acr.get(), o->acr_lag ? sl.d_acr_lag.get() : nullptr,
+                      need2, goff, zero3, sc, pl->d_base.get() + 3 * (s & 1), pl->d_base.get() + 3 * ((s + 1) & 1),
+                      pl->h_tot.get() + 3 * (s % kFeSlots), s > 0 ? pl->lanes[(s - 1) % kFeLanes].finish_done.get() : nullptr);
+        if (rc) return rc;
+        CUDA_TRY(cudaEventRecord(ln.finish_done.get(), sc));
+        CUDA_TRY(cudaEventRecord(sl.compute_done.get(), sc));
         if (s + 1 < n_slab) { rc = issue_h2d(s + 1); if (rc) return rc; }          // overlaps this slab's kernels
         if (s >= 1) { rc = drain(s - 1); if (rc) return rc; }                      // (that slab finished while this one was being queued)
     }
     rc = drain(n_slab - 1);
     if (rc) return rc;
-    CUDA_TRY(cudaStreamSynchronize(pl->s_out));
+    CUDA_TRY(cudaStreamSynchronize(pl->s_out.get()));
     if (totals) for (int k = 0; k < 3; ++k) totals[k] = base[k];
     return DSPFE_OK;
 }
@@ -411,9 +375,8 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
 /* ---- per-kernel timing ---- */
 int dspfe_timing_begin(void* stream) {
     StageTimer& t = g_timer;
-    for (auto& m : t.marks) cudaEventDestroy(m.second);
-    t.marks.clear();
-    if (!t.start) CUDA_TRY(cudaEventCreate(&t.start));
+    t.clear_marks();
+    CUDA_TRY(t.ensure_start());
     t.stream = (cudaStream_t)stream;
     CUDA_TRY(cudaEventRecord(t.start, t.stream));
     t.on = true;
@@ -437,8 +400,7 @@ int dspfe_timing_end(char* names, float* ms, int32_t cap, int32_t* n) {
         }
         prev = t.marks[i].second;
     }
-    for (auto& m : t.marks) cudaEventDestroy(m.second);
-    t.marks.clear();
+    t.clear_marks();
     return DSPFE_OK;
 }
 

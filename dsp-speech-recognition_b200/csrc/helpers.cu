@@ -220,12 +220,11 @@ int dspfe_row_windowed_amplitude_f64(const double* d_frames, int64_t n_rows, int
         c[m] = hi >= lo ? pre[hi + 1] - pre[lo] : 0.0;
     }
     cudaStream_t st = (cudaStream_t)stream;
-    double* d_c = nullptr;
-    CUDA_TRY(cudaMallocAsync(&d_c, (size_t)N * sizeof(double), st));
-    CUDA_TRY(cudaMemcpyAsync(d_c, c.data(), (size_t)N * sizeof(double), cudaMemcpyHostToDevice, st));
-    row_weighted_amp_kernel<<<grid_for(n_rows, 4), 128, 0, st>>>(d_frames, n_rows, len, d_c, use_sq, d_out);
+    StreamTemp<double> d_c;
+    CUDA_TRY(d_c.alloc(N, st));
+    CUDA_TRY(cudaMemcpyAsync(d_c.get(), c.data(), (size_t)N * sizeof(double), cudaMemcpyHostToDevice, st));
+    row_weighted_amp_kernel<<<grid_for(n_rows, 4), 128, 0, st>>>(d_frames, n_rows, len, d_c.get(), use_sq, d_out);
     cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_c, st);
     if (e != cudaSuccess) return fail(DSPFE_ERR_CUDA, std::string("row_weighted_amp_kernel: ") + cudaGetErrorString(e));
     return DSPFE_OK;
 }
@@ -269,13 +268,12 @@ int dspfe_fir_window_f64(const double* d_x, int32_t n, double rate, double low_f
     std::vector<double> hr, hi;
     fir_taps(n, rate, low_freq, high_freq, hamming != 0, hr, hi);
     cudaStream_t st = (cudaStream_t)stream;
-    double* d_h = nullptr;
-    CUDA_TRY(cudaMallocAsync(&d_h, 2 * (size_t)n * sizeof(double), st));
-    CUDA_TRY(cudaMemcpyAsync(d_h, hr.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(d_h + n, hi.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
-    fir_window_kernel<<<grid_for(n, 128), 128, 0, st>>>(d_x, n, d_h, d_h + n, d_y);
+    StreamTemp<double> d_h;
+    CUDA_TRY(d_h.alloc(2 * (int64_t)n, st));
+    CUDA_TRY(cudaMemcpyAsync(d_h.get(), hr.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(d_h.get() + n, hi.data(), n * sizeof(double), cudaMemcpyHostToDevice, st));
+    fir_window_kernel<<<grid_for(n, 128), 128, 0, st>>>(d_x, n, d_h.get(), d_h.get() + n, d_y);
     cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_h, st);
     if (e != cudaSuccess) return fail(DSPFE_ERR_CUDA, std::string("fir_window_kernel: ") + cudaGetErrorString(e));
     return DSPFE_OK;
 }
@@ -283,12 +281,11 @@ int dspfe_fir_window_f64(const double* d_x, int32_t n, double rate, double low_f
 int dspfe_acr_f64(const double* d_frame, int32_t len, int32_t n, double* d_out, void* stream) {
     if (!d_frame || !d_out || len < 1 || n < 0 || n >= len) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     cudaStream_t st = (cudaStream_t)stream;
-    double* d_prod = nullptr;
-    CUDA_TRY(cudaMallocAsync(&d_prod, (size_t)(len - n) * sizeof(double), st));
-    lag_products_kernel<<<grid_for(len - n, 256), 256, 0, st>>>(d_frame, len, n, d_prod);
-    acr_finish_kernel<<<1, 32, 0, st>>>(d_prod, len - n, len, n, d_out);
+    StreamTemp<double> d_prod;
+    CUDA_TRY(d_prod.alloc(len - n, st));
+    lag_products_kernel<<<grid_for(len - n, 256), 256, 0, st>>>(d_frame, len, n, d_prod.get());
+    acr_finish_kernel<<<1, 32, 0, st>>>(d_prod.get(), len - n, len, n, d_out);
     cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_prod, st);
     if (e != cudaSuccess) return fail(DSPFE_ERR_CUDA, std::string("acr kernels: ") + cudaGetErrorString(e));
     return DSPFE_OK;
 }

@@ -201,50 +201,36 @@ __global__ void center_clip_kernel(const float* in, int64_t n_rows, int len, int
 struct dspfe_pitch_plan {
     dspfe_pitch_params prm;
     PitchParams base;          // scalars + table pointers; per-call pointers filled in launch
-    float2* d_tab = nullptr;
+    Stream stream;             // host path
+    DeviceArray<float2> d_tab;
     // workspaces
-    int64_t cap_utt = 0, cap_frames = 0, cap_slots = 0;
-    int64_t* seg_start = nullptr; int32_t* seg_len = nullptr; int32_t* ds_len = nullptr; int64_t* frame_off = nullptr; int64_t* slot_off = nullptr;
-    int32_t* order = nullptr;
-    float2* clip = nullptr; int4* run_desc = nullptr; float* rows = nullptr; double* frame_amp = nullptr; double* pitch = nullptr; int32_t* lag = nullptr; double* scratch = nullptr;
+    DeviceArray<int64_t> seg_start; DeviceArray<int32_t> seg_len, ds_len; DeviceArray<int64_t> frame_off, slot_off;
+    DeviceArray<int32_t> order;
+    DeviceArray<float2> clip; DeviceArray<int4> run_desc; DeviceArray<float> rows; DeviceArray<double> frame_amp, pitch;
+    DeviceArray<int32_t> lag; DeviceArray<double> scratch;
     // host-path staging
-    cudaStream_t stream = nullptr;
-    void* d_pcm = nullptr; int64_t cap_bytes = 0;
-    int64_t* d_off = nullptr; int32_t* d_trim = nullptr; double* d_feat = nullptr; int64_t cap_hutt = 0;
+    DeviceArray<unsigned char> d_pcm;
+    DeviceArray<int64_t> d_off; DeviceArray<int32_t> d_trim; DeviceArray<double> d_feat;
 };
 
 namespace {
 
 int ensure(dspfe_pitch_plan* pl, int64_t n_utt, int64_t frames) {
-    if (n_utt + 1 > pl->cap_utt) {
-        cudaFree(pl->seg_start); cudaFree(pl->seg_len); cudaFree(pl->ds_len); cudaFree(pl->frame_off); cudaFree(pl->slot_off); cudaFree(pl->order);
-        pl->order = nullptr; pl->seg_start = nullptr; pl->seg_len = nullptr; pl->ds_len = nullptr; pl->frame_off = nullptr; pl->slot_off = nullptr; pl->cap_utt = 0;
-        CUDA_TRY(cudaMalloc(&pl->seg_start, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->seg_len, (n_utt + 1) * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->ds_len, (n_utt + 1) * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->frame_off, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->slot_off, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->order, (n_utt + 1) * sizeof(int32_t)));
-        pl->cap_utt = n_utt + 1;
-    }
-    if (frames > pl->cap_frames) {
-        cudaFree(pl->rows); cudaFree(pl->frame_amp); cudaFree(pl->pitch); cudaFree(pl->lag); cudaFree(pl->scratch);
-        pl->rows = nullptr; pl->frame_amp = nullptr; pl->pitch = nullptr; pl->lag = nullptr; pl->scratch = nullptr; pl->cap_frames = 0;
-        CUDA_TRY(cudaMalloc(&pl->rows, frames * pl->base.row_len * sizeof(float)));
-        CUDA_TRY(cudaMalloc(&pl->frame_amp, frames * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&pl->pitch, frames * sizeof(double)));
-        CUDA_TRY(cudaMalloc(&pl->lag, frames * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->scratch, 3 * frames * sizeof(double)));
-        pl->cap_frames = frames;
-    }
+    int rc = pl->seg_start.reserve(n_utt + 1);
+    if (!rc) rc = pl->seg_len.reserve(n_utt + 1);
+    if (!rc) rc = pl->ds_len.reserve(n_utt + 1);
+    if (!rc) rc = pl->frame_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->slot_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->order.reserve(n_utt + 1);
+    if (!rc) rc = pl->rows.reserve(frames * pl->base.row_len);
+    if (!rc) rc = pl->frame_amp.reserve(frames);
+    if (!rc) rc = pl->pitch.reserve(frames);
+    if (!rc) rc = pl->lag.reserve(frames);
+    if (!rc) rc = pl->scratch.reserve(3 * frames);
     const int64_t slots = frames + (kClipRun - 1) * n_utt;       // every utterance's frame count rounded up to a run
-    if (slots > pl->cap_slots) {
-        cudaFree(pl->clip); cudaFree(pl->run_desc); pl->clip = nullptr; pl->run_desc = nullptr; pl->cap_slots = 0;
-        CUDA_TRY(cudaMalloc(&pl->clip, ((slots + 1) / 2) * 512 * sizeof(float2)));
-        CUDA_TRY(cudaMalloc(&pl->run_desc, (slots / kClipRun + 1) * sizeof(int4)));
-        pl->cap_slots = slots;
-    }
-    return DSPFE_OK;
+    if (!rc) rc = pl->clip.reserve(((slots + 1) / 2) * 512);
+    if (!rc) rc = pl->run_desc.reserve(slots / kClipRun + 1);
+    return rc;
 }
 
 int track_smem(int row_len) { return (track_chunk(row_len) + 1) * row_len * (int)sizeof(float) + track_chunk(row_len) * kPeakLags * (int)sizeof(int) + kTrackMaxFrames * 12 + (kTrackThreads / 32) * kTrackListPerWarp * 2 + 8; }
@@ -273,27 +259,22 @@ int dspfe_pitch_create(const dspfe_pitch_params* q, dspfe_pitch_plan** plan) {
     std::string err;
     const int trc = build_pitch_tables(*q, b, tab, err);
     if (trc) { delete pl; return fail(trc, err); }
-    cudaError_t e = cudaMalloc(&pl->d_tab, kTabTotal * sizeof(float2));
-    if (e == cudaSuccess) e = cudaMemcpy(pl->d_tab, tab.data(), kTabTotal * sizeof(float2), cudaMemcpyHostToDevice);
+    if (int rc = pl->d_tab.reserve(kTabTotal)) { delete pl; return rc; }
+    cudaError_t e = cudaMemcpy(pl->d_tab.get(), tab.data(), kTabTotal * sizeof(float2), cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_clip_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kClipCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_clip_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kClipCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFrameCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFrameCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQuadCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, track_smem(kCepLen));
-    if (e != cudaSuccess) { cudaFree(pl->d_tab); delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
-    b.tab = pl->d_tab;
+    if (e != cudaSuccess) { delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
+    b.tab = pl->d_tab.get();
     *plan = pl;
     return DSPFE_OK;
 }
 
 void dspfe_pitch_destroy(dspfe_pitch_plan* pl) {
     if (!pl) return;
-    cudaFree(pl->d_tab);
-    cudaFree(pl->seg_start); cudaFree(pl->seg_len); cudaFree(pl->ds_len); cudaFree(pl->frame_off); cudaFree(pl->slot_off); cudaFree(pl->order);
-    cudaFree(pl->clip); cudaFree(pl->run_desc); cudaFree(pl->rows); cudaFree(pl->frame_amp); cudaFree(pl->pitch); cudaFree(pl->lag); cudaFree(pl->scratch);
-    cudaFree(pl->d_pcm); cudaFree(pl->d_off); cudaFree(pl->d_trim); cudaFree(pl->d_feat);
-    if (pl->stream) cudaStreamDestroy(pl->stream);
     delete pl;
 }
 
@@ -341,10 +322,11 @@ int dspfe_pitch(dspfe_pitch_plan* pl, const void* d_pcm, int32_t sample_dtype, i
     cudaStream_t st = (cudaStream_t)stream;
     PitchParams p = pl->base;
     p.pcm = d_pcm; p.in_f32 = sample_dtype; p.total_samples = total_samples; p.offsets = d_offsets; p.trim = d_trim; p.n_utt = n_utt;
-    p.frame_off = d_frame_off ? d_frame_off : pl->frame_off; p.slot_off = pl->slot_off; p.seg_start = pl->seg_start; p.seg_len = pl->seg_len; p.ds_len = pl->ds_len;
-    p.clip = pl->clip; p.run_desc = pl->run_desc; p.rows = d_rows ? d_rows : pl->rows; p.rows_out = nullptr; p.score = nullptr; p.frame_amp = pl->frame_amp;
-    p.pitch = d_pitch ? d_pitch : pl->pitch; p.lag = d_lag ? d_lag : pl->lag; p.feat = d_feat; p.scratch = pl->scratch;
-    p.max_frames = bound; p.order = pl->order;
+    p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.slot_off = pl->slot_off.get(); p.seg_start = pl->seg_start.get();
+    p.seg_len = pl->seg_len.get(); p.ds_len = pl->ds_len.get(); p.clip = pl->clip.get(); p.run_desc = pl->run_desc.get();
+    p.rows = d_rows ? d_rows : pl->rows.get(); p.rows_out = nullptr; p.score = nullptr; p.frame_amp = pl->frame_amp.get();
+    p.pitch = d_pitch ? d_pitch : pl->pitch.get(); p.lag = d_lag ? d_lag : pl->lag.get(); p.feat = d_feat; p.scratch = pl->scratch.get();
+    p.max_frames = bound; p.order = pl->order.get();
     pitch_prep_kernel<<<1, kPitchPrepThreads, 0, st>>>(p);
     LAUNCH_CHECK("pitch_prep_kernel", st);
     const int64_t slots = bound + (int64_t)(kClipRun - 1) * n_utt;
@@ -377,19 +359,12 @@ int dspfe_pitch_host(dspfe_pitch_plan* pl, const void* h_pcm, int32_t sample_dty
     const int esz = sample_dtype ? 4 : 2;
     const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
     if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-    if (!pl->stream) CUDA_TRY(cudaStreamCreateWithFlags(&pl->stream, cudaStreamNonBlocking));
-    if ((total + 8) * esz > pl->cap_bytes) {
-        cudaFree(pl->d_pcm); pl->d_pcm = nullptr; pl->cap_bytes = 0;
-        CUDA_TRY(cudaMalloc(&pl->d_pcm, (total + 8) * esz));
-        pl->cap_bytes = (total + 8) * esz;
-    }
-    if (n_utt + 1 > pl->cap_hutt) {
-        cudaFree(pl->d_off); cudaFree(pl->d_trim); cudaFree(pl->d_feat); pl->d_off = nullptr; pl->d_trim = nullptr; pl->d_feat = nullptr; pl->cap_hutt = 0;
-        CUDA_TRY(cudaMalloc(&pl->d_off, (n_utt + 1) * sizeof(int64_t)));
-        CUDA_TRY(cudaMalloc(&pl->d_trim, (int64_t)n_utt * 2 * sizeof(int32_t)));
-        CUDA_TRY(cudaMalloc(&pl->d_feat, (int64_t)n_utt * 5 * sizeof(double)));
-        pl->cap_hutt = n_utt + 1;
-    }
+    CUDA_TRY(pl->stream.ensure());
+    int rc = pl->d_pcm.reserve((total + 8) * esz);
+    if (!rc) rc = pl->d_off.reserve(n_utt + 1);
+    if (!rc) rc = pl->d_trim.reserve((int64_t)n_utt * 2);
+    if (!rc) rc = pl->d_feat.reserve((int64_t)n_utt * 5);
+    if (rc) return rc;
     std::vector<int64_t> rel(n_utt + 1);
     int64_t frames = 0;
     for (int32_t u = 0; u <= n_utt; ++u) {
@@ -408,19 +383,19 @@ int dspfe_pitch_host(dspfe_pitch_plan* pl, const void* h_pcm, int32_t sample_dty
         }
     }
     if (h_frame_off) h_frame_off[n_utt] = frames;
-    cudaStream_t st = pl->stream;
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm, (const char*)h_pcm + base * esz, total * esz, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(pl->d_off, rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    if (h_trim) CUDA_TRY(cudaMemcpyAsync(pl->d_trim, h_trim, (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    cudaStream_t st = pl->stream.get();
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), (const char*)h_pcm + base * esz, total * esz, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    if (h_trim) CUDA_TRY(cudaMemcpyAsync(pl->d_trim.get(), h_trim, (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     const int64_t bound = dspfe_pitch_frames_bound(pl, total, n_utt);
-    int rc = ensure(pl, n_utt, bound);   // size the workspaces first: their pointers are the outputs of the device call
+    rc = ensure(pl, n_utt, bound);   // size the workspaces first: their pointers are the outputs of the device call
     if (rc) return rc;
-    rc = dspfe_pitch(pl, pl->d_pcm, sample_dtype, total, pl->d_off, h_trim ? pl->d_trim : nullptr, n_utt, pl->pitch, pl->lag,
-                     h_feat ? pl->d_feat : nullptr, nullptr, nullptr, bound, st);
+    rc = dspfe_pitch(pl, pl->d_pcm.get(), sample_dtype, total, pl->d_off.get(), h_trim ? pl->d_trim.get() : nullptr, n_utt, pl->pitch.get(),
+                     pl->lag.get(), h_feat ? pl->d_feat.get() : nullptr, nullptr, nullptr, bound, st);
     if (rc) return rc;
-    if (h_pitch) CUDA_TRY(cudaMemcpyAsync(h_pitch, pl->pitch, frames * sizeof(double), cudaMemcpyDeviceToHost, st));
-    if (h_lag) CUDA_TRY(cudaMemcpyAsync(h_lag, pl->lag, frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (h_feat) CUDA_TRY(cudaMemcpyAsync(h_feat, pl->d_feat, (int64_t)n_utt * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (h_pitch) CUDA_TRY(cudaMemcpyAsync(h_pitch, pl->pitch.get(), frames * sizeof(double), cudaMemcpyDeviceToHost, st));
+    if (h_lag) CUDA_TRY(cudaMemcpyAsync(h_lag, pl->lag.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (h_feat) CUDA_TRY(cudaMemcpyAsync(h_feat, pl->d_feat.get(), (int64_t)n_utt * 5 * sizeof(double), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return DSPFE_OK;
 }
@@ -442,19 +417,17 @@ int dspfe_track_rows_f32(const float* d_rows, int64_t n_rows, int32_t row_len, i
     if (row_len > 2 * kTrackThreads) return fail(DSPFE_ERR_UNSUPPORTED, "rows longer than 512 columns are not built");
     if (mode == 0 && (d_score || d_lag) && row_len < kMinLag + kPeakLags) return fail(DSPFE_ERR_INVALID_ARG, "peak_score needs rows of at least 100 columns");
     cudaStream_t st = (cudaStream_t)stream;
-    int64_t* d_fo = nullptr; int32_t* d_lag_tmp = nullptr;
-    CUDA_TRY(cudaMallocAsync(&d_fo, 2 * sizeof(int64_t), st));
-    if (!d_lag) CUDA_TRY(cudaMallocAsync(&d_lag_tmp, n_rows * sizeof(int32_t), st));
-    pitch_fill_off_kernel<<<1, 32, 0, st>>>(d_fo, n_rows);
+    StreamTemp<int64_t> d_fo; StreamTemp<int32_t> d_lag_tmp;
+    CUDA_TRY(d_fo.alloc(2, st));
+    if (!d_lag) CUDA_TRY(d_lag_tmp.alloc(n_rows, st));
+    pitch_fill_off_kernel<<<1, 32, 0, st>>>(d_fo.get(), n_rows);
     PitchParams p; std::memset(&p, 0, sizeof(p));
-    p.n_utt = 1; p.mode = mode; p.row_len = row_len; p.frame_off = d_fo; p.rows = const_cast<float*>(d_rows); p.rows_out = d_smoothed;
-    p.no_smooth = do_smooth ? 0 : 1; p.score = mode == 0 ? d_score : nullptr; p.lag = d_lag ? d_lag : d_lag_tmp; p.pitch = nullptr;
+    p.n_utt = 1; p.mode = mode; p.row_len = row_len; p.frame_off = d_fo.get(); p.rows = const_cast<float*>(d_rows); p.rows_out = d_smoothed;
+    p.no_smooth = do_smooth ? 0 : 1; p.score = mode == 0 ? d_score : nullptr; p.lag = d_lag ? d_lag : d_lag_tmp.get(); p.pitch = nullptr;
     static bool attr_done = false;
     if (!attr_done) { CUDA_TRY(cudaFuncSetAttribute(pitch_track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, track_smem(kCepLen))); attr_done = true; }
     pitch_track_kernel<<<1, kTrackThreads, track_smem(row_len), st>>>(p);
     cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_fo, st);
-    if (d_lag_tmp) cudaFreeAsync(d_lag_tmp, st);
     if (e != cudaSuccess) return fail(DSPFE_ERR_CUDA, std::string("pitch_track_kernel: ") + cudaGetErrorString(e));
     return DSPFE_OK;
 }
@@ -494,12 +467,11 @@ int dspfe_dp_max_pitch(const double* d_g, int32_t n_rows, int32_t n_cols, double
     if (!d_g || !d_path || n_rows < 2 || n_cols < 1) return fail(DSPFE_ERR_INVALID_ARG, "dp_max_pitch needs at least two rows");
     if (n_cols > kDpMaxCols) return fail(DSPFE_ERR_UNSUPPORTED, "dp_max_pitch is built for up to 1024 columns");
     cudaStream_t st = (cudaStream_t)stream;
-    int32_t* d_prev = nullptr;
-    CUDA_TRY(cudaMallocAsync(&d_prev, (size_t)n_rows * n_cols * sizeof(int32_t), st));
+    StreamTemp<int32_t> d_prev;
+    CUDA_TRY(d_prev.alloc((int64_t)n_rows * n_cols, st));
     const int threads = (n_cols + 31) & ~31;
-    dp_max_pitch_kernel<<<1, threads, 2 * n_cols * sizeof(double), st>>>(d_g, n_rows, n_cols, d_prev, d_path);
+    dp_max_pitch_kernel<<<1, threads, 2 * n_cols * sizeof(double), st>>>(d_g, n_rows, n_cols, d_prev.get(), d_path);
     cudaError_t e = cudaGetLastError();
-    cudaFreeAsync(d_prev, st);
     if (e != cudaSuccess) return fail(DSPFE_ERR_CUDA, std::string("dp_max_pitch_kernel: ") + cudaGetErrorString(e));
     return DSPFE_OK;
 }
