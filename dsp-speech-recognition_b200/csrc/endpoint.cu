@@ -16,8 +16,12 @@ struct dspfe_endpoint_plan {
     // workspaces
     DeviceArray<int64_t> frame_off, block_off; DeviceArray<int32_t> order;
     DeviceArray<int32_t> blk, asum, zcr;
-    // host-path staging
-    DeviceArray<int16_t> d_pcm;
+    DeviceArray<double> amp;    // float-sample path: K2f's float64 amplitudes, one per frame like asum
+    // float-sample path: the split tree of the pairwise sum over one frame (np_pairwise_tree), uploaded on first use
+    std::vector<int32_t> h_tree; int nleaf = 0;
+    DeviceArray<int32_t> tree; bool tree_ready = false;
+    // host-path staging (int16 or float32 samples)
+    DeviceArray<unsigned char> d_pcm;
     DeviceArray<int64_t> d_off; DeviceArray<int32_t> d_lr;
 };
 
@@ -43,6 +47,7 @@ int ensure(dspfe_endpoint_plan* pl, int64_t n_utt, int64_t blocks, int64_t frame
     if (!rc) rc = pl->blk.reserve(blocks * 6);
     if (!rc) rc = pl->asum.reserve(frames);
     if (!rc) rc = pl->zcr.reserve(frames);
+    if (!rc) rc = pl->amp.reserve(frames);
     return rc;
 }
 
@@ -123,6 +128,7 @@ int dspfe_endpoint_create(const dspfe_endpoint_params* p, dspfe_endpoint_plan** 
     int rc = fill_rule(*p, pl->rule, pl->frame_len, pl->frame_step);
     if (rc) { delete pl; return rc; }
     pl->q = pl->frame_len / pl->frame_step; pl->rem = pl->frame_len % pl->frame_step;
+    if (pl->frame_len <= kEpF32MaxLen) pl->h_tree = np_pairwise_tree(pl->frame_len, &pl->nleaf);
     *plan = pl;
     return DSPFE_OK;
 }
@@ -171,8 +177,48 @@ int dspfe_endpoint(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t total_
     LAUNCH_CHECK("ep_block_kernel", st);
     ep_frame_kernel<<<(unsigned)((frames_bound + 255) / 256), 256, 0, st>>>(p);
     LAUNCH_CHECK("ep_frame_kernel", st);
-    ep_decide_kernel<<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
+    ep_decide_kernel<AmpFromSum><<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
     LAUNCH_CHECK("ep_decide_kernel", st);
+    return DSPFE_OK;
+}
+
+int dspfe_endpoint_f32(dspfe_endpoint_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
+                       int32_t* d_lr, double* d_amp, int32_t* d_zcr, int64_t* d_frame_off, int64_t max_frames, void* stream) {
+    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (pl->frame_len > kEpF32MaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "float-sample endpoint frames longer than 8192 samples are not built");
+    if (n_utt == 0) return DSPFE_OK;
+    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
+    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
+    const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
+    if ((d_amp || d_zcr) && max_frames < frames_bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_endpoint_frames_bound()");
+    const int64_t blocks_bound = frames_bound + (int64_t)n_utt * (pl->q + 1);
+    int rc = ensure(pl, n_utt, blocks_bound, frames_bound);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!pl->tree_ready) {
+        rc = pl->tree.reserve((int64_t)pl->h_tree.size());
+        if (rc) return rc;
+        CUDA_TRY(cudaMemcpyAsync(pl->tree.get(), pl->h_tree.data(), pl->h_tree.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        pl->tree_ready = true;
+    }
+    EpParams p;
+    p.pcm = nullptr; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
+    p.q = pl->q; p.rem = pl->rem; p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.block_off = pl->block_off.get();
+    p.blk = pl->blk.get(); p.asum = nullptr; p.zcr = d_zcr ? d_zcr : pl->zcr.get(); p.lr = d_lr;
+    p.max_blocks = blocks_bound; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order.get();
+    p.amp = d_amp ? d_amp : pl->amp.get();
+    EpF32Params f;
+    f.pcm = d_pcm; f.total_samples = total_samples; f.offsets = d_offsets; f.frame_off = p.frame_off; f.n_utt = n_utt;
+    f.frame_len = pl->frame_len; f.frame_step = pl->frame_step; f.tree = pl->tree.get(); f.nleaf = pl->nleaf;
+    f.max_frames = frames_bound; f.amp = const_cast<double*>(p.amp); f.zcr = p.zcr;
+    ep_f32_layout(f);
+    ep_prep_kernel<<<1, kEpPrepThreads, 0, st>>>(p);
+    LAUNCH_CHECK("ep_prep_kernel", st);
+    if (f.sm_total > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(ep_stats_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, f.sm_total));
+    ep_stats_f32_kernel<<<(unsigned)((frames_bound + f.run - 1) / f.run), kEpF32Threads, f.sm_total, st>>>(f);
+    LAUNCH_CHECK("ep_stats_f32_kernel", st);
+    ep_decide_kernel<AmpFromF64><<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
+    LAUNCH_CHECK("ep_decide_kernel<f64>", st);
     return DSPFE_OK;
 }
 
@@ -207,21 +253,28 @@ int dspfe_endpoint_robust_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, co
     if (rc) return rc;
     const int64_t total = h_offsets[n_utt] - h_offsets[0];
     const cudaStream_t st = pl->stream.get();
-    rc = dspfe_endpoint_robust(pl, pl->d_pcm.get(), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
+    rc = dspfe_endpoint_robust(pl, reinterpret_cast<const int16_t*>(pl->d_pcm.get()), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return DSPFE_OK;
 }
 
-int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
-                        int32_t* h_asum, int32_t* h_zcr, int64_t* h_frame_off) {
+}  // extern "C"
+
+namespace {
+
+// the host-buffer path of either sample type: int16 samples give sum|x| per frame (Stat = int32_t), float32 samples the
+// float64 amplitude (Stat = double)
+template <class T, class Stat>
+int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
+                  Stat* h_stat, int32_t* h_zcr, int64_t* h_frame_off) {
     if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     if (n_utt == 0) return DSPFE_OK;
     const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
     if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
     CUDA_TRY(pl->stream.ensure());
-    int rc = pl->d_pcm.reserve(total + 8);
+    int rc = pl->d_pcm.reserve((total + 8) * (int64_t)sizeof(T));
     if (!rc) rc = pl->d_off.reserve(n_utt + 1);
     if (!rc) rc = pl->d_lr.reserve((int64_t)n_utt * 2);
     if (rc) return rc;
@@ -236,15 +289,31 @@ int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int
     }
     if (h_frame_off) h_frame_off[n_utt] = frames;
     cudaStream_t st = pl->stream.get();
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), h_pcm + base, total * sizeof(int16_t), cudaMemcpyHostToDevice, st));
+    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), h_pcm + base, total * sizeof(T), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    rc = dspfe_endpoint(pl, pl->d_pcm.get(), total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
+    const T* d_pcm = reinterpret_cast<const T*>(pl->d_pcm.get());
+    if constexpr (sizeof(T) == 2) rc = dspfe_endpoint(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
+    else rc = dspfe_endpoint_f32(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (h_asum) CUDA_TRY(cudaMemcpyAsync(h_asum, pl->asum.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (h_stat) CUDA_TRY(cudaMemcpyAsync(h_stat, sizeof(T) == 2 ? (void*)pl->asum.get() : (void*)pl->amp.get(), frames * sizeof(Stat), cudaMemcpyDeviceToHost, st));
     if (h_zcr) CUDA_TRY(cudaMemcpyAsync(h_zcr, pl->zcr.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     return DSPFE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
+                        int32_t* h_asum, int32_t* h_zcr, int64_t* h_frame_off) {
+    return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, h_asum, h_zcr, h_frame_off);
+}
+
+int dspfe_endpoint_host_f32(dspfe_endpoint_plan* pl, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
+                            double* h_amp, int32_t* h_zcr, int64_t* h_frame_off) {
+    return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, h_amp, h_zcr, h_frame_off);
 }
 
 }  // extern "C"

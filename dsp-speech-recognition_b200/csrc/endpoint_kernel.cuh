@@ -11,9 +11,18 @@
 //        NumPy's pairwise summation order so that thresholds, and therefore (left, right), are bit-exact.
 // All statistics are integers, so amp = sum/frame_len (one float64 divide on the host) equals the
 // reference's np.mean exactly.
+//   K2f  float32 samples instead (dspfe_endpoint_f32): the frame statistics in the reference's float64 arithmetic,
+//        amp = np.mean(np.abs(frame)) in NumPy's pairwise order (np_pairwise.h) and the exact sign-change count; K3
+//        then reads the float64 amplitudes (AmpFromF64).  Its body is also compiled onto the test emulator.
 #pragma once
 #include <math.h>
 #include <stdint.h>
+
+#include <vector>
+
+#include "dspfe_types.h"
+#include "np_pairwise.h"
+#include "simt.h"
 
 #ifdef __CUDACC__
 #define DSP_HD __host__ __device__ inline
@@ -217,7 +226,155 @@ struct EpParams {
     int64_t max_blocks, max_frames;
     EpRule rule;
     int32_t* order;            // optional [U]: the utterances by descending frame count (K3r takes them longest first); null = identity
+    const double* amp;         // float-sample path: [F_total] float64 amplitudes written by K2f (K3 reads them instead of asum)
 };
+
+// ---- K2f: frame statistics of float32 samples (basic_endpoint_detection's get_amplitude and get_zcr, endpoint.py:109,182).
+// framesig builds the frames in float64 (the zero padding is float64), so every sample enters as its exact float64 value:
+//   amp[f] = np.mean(np.abs(frame)): the pairwise sum of the L absolute values, then one division by L;
+//   zcr[f] = #{i : x[i] * x[i+1] < 0}: the float64 product of two float32 values is exact and never underflows to zero, so
+//            this is the sign test "both nonzero, opposite signs" (a zero, -0.0 included, never counts; NaN never counts).
+// The split tree of the pairwise sum depends only on L: the plan lays it out once (np_pairwise_tree).  A CTA takes a run of
+// consecutive frames, stages the samples they cover once with 16-byte loads (frames overlap about L / S times), and one
+// thread sums one leaf of one frame with pairwise_block; one thread per frame then adds the leaves in the tree's order.
+constexpr int kEpF32Threads = 256;
+constexpr int kEpF32MaxLen = 8192;        // frame lengths above this are not built (DSPFE_ERR_UNSUPPORTED)
+constexpr int kEpF32SpanFloats = 8192;    // staged samples a run aims at (32 KB)
+
+// The split tree of NumPy's pairwise sum of n terms: nleaf leaves (offset, length) in order, then the nleaf - 1 inner nodes
+// (left, right) in post order, where node k < nleaf is leaf k and node nleaf + j is inner node j.
+inline std::vector<int32_t> np_pairwise_tree(int n, int* nleaf) {
+    std::vector<int32_t> leaves, inner;
+    struct Walk {
+        std::vector<int32_t>& leaves; std::vector<int32_t>& inner;
+        int rec(int off, int len) {           // returns the node id with leaves numbered first (fixed up below)
+            if (len <= kNpPairwiseBlock) { leaves.push_back(off); leaves.push_back(len); return (int)leaves.size() / 2 - 1; }
+            const int n2 = np_pairwise_split(len);
+            const int l = rec(off, n2), r = rec(off + n2, len - n2);
+            inner.push_back(l); inner.push_back(r);
+            return -(int)inner.size() / 2;    // inner node j as -(j + 1)
+        }
+    } w{leaves, inner};
+    w.rec(0, n);
+    const int nl = (int)leaves.size() / 2;
+    for (auto& v : inner) if (v < 0) v = nl + (-v - 1);
+    *nleaf = nl;
+    leaves.insert(leaves.end(), inner.begin(), inner.end());
+    return leaves;
+}
+
+struct EpF32Params {
+    const float* pcm;          // 16-byte aligned
+    int64_t total_samples;
+    const int64_t* offsets;    // [U+1]
+    const int64_t* frame_off;  // [U+1] (ep_prep_kernel)
+    int n_utt;
+    int frame_len, frame_step;
+    const int32_t* tree;       // np_pairwise_tree(frame_len)
+    int nleaf;
+    int run;                   // frames per CTA
+    int span_floats;           // staging capacity, a multiple of 4
+    int sm_fr, sm_zc, sm_tree, sm_span, sm_total;   // shared-memory carve-up in bytes (nodes at 0)
+    int64_t max_frames;
+    double* amp;               // [F_total]
+    int32_t* zcr;              // [F_total]
+};
+
+// frames per CTA and the shared-memory carve-up
+inline void ep_f32_layout(EpF32Params& p) {
+    const int L = p.frame_len, S = p.frame_step, nl = p.nleaf;
+    int run = (kEpF32SpanFloats - L - 4) / S + 1;
+    const int by_tasks = (4 * kEpF32Threads) / nl;
+    if (run > by_tasks) run = by_tasks;
+    if (run < 1) run = 1;
+    p.run = run;
+    p.span_floats = (int)(((int64_t)(run - 1) * S + L + 3 + 3) & ~(int64_t)3);
+    const int node_bytes = run * (2 * nl - 1) * 8;
+    p.sm_fr = node_bytes;                                  // [run] (data start, data end) int64 pairs
+    p.sm_span = (p.sm_fr + run * 16 + 15) & ~15;
+    p.sm_zc = p.sm_span + p.span_floats * 4;
+    p.sm_tree = p.sm_zc + run * nl * 4;
+    p.sm_total = p.sm_tree + (4 * nl - 2) * 4;
+}
+
+// largest u with off[u] <= g
+#ifdef __CUDACC__
+__device__
+#endif
+inline int find_owner(const int64_t* off, int n, int64_t g) {
+    int lo = 0, hi = n;   // off[lo] <= g < off[hi]
+    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (off[mid] <= g) lo = mid; else hi = mid; }
+    return lo;
+}
+
+DEVFN void ep_f32_stats_cta(const EpF32Params& p, unsigned char* smem) {
+    double* s_node = reinterpret_cast<double*>(smem);
+    int64_t* s_fr = reinterpret_cast<int64_t*>(smem + p.sm_fr);
+    float* s_x = reinterpret_cast<float*>(smem + p.sm_span);
+    int32_t* s_zc = reinterpret_cast<int32_t*>(smem + p.sm_zc);
+    int32_t* s_tree = reinterpret_cast<int32_t*>(smem + p.sm_tree);
+    const int tid = simt::tid(), nt = simt::nthreads();
+    const int L = p.frame_len, S = p.frame_step, nl = p.nleaf, nnode = 2 * nl - 1;
+    int64_t F_total = p.frame_off[p.n_utt];
+    if (F_total > p.max_frames) F_total = p.max_frames;
+    const int64_t g0 = (int64_t)simt::bid() * p.run;
+    if (g0 >= F_total) return;                            // uniform over the CTA
+    const int nf = (int)(F_total - g0 < p.run ? F_total - g0 : p.run);
+    for (int i = tid; i < 4 * nl - 2; i += nt) s_tree[i] = p.tree[i];
+    // the samples of frame g: [ds, de) of the packed buffer, with ds <= de <= end of its utterance; both non-decreasing in g
+    for (int f = tid; f < nf; f += nt) {
+        const int64_t g = g0 + f;
+        const int u = find_owner(p.frame_off, p.n_utt, g);
+        const int64_t a = p.offsets[u] + (g - p.frame_off[u]) * S, e = p.offsets[u + 1];
+        s_fr[2 * f] = a < e ? a : e;
+        s_fr[2 * f + 1] = a + L < e ? a + L : e;
+    }
+    simt::cta_sync();
+    const int64_t lo4 = s_fr[0] & ~(int64_t)3, hi = s_fr[2 * nf - 1];
+    const bool staged = hi - lo4 <= p.span_floats;     // a run over many short utterances can cover more: it reads global memory
+    if (staged) {
+        const int nvec = (int)((hi - lo4 + 3) >> 2);
+        for (int v = tid; v < nvec; v += nt) {
+            const int64_t s = lo4 + 4 * (int64_t)v;
+            float4 w;
+            if (s + 4 <= p.total_samples) {
+                w = ldg(reinterpret_cast<const float4*>(p.pcm + s));
+            } else {
+                w.x = s < p.total_samples ? p.pcm[s] : 0.f;
+                w.y = s + 1 < p.total_samples ? p.pcm[s + 1] : 0.f;
+                w.z = s + 2 < p.total_samples ? p.pcm[s + 2] : 0.f;
+                w.w = 0.f;
+            }
+            *reinterpret_cast<float4*>(s_x + 4 * v) = w;
+        }
+    }
+    simt::cta_sync();
+    // one leaf of one frame per thread; samples past the data of the frame are framesig's zero padding
+    for (int t = tid; t < nf * nl; t += nt) {
+        const int f = t / nl, k = t - f * nl;
+        const int64_t ds = s_fr[2 * f];
+        const int avail = (int)(s_fr[2 * f + 1] - ds);
+        const float* x = staged ? s_x + (ds - lo4) : p.pcm + ds;
+        const int o = s_tree[2 * k], n = s_tree[2 * k + 1];
+        s_node[f * nnode + k] = pairwise_block([x, o, avail](int i) { const int j = o + i; return j < avail ? fabs((double)x[j]) : 0.0; }, n);
+        int zc = 0;
+        const int jend = o + n < avail - 1 ? o + n : avail - 1;
+        for (int j = o; j < jend; ++j) {
+            const float a = x[j], b = x[j + 1];
+            zc += ((a < 0.f && b > 0.f) || (a > 0.f && b < 0.f)) ? 1 : 0;
+        }
+        s_zc[t] = zc;
+    }
+    simt::cta_sync();
+    for (int f = tid; f < nf; f += nt) {
+        double* v = s_node + f * nnode;
+        for (int j = 0; j < nl - 1; ++j) v[nl + j] = v[s_tree[2 * nl + 2 * j]] + v[s_tree[2 * nl + 2 * j + 1]];
+        int zc = 0;
+        for (int k = 0; k < nl; ++k) zc += s_zc[f * nl + k];
+        p.amp[g0 + f] = v[nnode - 1] / (double)L;
+        p.zcr[g0 + f] = zc;
+    }
+}
 
 #ifdef __CUDACC__
 constexpr int kEpPrepThreads = 1024;
@@ -278,13 +435,6 @@ __global__ void __launch_bounds__(kEpPrepThreads) ep_prep_kernel(EpParams p) {
             p.order[atomicAdd(&start[F < kEpPrepThreads - 1 ? (int)F : kEpPrepThreads - 1], 1)] = u;
         }
     }
-}
-
-// largest u with off[u] <= g
-__device__ inline int find_owner(const int64_t* off, int n, int64_t g) {
-    int lo = 0, hi = n;   // off[lo] <= g < off[hi]
-    while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (off[mid] <= g) lo = mid; else hi = mid; }
-    return lo;
 }
 
 // K2a: one THREAD per hop block (frame_step samples): the lane streams its own hop with 16-byte loads and keeps the
@@ -378,8 +528,9 @@ constexpr int kEpDecideWarps = 2;
 // amp[i] = sum|x| / frame_len as the reference's float64 mean, computed once per frame by the whole warp: the rule
 // compares every frame against its thresholds several times and a float64 division per comparison on one lane was the
 // kernel's critical path
-__device__ __forceinline__ void ep_stage(const int32_t* asum, const int32_t* zcr, int F, double len, double* s_amp, int32_t* s_zcr, int lane) {
-    for (int i = lane; i < F; i += 32) { s_amp[i] = (double)asum[i] / len; s_zcr[i] = zcr[i]; }
+template <class Amp>
+__device__ __forceinline__ void ep_stage(Amp amp, const int32_t* zcr, int F, double* s_amp, int32_t* s_zcr, int lane) {
+    for (int i = lane; i < F; i += 32) { s_amp[i] = amp(i); s_zcr[i] = zcr[i]; }
     __syncwarp();
 }
 // ---- warp-parallel form of basic_endpoint_detection's decision (endpoint.py:34-66, 133-179, 201-220).
@@ -528,6 +679,13 @@ __device__ __forceinline__ void ep_decide_warp(EpWarpSmem& s, int F, const EpRul
     }
 }
 
+// the utterance's amplitudes from the frame starting at f0: int16 path sum|x| / frame_len (AmpFromSum), float path K2f's float64
+// values (AmpFromF64)
+template <class Amp> __device__ __forceinline__ Amp ep_amp(const EpParams& p, int64_t f0);
+template <> __device__ __forceinline__ AmpFromSum ep_amp<AmpFromSum>(const EpParams& p, int64_t f0) { return AmpFromSum{p.asum + f0, (double)p.frame_len}; }
+template <> __device__ __forceinline__ AmpFromF64 ep_amp<AmpFromF64>(const EpParams& p, int64_t f0) { return AmpFromF64{p.amp + f0}; }
+
+template <class Amp>
 __global__ void __launch_bounds__(32 * kEpDecideWarps) ep_decide_kernel(EpParams p) {
     __shared__ EpWarpSmem s_all[kEpDecideWarps];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -539,11 +697,17 @@ __global__ void __launch_bounds__(32 * kEpDecideWarps) ep_decide_kernel(EpParams
     const EpRule& r = p.rule;
     const int nl = (int)(r.l_sil / r.cfg_step), nr = (int)(r.r_sil / r.cfg_step), zr = (int)(r.zcr_r_sil / r.cfg_step);
     if (F <= kEpStageFrames && nl >= 0 && nr >= 1 && nl + nr <= 32 && zr >= 1 && zr <= 32 && r.zcr_max_shift >= 0.0 && r.cfg_frame > 0.0) {
-        ep_stage(p.asum + f0, p.zcr + f0, F, (double)p.frame_len, s.amp, s.zcr, lane);
+        ep_stage(ep_amp<Amp>(p, f0), p.zcr + f0, F, s.amp, s.zcr, lane);
         ep_decide_warp(s, F, r, lane, p.lr + 2 * u);
     } else if (lane == 0) {
-        endpoint_decide(p.asum + f0, p.zcr + f0, F, p.frame_len, p.rule, p.lr + 2 * u);
+        endpoint_decide_amp(ep_amp<Amp>(p, f0), p.zcr + f0, F, p.rule, p.lr + 2 * u);
     }
+}
+
+// K2f on the device
+__global__ void __launch_bounds__(kEpF32Threads) ep_stats_f32_kernel(const EpF32Params p) {
+    extern __shared__ __align__(16) unsigned char ep_fsm[];
+    ep_f32_stats_cta(p, ep_fsm);
 }
 
 // K3r gate (acr_rule, endpoint.py:142-144), one warp per frame.  The frame is staged in shared memory as float32 (int16

@@ -44,7 +44,7 @@ __global__ void fe_finish_kernel(const FeFinish f) {
 
 struct FeSlot {
     Event h2d_done, compute_done, d2h_done;
-    DeviceArray<int16_t> d_pcm;
+    DeviceArray<unsigned char> d_pcm;    // int16 or float32 samples
     DeviceArray<int64_t> d_rel; PinnedArray<int64_t> h_rel;
     DeviceArray<int32_t> d_lr; DeviceArray<double> d_feat; DeviceArray<int64_t> d_goff[3];
     DeviceArray<float> d_mfcc;
@@ -107,13 +107,38 @@ int create_lane(FeLane& ln, const dspfe_frontend_params& q) {
     return rc;
 }
 
+// The sample types of the batch: int16 (dspfe_frontend*) and float32 (dspfe_frontend*_f32).  A slab starts at the 16-byte
+// aligned sample at or before its first utterance: a multiple of kAlign samples.
+template <class T> struct FeSamples;
+template <> struct FeSamples<int16_t> {
+    static constexpr int kAlign = 8, kDtype = 0;
+    static int endpoint(dspfe_endpoint_plan* p, const int16_t* x, int64_t n, const int64_t* off, int32_t nu, int32_t* lr, cudaStream_t st) {
+        return dspfe_endpoint(p, x, n, off, nu, lr, nullptr, nullptr, nullptr, 0, st);
+    }
+    static int mfcc(dspfe_plan* p, const int16_t* x, int64_t n, const int64_t* off, const int32_t* lr, int32_t nu, float* out, int64_t cap,
+                    int64_t* fo, cudaStream_t st) {
+        return dspfe_mfcc_delta(p, x, n, off, lr, nu, out, cap, fo, st);
+    }
+};
+template <> struct FeSamples<float> {
+    static constexpr int kAlign = 4, kDtype = 1;
+    static int endpoint(dspfe_endpoint_plan* p, const float* x, int64_t n, const int64_t* off, int32_t nu, int32_t* lr, cudaStream_t st) {
+        return dspfe_endpoint_f32(p, x, n, off, nu, lr, nullptr, nullptr, nullptr, 0, st);
+    }
+    static int mfcc(dspfe_plan* p, const float* x, int64_t n, const int64_t* off, const int32_t* lr, int32_t nu, float* out, int64_t cap,
+                    int64_t* fo, cudaStream_t st) {
+        return dspfe_mfcc_delta_f32(p, x, n, off, lr, nu, out, cap, fo, st);
+    }
+};
+
 // the slab's kernels on `st`: endpoints -> MFCC -> cepstrum pitch + pitch_feature -> autocorrelation pitch -> offsets.
 // `wait_prev` (host path): the previous slab's finish kernel, which wrote the running bases this slab's finish kernel reads.
-int run_slab(dspfe_frontend_plan* pl, FeLane& ln, const int16_t* pcm, int64_t total, const int64_t* rel_off, int32_t nu, int32_t* lr,
+template <class T>
+int run_slab(dspfe_frontend_plan* pl, FeLane& ln, const T* pcm, int64_t total, const int64_t* rel_off, int32_t nu, int32_t* lr,
              float* mfcc, int64_t mfcc_cap, double* cep, int32_t* cep_lag, int64_t cep_cap, double* feat, double* acr, int32_t* acr_lag,
              int64_t acr_cap, int64_t* const glob[3], const int64_t base[3], cudaStream_t st, const int64_t* dbase_in = nullptr,
              int64_t* dbase_out = nullptr, int64_t* h_tot = nullptr, cudaEvent_t wait_prev = nullptr) {
-    int rc = dspfe_endpoint(ln.ep.get(), pcm, total, rel_off, nu, lr, nullptr, nullptr, nullptr, 0, st);
+    int rc = FeSamples<T>::endpoint(ln.ep.get(), pcm, total, rel_off, nu, lr, st);
     if (rc) return rc;
     // MFCC, cepstrum pitch and autocorrelation pitch depend on the endpoints only: three branches, so that the single-CTA
     // prefix sums, the latency-bound pitch_feature kernel and the ragged tails of the track kernels of one branch are filled
@@ -131,11 +156,11 @@ int run_slab(dspfe_frontend_plan* pl, FeLane& ln, const int16_t* pcm, int64_t to
         CUDA_TRY(cudaStreamWaitEvent(sa, ln.ev_fork.get(), 0));
         CUDA_TRY(cudaStreamWaitEvent(sb, ln.ev_fork.get(), 0));
     }
-    rc = dspfe_pitch(ln.cep.get(), pcm, 0, total, rel_off, lr, nu, cep, cep_lag, feat, nullptr, ln.loc_off[1].get(), cep_cap, sa);
+    rc = dspfe_pitch(ln.cep.get(), pcm, FeSamples<T>::kDtype, total, rel_off, lr, nu, cep, cep_lag, feat, nullptr, ln.loc_off[1].get(), cep_cap, sa);
     if (rc) return rc;
-    rc = dspfe_pitch(ln.acr.get(), pcm, 0, total, rel_off, lr, nu, acr, acr_lag, nullptr, nullptr, ln.loc_off[2].get(), acr_cap, sb);
+    rc = dspfe_pitch(ln.acr.get(), pcm, FeSamples<T>::kDtype, total, rel_off, lr, nu, acr, acr_lag, nullptr, nullptr, ln.loc_off[2].get(), acr_cap, sb);
     if (rc) return rc;
-    rc = dspfe_mfcc_delta(ln.mf.get(), pcm, total, rel_off, lr, nu, mfcc, mfcc_cap, ln.loc_off[0].get(), st);
+    rc = FeSamples<T>::mfcc(ln.mf.get(), pcm, total, rel_off, lr, nu, mfcc, mfcc_cap, ln.loc_off[0].get(), st);
     if (rc) return rc;
     if (fork) {
         CUDA_TRY(cudaEventRecord(ln.ev_join[0].get(), sa));
@@ -205,8 +230,14 @@ int dspfe_frontend_bounds(const dspfe_frontend_plan* pl, int64_t total_samples, 
     return DSPFE_OK;
 }
 
-int dspfe_frontend(dspfe_frontend_plan* pl, const int16_t* d_pcm, const int64_t* d_offsets, const int64_t* h_off, int32_t n_utt,
-                   const dspfe_frontend_out* o, int64_t* totals, void* stream) {
+}  // extern "C"
+
+namespace {
+
+template <class T>
+int frontend_device(dspfe_frontend_plan* pl, const T* d_pcm, const int64_t* d_offsets, const int64_t* h_off, int32_t n_utt,
+                    const dspfe_frontend_out* o, int64_t* totals, void* stream) {
+    constexpr int64_t kAlign = FeSamples<T>::kAlign;
     if (!pl || !d_offsets || !h_off || !o || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     if (totals) totals[0] = totals[1] = totals[2] = 0;
     if (n_utt == 0) return DSPFE_OK;
@@ -217,7 +248,7 @@ int dspfe_frontend(dspfe_frontend_plan* pl, const int16_t* d_pcm, const int64_t*
     int64_t base[3] = {0, 0, 0};
     for (int32_t u0 = 0; u0 < n_utt;) {
         const int32_t u1 = slab_end(h_off, u0, n_utt, pl->prm.slab_samples), nu = u1 - u0;
-        const int64_t a0 = h_off[u0] & ~(int64_t)7, total = h_off[u1] - a0;
+        const int64_t a0 = h_off[u0] & ~(kAlign - 1), total = h_off[u1] - a0;
         FeLane& ln = pl->lanes[0];
         int rc = DSPFE_OK;
         for (auto& q : ln.loc_off) if (!rc) rc = q.reserve(nu + 1);
@@ -249,8 +280,10 @@ int dspfe_frontend(dspfe_frontend_plan* pl, const int16_t* d_pcm, const int64_t*
     return DSPFE_OK;
 }
 
-int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int64_t* h_off, int32_t n_utt,
-                        const dspfe_frontend_out* o, int64_t* totals) {
+template <class T>
+int frontend_host(dspfe_frontend_plan* pl, const T* h_pcm, const int64_t* h_off, int32_t n_utt, const dspfe_frontend_out* o,
+                  int64_t* totals) {
+    constexpr int64_t kAlign = FeSamples<T>::kAlign;
     if (!pl || !h_off || !o || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     if (totals) totals[0] = totals[1] = totals[2] = 0;
     if (n_utt == 0) return DSPFE_OK;
@@ -278,15 +311,15 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
         cut.push_back(slab_end(h_off, cut.back(), n_utt, cap));
     }
     const int n_slab = (int)cut.size() - 1;
-    const int64_t base0 = h_off[0] & ~(int64_t)7;     // h_pcm is addressed from this sample on (its predecessors are never read)
+    const int64_t base0 = h_off[0] & ~(kAlign - 1);     // h_pcm is addressed from this sample on (its predecessors are never read)
     auto issue_h2d = [&](int s) -> int {
         FeSlot& sl = pl->slots[s % kFeSlots];
         const int32_t u0 = cut[s], u1 = cut[s + 1], nu = u1 - u0;
-        const int64_t a0 = std::max(h_off[u0] & ~(int64_t)7, base0), total = h_off[u1] - a0;
+        const int64_t a0 = std::max(h_off[u0] & ~(kAlign - 1), base0), total = h_off[u1] - a0;
         const cudaStream_t scopy = pl->s_copy.get();
         CUDA_TRY(cudaStreamWaitEvent(scopy, sl.compute_done.get(), 0));            // the slab that used this slot has been processed
         const int64_t n = nu + 1;
-        int rc = sl.d_pcm.reserve(total + 16, pl->prm.host_slab_samples + 16);
+        int rc = sl.d_pcm.reserve((total + 16) * (int64_t)sizeof(T), (pl->prm.host_slab_samples + 16) * (int64_t)sizeof(T));
         if (!rc) rc = sl.d_rel.reserve(n, 1024);
         if (!rc) rc = sl.d_lr.reserve(2 * n, 2 * 1024);
         if (!rc) rc = sl.d_feat.reserve(5 * n, 5 * 1024);
@@ -296,7 +329,7 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
         CUDA_TRY(cudaEventSynchronize(sl.h2d_done.get()));                         // the slot's previous offsets have left h_rel
         for (int32_t i = 0; i <= nu; ++i) sl.h_rel.get()[i] = h_off[u0 + i] - a0;
         // (a0 - base0 .. ) may start before h_off[u0]: those samples belong to the previous utterance and exist in h_pcm
-        if (total > 0) CUDA_TRY(cudaMemcpyAsync(sl.d_pcm.get(), h_pcm + a0, total * sizeof(int16_t), cudaMemcpyHostToDevice, scopy));
+        if (total > 0) CUDA_TRY(cudaMemcpyAsync(sl.d_pcm.get(), h_pcm + a0, total * sizeof(T), cudaMemcpyHostToDevice, scopy));
         CUDA_TRY(cudaMemcpyAsync(sl.d_rel.get(), sl.h_rel.get(), n * sizeof(int64_t), cudaMemcpyHostToDevice, scopy));
         CUDA_TRY(cudaEventRecord(sl.h2d_done.get(), scopy));
         return DSPFE_OK;
@@ -340,7 +373,7 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
     for (int s = 0; s < n_slab; ++s) {
         FeSlot& sl = pl->slots[s % kFeSlots];
         const int32_t u0 = cut[s], u1 = cut[s + 1], nu = u1 - u0;
-        const int64_t a0 = std::max(h_off[u0] & ~(int64_t)7, base0), total = h_off[u1] - a0;
+        const int64_t a0 = std::max(h_off[u0] & ~(kAlign - 1), base0), total = h_off[u1] - a0;
         FeLane& ln = pl->lanes[s % kFeLanes];
         cudaStream_t sc = ln.stream.get();
         const int64_t need0 = dspfe_rows_bound(ln.mf.get(), total, nu), need1 = dspfe_pitch_frames_bound(ln.cep.get(), total, nu),
@@ -355,7 +388,7 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
         if (rc) return rc;
         CUDA_TRY(cudaStreamWaitEvent(sc, sl.h2d_done.get(), 0));
         int64_t* const goff[3] = {sl.d_goff[0].get(), sl.d_goff[1].get(), sl.d_goff[2].get()};
-        rc = run_slab(pl, ln, sl.d_pcm.get(), total, sl.d_rel.get(), nu, sl.d_lr.get(), sl.d_mfcc.get(), need0, sl.d_cep.get(),
+        rc = run_slab(pl, ln, reinterpret_cast<const T*>(sl.d_pcm.get()), total, sl.d_rel.get(), nu, sl.d_lr.get(), sl.d_mfcc.get(), need0, sl.d_cep.get(),
                       o->cep_lag ? sl.d_cep_lag.get() : nullptr, need1, sl.d_feat.get(), sl.d_acr.get(), o->acr_lag ? sl.d_acr_lag.get() : nullptr,
                       need2, goff, zero3, sc, pl->d_base.get() + 3 * (s & 1), pl->d_base.get() + 3 * ((s + 1) & 1),
                       pl->h_tot.get() + 3 * (s % kFeSlots), s > 0 ? pl->lanes[(s - 1) % kFeLanes].finish_done.get() : nullptr);
@@ -370,6 +403,30 @@ int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int
     CUDA_TRY(cudaStreamSynchronize(pl->s_out.get()));
     if (totals) for (int k = 0; k < 3; ++k) totals[k] = base[k];
     return DSPFE_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int dspfe_frontend(dspfe_frontend_plan* pl, const int16_t* d_pcm, const int64_t* d_offsets, const int64_t* h_off, int32_t n_utt,
+                   const dspfe_frontend_out* o, int64_t* totals, void* stream) {
+    return frontend_device(pl, d_pcm, d_offsets, h_off, n_utt, o, totals, stream);
+}
+
+int dspfe_frontend_f32(dspfe_frontend_plan* pl, const float* d_pcm, const int64_t* d_offsets, const int64_t* h_off, int32_t n_utt,
+                       const dspfe_frontend_out* o, int64_t* totals, void* stream) {
+    return frontend_device(pl, d_pcm, d_offsets, h_off, n_utt, o, totals, stream);
+}
+
+int dspfe_frontend_host(dspfe_frontend_plan* pl, const int16_t* h_pcm, const int64_t* h_off, int32_t n_utt,
+                        const dspfe_frontend_out* o, int64_t* totals) {
+    return frontend_host(pl, h_pcm, h_off, n_utt, o, totals);
+}
+
+int dspfe_frontend_host_f32(dspfe_frontend_plan* pl, const float* h_pcm, const int64_t* h_off, int32_t n_utt,
+                            const dspfe_frontend_out* o, int64_t* totals) {
+    return frontend_host(pl, h_pcm, h_off, n_utt, o, totals);
 }
 
 /* ---- per-kernel timing ---- */

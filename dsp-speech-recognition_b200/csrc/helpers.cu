@@ -6,6 +6,7 @@
 
 #include "abi_common.h"
 #include "dspfe_types.h"
+#include "np_pairwise.h"
 #include "pitch_tables.h"
 
 using namespace dspfe;
@@ -30,22 +31,14 @@ __global__ void preemph_kernel(const double* x, int64_t n, double coeff, double*
     y[i] = i == 0 ? x[0] : __dsub_rn(x[i], __dmul_rn(coeff, x[i - 1]));   // product rounded first, as NumPy does (no FMA contraction): bit-exact
 }
 
-// numpy's pairwise sum for any n, evaluated without recursion (explicit stack of pending right halves)
-__device__ double pairwise_block(const double* a, int n, bool absval, bool sq) {
-    auto f = [&](double v) { return sq ? v * v : (absval ? fabs(v) : v); };
-    if (n < 8) { double r = 0.; for (int i = 0; i < n; ++i) r += f(a[i]); return r; }
-    double r0 = f(a[0]), r1 = f(a[1]), r2 = f(a[2]), r3 = f(a[3]), r4 = f(a[4]), r5 = f(a[5]), r6 = f(a[6]), r7 = f(a[7]);
-    int i = 8;
-    for (; i < n - (n % 8); i += 8) {
-        r0 += f(a[i]); r1 += f(a[i + 1]); r2 += f(a[i + 2]); r3 += f(a[i + 3]);
-        r4 += f(a[i + 4]); r5 += f(a[i + 5]); r6 += f(a[i + 6]); r7 += f(a[i + 7]);
-    }
-    double res = ((r0 + r1) + (r2 + r3)) + ((r4 + r5) + (r6 + r7));
-    for (; i < n; ++i) res += f(a[i]);
-    return res;
+// numpy's pairwise sum for any n (np_pairwise.h), evaluated without recursion (explicit stack of pending right halves).
+// The lambdas capture by value: the flags stay loop invariants of the block sum, which the compiler specialises the loop on.
+__device__ double pairwise_block_f64(const double* a, int n, bool absval, bool sq) {
+    auto f = [absval, sq](double v) { return sq ? v * v : (absval ? fabs(v) : v); };
+    return pairwise_block([f, a](int i) { return f(a[i]); }, n);
 }
 __device__ double np_sum_any(const double* a, int n, bool absval, bool sq) {
-    // numpy: n > 128 -> n2 = n/2 rounded down to a multiple of 8; sum(left) + sum(right).  Post-order walk.
+    // post-order walk of the split tree
     struct Item { const double* p; int n; int state; double left; };
     Item st[24];
     int sp = 0;
@@ -53,8 +46,8 @@ __device__ double np_sum_any(const double* a, int n, bool absval, bool sq) {
     double ret = 0.;
     while (sp >= 0) {
         Item& t = st[sp];
-        if (t.n <= 128) { ret = pairwise_block(t.p, t.n, absval, sq); --sp; continue; }
-        int n2 = t.n / 2; n2 -= n2 % 8;
+        if (t.n <= kNpPairwiseBlock) { ret = pairwise_block_f64(t.p, t.n, absval, sq); --sp; continue; }
+        const int n2 = np_pairwise_split(t.n);
         if (t.state == 0) { t.state = 1; st[++sp] = {t.p, n2, 0, 0.}; }
         else if (t.state == 1) { t.left = ret; t.state = 2; st[++sp] = {t.p + n2, t.n - n2, 0, 0.}; }
         else { ret = t.left + ret; --sp; }

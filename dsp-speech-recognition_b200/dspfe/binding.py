@@ -339,6 +339,55 @@ class EndpointPlan:
                                          zcr.ctypes.data_as(ctypes.c_void_p), fo.ctypes.data_as(ctypes.c_void_p)))
         return lr, asum, zcr, fo
 
+    def detect_f32(self, pcm, offsets, want_features=False, stream=None):
+        """Device path on float32 samples (dspfe_endpoint_f32): pcm float32 CUDA tensor, offsets int64 CUDA tensor [U+1].
+        Returns lr int32 [U,2] (and amp float64, zcr int32 [frames_bound], frame_off int64 [U+1] when want_features)."""
+        import torch
+        L = lib(); _bind_endpoint_f32(L)
+        assert pcm.is_cuda and pcm.dtype == torch.float32 and pcm.is_contiguous()
+        assert offsets.is_cuda and offsets.dtype == torch.int64
+        n_utt = offsets.numel() - 1
+        lr = torch.empty((n_utt, 2), dtype=torch.int32, device=pcm.device)
+        st = ctypes.c_void_p(stream if stream is not None else torch.cuda.current_stream(pcm.device).cuda_stream)
+        if not want_features:
+            _check(L.dspfe_endpoint_f32(self._h, pcm.data_ptr(), pcm.numel(), offsets.data_ptr(), n_utt, lr.data_ptr(),
+                                        None, None, None, 0, st))
+            return lr
+        fb = self.frames_bound(pcm.numel(), n_utt)
+        amp = torch.empty(fb, dtype=torch.float64, device=pcm.device)
+        zcr = torch.empty(fb, dtype=torch.int32, device=pcm.device)
+        fo = torch.empty(n_utt + 1, dtype=torch.int64, device=pcm.device)
+        _check(L.dspfe_endpoint_f32(self._h, pcm.data_ptr(), pcm.numel(), offsets.data_ptr(), n_utt, lr.data_ptr(),
+                                    amp.data_ptr(), zcr.data_ptr(), fo.data_ptr(), fb, st))
+        return lr, amp, zcr, fo
+
+    def detect_host_f32(self, pcm, offsets, want_features=False):
+        """Host path on float32 samples: NumPy float32 pcm + int64 offsets -> lr int32 [U,2] (+ amp float64, zcr, frame_off)."""
+        L = lib(); _bind_endpoint_f32(L)
+        pcm = np.ascontiguousarray(pcm, dtype=np.float32)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        n_utt = len(offsets) - 1
+        lr = np.zeros((n_utt, 2), dtype=np.int32)
+        if not want_features:
+            _check(L.dspfe_endpoint_host_f32(self._h, _np_ptr(pcm), _np_ptr(offsets), n_utt, _np_ptr(lr), None, None, None))
+            return lr
+        nf = int(frame_counts(np.diff(offsets), self.frame_len, self.frame_step).sum())
+        amp = np.zeros(nf, dtype=np.float64)
+        zcr = np.zeros(nf, dtype=np.int32)
+        fo = np.zeros(n_utt + 1, dtype=np.int64)
+        _check(L.dspfe_endpoint_host_f32(self._h, _np_ptr(pcm), _np_ptr(offsets), n_utt, _np_ptr(lr), _np_ptr(amp), _np_ptr(zcr),
+                                         _np_ptr(fo)))
+        return lr, amp, zcr, fo
+
+
+def _bind_endpoint_f32(L):
+    if getattr(L, "_ep_f32_bound", False):
+        return
+    vp, i64, i32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32
+    L.dspfe_endpoint_f32.argtypes = [vp, vp, i64, vp, i32, vp, vp, vp, vp, i64, vp]
+    L.dspfe_endpoint_host_f32.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
+    L._ep_f32_bound = True
+
 
 # ------------------------------------------------------------------------------------------------ taps + helpers
 def _bind_helpers(L):
@@ -852,6 +901,8 @@ def _bind_frontend(L):
     L.dspfe_frontend_bounds.argtypes = [vp, i64, i64, vp]
     L.dspfe_frontend.argtypes = [vp, vp, vp, vp, i32, ctypes.POINTER(_FrontendOut), vp, vp]
     L.dspfe_frontend_host.argtypes = [vp, vp, vp, i32, ctypes.POINTER(_FrontendOut), vp]
+    L.dspfe_frontend_f32.argtypes = [vp, vp, vp, vp, i32, ctypes.POINTER(_FrontendOut), vp, vp]
+    L.dspfe_frontend_host_f32.argtypes = [vp, vp, vp, i32, ctypes.POINTER(_FrontendOut), vp]
     L.dspfe_timing_begin.argtypes = [vp]
     L.dspfe_timing_end.argtypes = [vp, vp, i32, ctypes.POINTER(i32)]
     L.dspfe_launch_count.restype = i64
@@ -938,6 +989,30 @@ class FrontendPlan:
         s = self._out_struct(out, lambda t: t.data_ptr() if hasattr(t, "data_ptr") else t.ctypes.data)
         tot = (ctypes.c_int64 * 3)()
         _check(lib().dspfe_frontend_host(self._h, _np_ptr(pcm), _np_ptr(offsets), n_utt, ctypes.byref(s), tot))
+        return tuple(int(t) for t in tot)
+
+    def run_f32(self, pcm, offsets, h_offsets, out, stream=None):
+        """run() on float32 samples (dspfe_frontend_f32): pcm float32 CUDA tensor, the rest as for run()."""
+        import torch
+        assert pcm.is_cuda and pcm.dtype == torch.float32 and pcm.is_contiguous()
+        assert offsets.is_cuda and offsets.dtype == torch.int64 and offsets.is_contiguous()
+        h_offsets = np.ascontiguousarray(h_offsets, dtype=np.int64)
+        n_utt = len(h_offsets) - 1
+        s = self._out_struct(out, lambda t: t.data_ptr())
+        tot = (ctypes.c_int64 * 3)()
+        st = stream if stream is not None else torch.cuda.current_stream(pcm.device).cuda_stream
+        _check(lib().dspfe_frontend_f32(self._h, pcm.data_ptr(), offsets.data_ptr(), _np_ptr(h_offsets), n_utt, ctypes.byref(s), tot,
+                                        ctypes.c_void_p(st)))
+        return tuple(int(t) for t in tot)
+
+    def run_host_f32(self, pcm, offsets, out):
+        """run_host() on float32 samples (dspfe_frontend_host_f32): pcm float32 NumPy array, the rest as for run_host()."""
+        pcm = np.ascontiguousarray(pcm, dtype=np.float32)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        n_utt = len(offsets) - 1
+        s = self._out_struct(out, lambda t: t.data_ptr() if hasattr(t, "data_ptr") else t.ctypes.data)
+        tot = (ctypes.c_int64 * 3)()
+        _check(lib().dspfe_frontend_host_f32(self._h, _np_ptr(pcm), _np_ptr(offsets), n_utt, ctypes.byref(s), tot))
         return tuple(int(t) for t in tot)
 
 

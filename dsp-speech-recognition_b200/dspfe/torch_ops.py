@@ -2,6 +2,7 @@
 custom op taking CUDA tensors"; north_star: "thin C-ABI (ctypes / torch custom-op) layer").
 
     torch.ops.dspfe.endpoint(pcm, offsets, samplerate)                      -> lr int32 [U,2]            (endpoint.py:34)
+                                                                            (int16 or float32 samples)
     torch.ops.dspfe.mfcc_delta(pcm, offsets, trim, samplerate, frame_len, frame_step, nfft, delta_n, preemph, hamming)
                                                                             -> (rows float32 [bound,39], frame_off int64 [U+1])
                                                                                                          (base.py:8, :70; model.py:74-77)
@@ -46,6 +47,8 @@ def _pitch_plan(method, samplerate, frame_len, preemph):
 
 
 def _endpoint_cuda(pcm, offsets, samplerate=16000):
+    if pcm.dtype == torch.float32:
+        return _endpoint_plan(int(samplerate)).detect_f32(pcm.contiguous(), offsets.contiguous())
     return _endpoint_plan(int(samplerate)).detect(pcm.contiguous(), offsets.contiguous())
 
 

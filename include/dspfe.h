@@ -18,7 +18,8 @@
  *     once; dspfe_*_reserve() pre-sizes them so that later calls never allocate;
  *   - a packed ragged batch is int16 PCM `pcm[total_samples]` plus `offsets[n_utt+1]` (int64,
  *     samples); utterance u is pcm[offsets[u] .. offsets[u+1]).  No padding between utterances
- *     is required; `d_pcm` itself must be 16-byte aligned.
+ *     is required; `d_pcm` itself must be 16-byte aligned.  The `_f32` entry points take the same
+ *     layout with float32 samples.
  *   - there is no CPU fallback: without a CUDA device every compute entry point fails with
  *     DSPFE_ERR_CUDA.
  */
@@ -168,6 +169,25 @@ int dspfe_endpoint(dspfe_endpoint_plan* plan, const int16_t* d_pcm, int64_t tota
 /* Host-buffer path: H2D, kernels, D2H; returns when the results are in the host arrays. */
 int dspfe_endpoint_host(dspfe_endpoint_plan* plan, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt,
                         int32_t* h_lr, int32_t* h_asum, int32_t* h_zcr, int64_t* h_frame_off);
+
+/* Float32 samples (a signal already scaled, e.g. what soundfile / torchaudio return in [-1, 1]; model.py:62-63 scales each
+ * utterance before its feature calls): basic_endpoint_detection (endpoint.py:34-66) with the frame statistics in the reference's
+ * float64 arithmetic.  framesig pads with float64 zeros, so every sample enters as its exact float64 value:
+ *   d_amp [frames] float64 = get_amplitude (endpoint.py:109): np.mean(np.abs(frame)) bit for bit, NumPy's pairwise summation
+ *                            order over the frame_len values, then one division by frame_len;
+ *   d_zcr [frames] int32  = get_zcr (endpoint.py:182): neighbours x[i], x[i+1] inside the frame (zero padding included) that
+ *                            are both nonzero and of opposite sign, i.e. x[i] * x[i+1] < 0, which is exact in float64;
+ *   d_lr                  = the same decision rule (K3) on these amplitudes.
+ * Bit-exact against the reference for any float32 input.  d_pcm must be 16-byte aligned; utterance starts need only be
+ * 4-byte aligned.  Optional outputs, validation and error codes as for dspfe_endpoint (max_frames is the capacity of d_amp /
+ * d_zcr).  Frames longer than 8192 samples (int(rate * cfg_frame)) are not built: DSPFE_ERR_UNSUPPORTED.  The float64
+ * amplitude workspace is part of the plan and dspfe_endpoint_reserve pre-sizes it. */
+int dspfe_endpoint_f32(dspfe_endpoint_plan* plan, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets,
+                       int32_t n_utt, int32_t* d_lr, double* d_amp, int32_t* d_zcr, int64_t* d_frame_off,
+                       int64_t max_frames, void* stream);
+/* Host-buffer form: H2D, kernels, D2H; h_amp [frames] float64, h_zcr, h_frame_off optional. */
+int dspfe_endpoint_host_f32(dspfe_endpoint_plan* plan, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt,
+                            int32_t* h_lr, double* h_amp, int32_t* h_zcr, int64_t* h_frame_off);
 
 /* robust_endpoint_detection (endpoint.py:68-92): the same frame statistics, amplitude_rule(mh = 0.5) whose expansion is
  * gated by acr_rule (endpoint.py:142-144: max over lags rate//500 .. rate//50 of acr(frame, n) / acr(frame, 0) > 0.55,
@@ -371,6 +391,14 @@ int dspfe_frontend(dspfe_frontend_plan* plan, const int16_t* d_pcm, const int64_
 /* Host-buffer path: slabs are copied H2D, processed and copied back D2H on three internal streams, overlapped. */
 int dspfe_frontend_host(dspfe_frontend_plan* plan, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt,
                         const dspfe_frontend_out* h_out, int64_t* totals);
+/* The same chain on float32 samples: dspfe_endpoint_f32, dspfe_mfcc_delta_f32 on sig[l:r], dspfe_pitch with sample_dtype 1
+ * for both methods (the cepstrum chain's pre-emphasis included).  Outputs, capacities (dspfe_frontend_bounds) and slabs as
+ * above; d_pcm 16-byte aligned.  A slab starts at the 16-byte aligned sample at or before its first utterance (a multiple
+ * of 4 samples), and host_slab_samples counts samples, so a float slab moves twice the bytes of an int16 one. */
+int dspfe_frontend_f32(dspfe_frontend_plan* plan, const float* d_pcm, const int64_t* d_offsets, const int64_t* h_offsets,
+                       int32_t n_utt, const dspfe_frontend_out* d_out, int64_t* totals, void* stream);
+int dspfe_frontend_host_f32(dspfe_frontend_plan* plan, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt,
+                            const dspfe_frontend_out* h_out, int64_t* totals);
 
 /* ------------------------------------------------------------------------------------------------
  * Per-kernel timing for reports (bench.py): between dspfe_timing_begin(stream) and dspfe_timing_end every kernel the
