@@ -238,10 +238,31 @@ int dspfe_endpoint_robust(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t
     p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off.get(); p.block_off = pl->block_off.get(); p.blk = pl->blk.get();
     p.asum = pl->asum.get(); p.zcr = pl->zcr.get(); p.lr = d_lr; p.max_blocks = 0; p.max_frames = frames_bound; p.rule = pl->rule;
     p.order = pl->order.get();
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    ep_decide_robust_kernel<<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<int16_t>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    ep_decide_robust_kernel<int16_t><<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
     LAUNCH_CHECK("ep_decide_robust_kernel", st);
+    return DSPFE_OK;
+}
+
+int dspfe_endpoint_robust_f32(dspfe_endpoint_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
+                              int32_t* d_lr, void* stream) {
+    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (pl->frame_len > kEpGateMaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "robust endpoint frames longer than 1536 samples are not built");
+    if (n_utt == 0) return DSPFE_OK;
+    // K2f's frame statistics exactly as the basic float path (its own decision is discarded), then the gated rule
+    int rc = dspfe_endpoint_f32(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, nullptr, nullptr, nullptr, 0, stream);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    EpParams p;
+    std::memset(&p, 0, sizeof(p));
+    p.pcm_f32 = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
+    p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off.get(); p.amp = pl->amp.get(); p.zcr = pl->zcr.get(); p.lr = d_lr;
+    p.max_frames = dspfe_endpoint_frames_bound(pl, total_samples, n_utt); p.rule = pl->rule; p.order = pl->order.get();
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<float>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    ep_decide_robust_kernel<float><<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
+    LAUNCH_CHECK("ep_decide_robust_kernel<f32>", st);
     return DSPFE_OK;
 }
 
@@ -264,13 +285,11 @@ int dspfe_endpoint_robust_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, co
 
 namespace {
 
-// the host-buffer path of either sample type: int16 samples give sum|x| per frame (Stat = int32_t), float32 samples the
-// float64 amplitude (Stat = double)
-template <class T, class Stat>
-int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
-                  Stat* h_stat, int32_t* h_zcr, int64_t* h_frame_off) {
-    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
+// stages a host batch on the plan's stream: the samples into d_pcm, the offsets relative to the first into d_off; *total = the
+// sample count, h_frame_off (optional) = the frame prefix sums
+template <class T>
+int stage_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int64_t* h_frame_off, int64_t* total_out,
+               int64_t* frames_out) {
     const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
     if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
     CUDA_TRY(pl->stream.ensure());
@@ -291,6 +310,22 @@ int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offs
     cudaStream_t st = pl->stream.get();
     if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), h_pcm + base, total * sizeof(T), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    *total_out = total;
+    if (frames_out) *frames_out = frames;
+    return DSPFE_OK;
+}
+
+// the host-buffer path of either sample type: int16 samples give sum|x| per frame (Stat = int32_t), float32 samples the
+// float64 amplitude (Stat = double)
+template <class T, class Stat>
+int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
+                  Stat* h_stat, int32_t* h_zcr, int64_t* h_frame_off) {
+    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (n_utt == 0) return DSPFE_OK;
+    int64_t total = 0, frames = 0;
+    int rc = stage_host(pl, h_pcm, h_offsets, n_utt, h_frame_off, &total, &frames);
+    if (rc) return rc;
+    cudaStream_t st = pl->stream.get();
     const T* d_pcm = reinterpret_cast<const T*>(pl->d_pcm.get());
     if constexpr (sizeof(T) == 2) rc = dspfe_endpoint(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
     else rc = dspfe_endpoint_f32(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
@@ -314,6 +349,22 @@ int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int
 int dspfe_endpoint_host_f32(dspfe_endpoint_plan* pl, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
                             double* h_amp, int32_t* h_zcr, int64_t* h_frame_off) {
     return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, h_amp, h_zcr, h_frame_off);
+}
+
+int dspfe_endpoint_robust_host_f32(dspfe_endpoint_plan* pl, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr) {
+    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (pl->frame_len > kEpGateMaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "robust endpoint frames longer than 1536 samples are not built");
+    if (n_utt == 0) return DSPFE_OK;
+    // the batch is staged once; the device form computes the frame statistics once and then runs the gated rule
+    int64_t total = 0;
+    int rc = stage_host(pl, h_pcm, h_offsets, n_utt, nullptr, &total, nullptr);
+    if (rc) return rc;
+    const cudaStream_t st = pl->stream.get();
+    rc = dspfe_endpoint_robust_f32(pl, reinterpret_cast<const float*>(pl->d_pcm.get()), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return DSPFE_OK;
 }
 
 }  // extern "C"

@@ -14,6 +14,8 @@
 //   K2f  float32 samples instead (dspfe_endpoint_f32): the frame statistics in the reference's float64 arithmetic,
 //        amp = np.mean(np.abs(frame)) in NumPy's pairwise order (np_pairwise.h) and the exact sign-change count; K3
 //        then reads the float64 amplitudes (AmpFromF64).  Its body is also compiled onto the test emulator.
+//   K3r  robust_endpoint_detection (endpoint.py:68-92): the rule gated by acr_rule, a CTA per utterance; a template over the sample
+//        type (int16: exact integer lag sums, float32: NumPy's pairwise float64 sums, acr_lag).
 #pragma once
 #include <math.h>
 #include <stdint.h>
@@ -198,6 +200,28 @@ DSP_HD bool acr_gate_frame(const int16_t* x, long long avail, int len, int n0, i
     return any && acr_gate_decide(best, s0, len);
 }
 
+// acr(frame, n) (sigproc.py:48-53) of a float32 frame x[0..avail) with framesig's float64 zero tail up to len samples: NumPy's
+// pairwise float64 sum of the len - n products x[i] x[i+n], divided by len - n; n = 0 is acr(frame, 0).  The product of two
+// float32 values is exact in float64 (it neither overflows nor underflows to zero), so only the order of the sum matters, and
+// every lag has its own split tree.  Shared by the serial gate below and the exact fallback of K3r's float gate.
+DSP_HD double acr_lag(const float* x, int avail, int len, int n) {
+    const double s = np_pairwise_sum_any([x, avail, n](int i) { return i + n < avail ? (double)x[i] * (double)x[i + n] : 0.0; }, len - n);
+    return s / (double)(len - n);
+}
+// acr_rule of a float32 frame, serial.  A NaN or +-inf sample makes acr(frame, 0) NaN or +inf, and every ratio NaN, 0 or
+// NaN / inf: the gate is false.  An all-zero frame gives 0 / 0, false as well.
+DSP_HD bool acr_gate_frame(const float* x, long long avail, int len, int n0, int n1) {
+    const int nv = avail < (long long)len ? (avail > 0 ? (int)avail : 0) : len;
+    const double a0 = acr_lag(x, nv, len, 0);
+    if (!isfinite(a0)) return false;
+    double best = 0.0; bool any = false;
+    for (int n = n0; n < n1 && n < len; ++n) {
+        const double a = acr_lag(x, nv, len, n);
+        if (!any || a > best) { best = a; any = true; }
+    }
+    return any && best / a0 > 0.55;
+}
+
 // robust_endpoint_detection (endpoint.py:68-92): amplitude_rule(mh = 0.5) with the gate, zcr_rule, whole-signal fallback
 template <class Amp, class Gate>
 DSP_HD void endpoint_decide_robust(Amp amp, const int32_t* zcr, int F, const EpRule& r, Gate gate, int32_t* out_lr) {
@@ -227,6 +251,7 @@ struct EpParams {
     EpRule rule;
     int32_t* order;            // optional [U]: the utterances by descending frame count (K3r takes them longest first); null = identity
     const double* amp;         // float-sample path: [F_total] float64 amplitudes written by K2f (K3 reads them instead of asum)
+    const float* pcm_f32;      // float-sample path: the samples K3r's gate reads instead of pcm
 };
 
 // ---- K2f: frame statistics of float32 samples (basic_endpoint_detection's get_amplitude and get_zcr, endpoint.py:109,182).
@@ -765,6 +790,39 @@ __device__ __forceinline__ int warp_arg_of_max(double v, double vmax, int n, int
     const unsigned m = __ballot_sync(0xffffffffu, v == vmax);
     return __shfl_sync(0xffffffffu, n, m ? __ffs((int)m) - 1 : 0);
 }
+// The probe and the float32 screening of a staged frame (exact staged values, a0 = acr(frame, 0) of them): 1 / 0 the gate is
+// settled, -1 probe_only and not settled, 2 the ratio lies within delta of 0.55 and the exact sums must decide.
+__device__ __forceinline__ int gate_screen(const float* sx, int len, int n0, int nl, double a0, int lane, int& pred, bool probe_only) {
+    const double delta = 1.5 * (double)len * 5.9604644775390625e-08 * (double)len / (double)(len - (n0 + nl - 1));
+    int bn;
+    if (delta < 0.01) {
+        if (pred >= 0 && nl >= 32) {
+            int p0 = pred - 16;
+            p0 = p0 < n0 ? n0 : (p0 > n0 + nl - 32 ? n0 + nl - 32 : p0);
+            const int n = p0 + lane;
+            float acc[8];
+#pragma unroll
+            for (int u = 0; u < 8; ++u) acc[u] = 0.f;
+            for (int i = 0; i < len - p0; i += 8) {      // terms past the frame (i + n >= len) multiply the zero tail
+                const float4 a0v = *reinterpret_cast<const float4*>(sx + i), a1v = *reinterpret_cast<const float4*>(sx + i + 4);
+                const float av[8] = {a0v.x, a0v.y, a0v.z, a0v.w, a1v.x, a1v.y, a1v.z, a1v.w};
+#pragma unroll
+                for (int u = 0; u < 8; ++u) acc[u] = fmaf(av[u], sx[i + n + u], acc[u]);
+            }
+            const float sn = ((acc[0] + acc[1]) + (acc[2] + acc[3])) + ((acc[4] + acc[5]) + (acc[6] + acc[7]));
+            const double r = (double)(sn / (float)(len - n));
+            const double rmax = warp_max_f64(r);
+            if (rmax / a0 > 0.55 + delta) { pred = warp_arg_of_max(r, rmax, n, lane); return 1; }
+        }
+        if (probe_only) return -1;
+        const double bf = (double)gate_best<float>(sx, len, n0, nl, lane, bn);
+        const double bmax = warp_max_f64(bf);
+        const double ratio = bmax / a0;
+        if (ratio > 0.55 + delta) { pred = warp_arg_of_max(bf, bmax, bn, lane); return 1; }
+        if (ratio < 0.55 - delta) return 0;
+    } else if (probe_only) return -1;
+    return 2;
+}
 // The gate of the frame starting at sample b of the utterance x[0..S); warp-uniform result.  `pred` (in): a lag at which the
 // neighbouring frame's autocorrelation peaked, or -1; (out) this frame's peak lag when the gate holds.
 // With a prediction the warp first PROBES the 32 lags around it, one lag per lane: the rule only asks whether SOME lag exceeds
@@ -804,37 +862,88 @@ __device__ int gate_frame_warp(const int16_t* x, long long S, long long b, int l
     for (int m = 16; m >= 1; m >>= 1) s0i += __shfl_xor_sync(0xffffffffu, s0i, m);
     if (s0i == 0) return 0;                              // 0 / 0 = NaN compares false, as in the reference
     const double a0 = (double)s0i / (double)len;
-    const double delta = 1.5 * (double)len * 5.9604644775390625e-08 * (double)len / (double)(len - (n0 + nl - 1));
+    const int g = gate_screen(sx, len, n0, nl, a0, lane, pred, probe_only);
+    if (g != 2) return g;
     int bn;
-    if (delta < 0.01) {
-        if (pred >= 0 && nl >= 32) {
-            int p0 = pred - 16;
-            p0 = p0 < n0 ? n0 : (p0 > n0 + nl - 32 ? n0 + nl - 32 : p0);
-            const int n = p0 + lane;
-            float acc[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) acc[u] = 0.f;
-            for (int i = 0; i < len - p0; i += 8) {      // terms past the frame (i + n >= len) multiply the zero tail
-                const float4 a0v = *reinterpret_cast<const float4*>(sx + i), a1v = *reinterpret_cast<const float4*>(sx + i + 4);
-                const float av[8] = {a0v.x, a0v.y, a0v.z, a0v.w, a1v.x, a1v.y, a1v.z, a1v.w};
-#pragma unroll
-                for (int u = 0; u < 8; ++u) acc[u] = fmaf(av[u], sx[i + n + u], acc[u]);
-            }
-            const float sn = ((acc[0] + acc[1]) + (acc[2] + acc[3])) + ((acc[4] + acc[5]) + (acc[6] + acc[7]));
-            const double r = (double)(sn / (float)(len - n));
-            const double rmax = warp_max_f64(r);
-            if (rmax / a0 > 0.55 + delta) { pred = warp_arg_of_max(r, rmax, n, lane); return 1; }
-        }
-        if (probe_only) return -1;
-        const double bf = (double)gate_best<float>(sx, len, n0, nl, lane, bn);
-        const double bmax = warp_max_f64(bf);
-        const double ratio = bmax / a0;
-        if (ratio > 0.55 + delta) { pred = warp_arg_of_max(bf, bmax, bn, lane); return 1; }
-        if (ratio < 0.55 - delta) return 0;
-    } else if (probe_only) return -1;
     const double bd = gate_best<double>(sx, len, n0, nl, lane, bn);
     const double dmax = warp_max_f64(bd);
     if (dmax / a0 > 0.55) { pred = warp_arg_of_max(bd, dmax, bn, lane); return 1; }   // acr_gate_decide on exact sums
+    return 0;
+}
+
+// The same gate on float32 samples (x: the utterance, 4-byte aligned).  framesig's frame is float64 and every float32 sample
+// enters it exactly, so acr(frame, n) is NumPy's pairwise float64 sum of exact products (acr_lag):
+//   * the frame is staged with its zero tail, through 16-byte loads when x + b is 16-byte aligned; a NaN or +-inf sample
+//     makes the gate false (acr_gate_frame), an all-zero frame too;
+//   * a0 = acr(frame, 0) exactly (acr_lag on the staged, unscaled values);
+//   * the staged frame is then scaled by 2^k so that max|x| lies in [1, 2).  The ratio is invariant under power-of-two scaling
+//     and the screening's float32 sums neither overflow (above max|x| ~ 1.8e19 they would) nor underflow (quiet input near 1e-20
+//     would flush to zero and void the bound).  The probe and the screening then run unchanged with the same delta: its
+//     derivation only needs the staged values exact.  Scaling down may round samples below 2^-126 max|x| to subnormals, and the
+//     float32 sums may run through subnormals: at most about k 2^-149 on lag sums with a0 >= 1 / len, negligible against delta;
+//   * the exact fallback is acr_lag per lag (one lane per lag, unscaled samples from x), a warp max and the 0.55 test.  The
+//     chunked float64 FMA order of gate_best<double> is exact for int16 samples only.
+__device__ int gate_frame_warp(const float* x, long long S, long long b, int len, int n0, int n1, float* sx, int lane, int& pred, bool probe_only) {
+    __syncwarp();
+    const int nv = (int)(S - b < (long long)len ? (S - b > 0 ? S - b : 0) : (long long)len);      // samples of the frame that exist
+    const float* xb = x + b;
+    const int nvec = (len + kGatePad + 3) >> 2;          // the staging area holds kEpGateMaxLen + kGatePad floats, a multiple of 4
+    float mx = 0.f;
+    bool bad = false;
+    if ((reinterpret_cast<uintptr_t>(xb) & 15) == 0) {
+        for (int v = lane; v < nvec; v += 32) {
+            const int i = 4 * v;
+            float4 w;
+            if (i + 3 < nv) {
+                w = __ldg(reinterpret_cast<const float4*>(xb) + v);
+            } else {
+                w.x = i < nv ? xb[i] : 0.f; w.y = i + 1 < nv ? xb[i + 1] : 0.f;
+                w.z = i + 2 < nv ? xb[i + 2] : 0.f; w.w = i + 3 < nv ? xb[i + 3] : 0.f;
+            }
+            *reinterpret_cast<float4*>(sx + i) = w;
+            const float m = fmaxf(fmaxf(fabsf(w.x), fabsf(w.y)), fmaxf(fabsf(w.z), fabsf(w.w)));
+            bad |= !(isfinite(w.x) && isfinite(w.y) && isfinite(w.z) && isfinite(w.w));
+            mx = fmaxf(mx, m);
+        }
+    } else {
+        for (int i = lane; i < 4 * nvec; i += 32) {
+            const float v = i < nv ? xb[i] : 0.f;
+            sx[i] = v;
+            bad |= !isfinite(v);
+            mx = fmaxf(mx, fabsf(v));
+        }
+    }
+    const int nl = (n1 < len ? n1 : len) - n0;           // lags n0 .. n0 + nl - 1
+    if (nl <= 0 || __any_sync(0xffffffffu, bad)) return 0;
+#pragma unroll
+    for (int m = 16; m >= 1; m >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, m));
+    if (mx == 0.f) return 0;                             // 0 / 0 = NaN compares false, as in the reference
+    __syncwarp();
+    const double a0 = acr_lag(sx, nv, len, 0);
+    int e;
+    frexpf(mx, &e);
+    const int k = 1 - e;                                 // mx 2^k in [1, 2)
+    __syncwarp();
+    if ((reinterpret_cast<uintptr_t>(xb) & 15) == 0) {
+        for (int i = 4 * lane; i < 4 * nvec; i += 128) {
+            float4 w = *reinterpret_cast<float4*>(sx + i);
+            w.x = ldexpf(w.x, k); w.y = ldexpf(w.y, k); w.z = ldexpf(w.z, k); w.w = ldexpf(w.w, k);
+            *reinterpret_cast<float4*>(sx + i) = w;
+        }
+    } else {
+        for (int i = lane; i < 4 * nvec; i += 32) sx[i] = ldexpf(sx[i], k);
+    }
+    __syncwarp();
+    const int g = gate_screen(sx, len, n0, nl, ldexp(a0, 2 * k), lane, pred, probe_only);   // a0 of the scaled frame, exact
+    if (g != 2) return g;
+    double bd = -INFINITY;
+    int bn = n0;
+    for (int n = n0 + lane; n < n0 + nl; n += 32) {
+        const double a = acr_lag(xb, nv, len, n);
+        if (a > bd) { bd = a; bn = n; }
+    }
+    const double dmax = warp_max_f64(bd);
+    if (dmax / a0 > 0.55) { pred = warp_arg_of_max(bd, dmax, bn, lane); return 1; }
     return 0;
 }
 
@@ -848,8 +957,8 @@ constexpr int kEpRobustWarps = 4;     // (8 warps: 1.56 -> 1.80 ms with probe-on
 struct GateRequest { int j, dir, pred, done; double m_l; double pad; };      // 32 bytes: the staging areas behind it stay 16-byte aligned
 __device__ __forceinline__ void robust_bar(int id) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(32 * kEpRobustWarps) : "memory"); }
 // one window: warp w evaluates frame j + dir * w when the walk can reach it
-template <class Amp>
-__device__ __forceinline__ int gate_window_warp(const GateRequest& q, const int16_t* x, long long S, int step, int len, int n0, int n1, int F,
+template <class T, class Amp>
+__device__ __forceinline__ int gate_window_warp(const GateRequest& q, const T* x, long long S, int step, int len, int n0, int n1, int F,
                                                 Amp amp, float* sx, int w, int lane) {
     const int fj = q.j + q.dir * w;
     bool want = q.dir < 0 ? fj >= 1 : fj < F;
@@ -862,9 +971,9 @@ __device__ __forceinline__ int gate_window_warp(const GateRequest& q, const int1
     }
     return res | ((lag < 0 ? 0 : lag) << 2);
 }
-template <class Amp>
+template <class T, class Amp>
 struct GateCta {           // lives in warp 0
-    const int16_t* x; long long S; int step, len, n0, n1, F;
+    const T* x; long long S; int step, len, n0, n1, F;
     Amp amp; float* sx; int* s_res; GateRequest* req;
     int dir; double m_l; int win_base, win_dir, win_known, win_val;
     int pred;                              // the peak lag of the last frame whose gate held (the probe's centre), -1: none yet
@@ -888,13 +997,13 @@ struct GateCta {           // lives in warp 0
         return win_val & 1;
     }
 };
-template <class Amp>
-__device__ __forceinline__ void robust_cta(const EpParams& p, Amp amp, const int32_t* zcr, int F, const int16_t* x, long long S, float* s_x, int* s_res,
+template <class T, class Amp>
+__device__ __forceinline__ void robust_cta(const EpParams& p, Amp amp, const int32_t* zcr, int F, const T* x, long long S, float* s_x, int* s_res,
                                            GateRequest* req, int u) {
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n0 = p.rule.rate / 500, n1 = p.rule.rate / 50;
     if (w == 0) {
-        GateCta<Amp> gate{x, S, p.frame_step, p.frame_len, n0, n1, F, amp, s_x, s_res, req, -1, 0.0, 0, 1, 0, 0, -1};
+        GateCta<T, Amp> gate{x, S, p.frame_step, p.frame_len, n0, n1, F, amp, s_x, s_res, req, -1, 0.0, 0, 1, 0, 0, -1};
         int32_t lr[2];
         endpoint_decide_robust(amp, zcr, F, p.rule, gate, lr);
         if (lane == 0) { req->done = 1; p.lr[2 * u] = lr[0]; p.lr[2 * u + 1] = lr[1]; }
@@ -910,6 +1019,20 @@ __device__ __forceinline__ void robust_cta(const EpParams& p, Amp amp, const int
     }
 }
 
+// what K3r reads for each sample type: the samples its gate stages (int16: p.pcm, float32: p.pcm_f32) and the frame amplitudes
+// (int16: K2b's sums / frame_len, float32: K2f's float64 values), one frame g at a time or as the source Amp of an utterance
+template <class T> struct EpSamples;
+template <> struct EpSamples<int16_t> {
+    using Amp = AmpFromSum;
+    static __device__ __forceinline__ const int16_t* pcm(const EpParams& p) { return p.pcm; }
+    static __device__ __forceinline__ double amp(const EpParams& p, int64_t g) { return (double)p.asum[g] / (double)p.frame_len; }
+};
+template <> struct EpSamples<float> {
+    using Amp = AmpFromF64;
+    static __device__ __forceinline__ const float* pcm(const EpParams& p) { return p.pcm_f32; }
+    static __device__ __forceinline__ double amp(const EpParams& p, int64_t g) { return p.amp[g]; }
+};
+template <class T>
 __global__ void __launch_bounds__(32 * kEpRobustWarps, 6) ep_decide_robust_kernel(EpParams p) {
     extern __shared__ __align__(16) unsigned char ep_rsm[];
     double* s_amp = reinterpret_cast<double*>(ep_rsm);                                   // [kEpStageFrames]
@@ -921,14 +1044,14 @@ __global__ void __launch_bounds__(32 * kEpRobustWarps, 6) ep_decide_robust_kerne
     const int u = p.order ? p.order[blockIdx.x] : (int)blockIdx.x;
     const int64_t f0 = p.frame_off[u];
     const int F = (int)(p.frame_off[u + 1] - f0);
-    const int16_t* x = p.pcm + p.offsets[u];
+    const T* x = EpSamples<T>::pcm(p) + p.offsets[u];
     const long long S = (long long)(p.offsets[u + 1] - p.offsets[u]);
     if (F <= kEpStageFrames) {
-        for (int i = threadIdx.x; i < F; i += blockDim.x) { s_amp[i] = (double)p.asum[f0 + i] / (double)p.frame_len; s_zcr[i] = p.zcr[f0 + i]; }
+        for (int i = threadIdx.x; i < F; i += blockDim.x) { s_amp[i] = EpSamples<T>::amp(p, f0 + i); s_zcr[i] = p.zcr[f0 + i]; }
         __syncthreads();
         robust_cta(p, AmpFromF64{s_amp}, s_zcr, F, x, S, s_x, s_res, req, u);
     } else {
-        robust_cta(p, AmpFromSum{p.asum + f0, (double)p.frame_len}, p.zcr + f0, F, x, S, s_x, s_res, req, u);
+        robust_cta(p, ep_amp<typename EpSamples<T>::Amp>(p, f0), p.zcr + f0, F, x, S, s_x, s_res, req, u);
     }
 }
 constexpr int kEpRobustSmem = kEpStageFrames * 12 + kEpRobustWarps * 4 + (int)sizeof(GateRequest) + kEpRobustWarps * (kEpGateMaxLen + kGatePad) * 4;

@@ -38,21 +38,7 @@ __device__ double pairwise_block_f64(const double* a, int n, bool absval, bool s
     return pairwise_block([f, a](int i) { return f(a[i]); }, n);
 }
 __device__ double np_sum_any(const double* a, int n, bool absval, bool sq) {
-    // post-order walk of the split tree
-    struct Item { const double* p; int n; int state; double left; };
-    Item st[24];
-    int sp = 0;
-    st[0] = {a, n, 0, 0.};
-    double ret = 0.;
-    while (sp >= 0) {
-        Item& t = st[sp];
-        if (t.n <= kNpPairwiseBlock) { ret = pairwise_block_f64(t.p, t.n, absval, sq); --sp; continue; }
-        const int n2 = np_pairwise_split(t.n);
-        if (t.state == 0) { t.state = 1; st[++sp] = {t.p, n2, 0, 0.}; }
-        else if (t.state == 1) { t.left = ret; t.state = 2; st[++sp] = {t.p + n2, t.n - n2, 0, 0.}; }
-        else { ret = t.left + ret; --sp; }
-    }
-    return ret;
+    return pairwise_walk(a, n, [absval, sq](const double* p, int m) { return pairwise_block_f64(p, m, absval, sq); });
 }
 
 // get_amplitude (endpoint.py:109-126, window='square'): mean |x| (or x^2) per frame, numpy summation order

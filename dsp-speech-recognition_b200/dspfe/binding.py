@@ -379,6 +379,28 @@ class EndpointPlan:
                                          _np_ptr(fo)))
         return lr, amp, zcr, fo
 
+    def detect_robust_f32(self, pcm, offsets, stream=None):
+        """robust_endpoint_detection (reference endpoint.py:68) on float32 samples (dspfe_endpoint_robust_f32): pcm float32 CUDA
+        tensor, offsets int64 CUDA tensor [U+1].  Returns lr int32 [U,2]."""
+        import torch
+        L = lib(); _bind_endpoint_f32(L)
+        assert pcm.is_cuda and pcm.dtype == torch.float32 and pcm.is_contiguous()
+        assert offsets.is_cuda and offsets.dtype == torch.int64
+        n_utt = offsets.numel() - 1
+        lr = torch.empty((n_utt, 2), dtype=torch.int32, device=pcm.device)
+        st = ctypes.c_void_p(stream if stream is not None else torch.cuda.current_stream(pcm.device).cuda_stream)
+        _check(L.dspfe_endpoint_robust_f32(self._h, pcm.data_ptr(), pcm.numel(), offsets.data_ptr(), n_utt, lr.data_ptr(), st))
+        return lr
+
+    def detect_robust_host_f32(self, pcm, offsets):
+        """Host form of detect_robust_f32: NumPy float32 pcm + int64 offsets -> lr int32 [U,2]."""
+        L = lib(); _bind_endpoint_f32(L)
+        pcm = np.ascontiguousarray(pcm, dtype=np.float32)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        lr = np.zeros((len(offsets) - 1, 2), dtype=np.int32)
+        _check(L.dspfe_endpoint_robust_host_f32(self._h, _np_ptr(pcm), _np_ptr(offsets), len(offsets) - 1, _np_ptr(lr)))
+        return lr
+
 
 def _bind_endpoint_f32(L):
     if getattr(L, "_ep_f32_bound", False):
@@ -386,6 +408,8 @@ def _bind_endpoint_f32(L):
     vp, i64, i32 = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int32
     L.dspfe_endpoint_f32.argtypes = [vp, vp, i64, vp, i32, vp, vp, vp, vp, i64, vp]
     L.dspfe_endpoint_host_f32.argtypes = [vp, vp, vp, i32, vp, vp, vp, vp]
+    L.dspfe_endpoint_robust_f32.argtypes = [vp, vp, i64, vp, i32, vp, vp]
+    L.dspfe_endpoint_robust_host_f32.argtypes = [vp, vp, vp, i32, vp]
     L._ep_f32_bound = True
 
 

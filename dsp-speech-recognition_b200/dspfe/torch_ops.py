@@ -3,6 +3,8 @@ custom op taking CUDA tensors"; north_star: "thin C-ABI (ctypes / torch custom-o
 
     torch.ops.dspfe.endpoint(pcm, offsets, samplerate)                      -> lr int32 [U,2]            (endpoint.py:34)
                                                                             (int16 or float32 samples)
+    torch.ops.dspfe.endpoint_robust(pcm, offsets, samplerate)               -> lr int32 [U,2]            (endpoint.py:68)
+                                                                            (int16 or float32 samples)
     torch.ops.dspfe.mfcc_delta(pcm, offsets, trim, samplerate, frame_len, frame_step, nfft, delta_n, preemph, hamming)
                                                                             -> (rows float32 [bound,39], frame_off int64 [U+1])
                                                                                                          (base.py:8, :70; model.py:74-77)
@@ -24,6 +26,7 @@ from . import binding
 
 _lib = torch.library.Library("dspfe", "DEF")
 _lib.define("endpoint(Tensor pcm, Tensor offsets, int samplerate=16000) -> Tensor")
+_lib.define("endpoint_robust(Tensor pcm, Tensor offsets, int samplerate=16000) -> Tensor")
 _lib.define("mfcc_delta(Tensor pcm, Tensor offsets, Tensor? trim=None, int samplerate=16000, int frame_len=400, int frame_step=160, "
             "int nfft=512, int delta_n=2, float preemph=0.97, bool hamming=False) -> (Tensor, Tensor)")
 _lib.define("pitch(Tensor pcm, Tensor offsets, Tensor? trim=None, int method=0, int samplerate=16000, int frame_len=512, "
@@ -52,6 +55,12 @@ def _endpoint_cuda(pcm, offsets, samplerate=16000):
     return _endpoint_plan(int(samplerate)).detect(pcm.contiguous(), offsets.contiguous())
 
 
+def _endpoint_robust_cuda(pcm, offsets, samplerate=16000):
+    if pcm.dtype == torch.float32:
+        return _endpoint_plan(int(samplerate)).detect_robust_f32(pcm.contiguous(), offsets.contiguous())
+    return _endpoint_plan(int(samplerate)).detect_robust(pcm.contiguous(), offsets.contiguous())
+
+
 def _mfcc_cuda(pcm, offsets, trim=None, samplerate=16000, frame_len=400, frame_step=160, nfft=512, delta_n=2, preemph=0.97, hamming=False):
     plan = _mfcc_plan(int(samplerate), int(frame_len), int(frame_step), int(nfft), int(delta_n), float(preemph), bool(hamming))
     t = None if trim is None else trim.contiguous()
@@ -67,12 +76,18 @@ def _pitch_cuda(pcm, offsets, trim=None, method=0, samplerate=16000, frame_len=5
 
 
 _lib.impl("endpoint", _endpoint_cuda, "CUDA")
+_lib.impl("endpoint_robust", _endpoint_robust_cuda, "CUDA")
 _lib.impl("mfcc_delta", _mfcc_cuda, "CUDA")
 _lib.impl("pitch", _pitch_cuda, "CUDA")
 
 
 # shape-only implementations: the row / frame bounds of the plans depend on sizes alone
 @torch.library.register_fake("dspfe::endpoint")
+def _(pcm, offsets, samplerate=16000):
+    return pcm.new_empty((offsets.shape[0] - 1, 2), dtype=torch.int32)
+
+
+@torch.library.register_fake("dspfe::endpoint_robust")
 def _(pcm, offsets, samplerate=16000):
     return pcm.new_empty((offsets.shape[0] - 1, 2), dtype=torch.int32)
 

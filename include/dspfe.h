@@ -195,6 +195,16 @@ int dspfe_endpoint_host_f32(dspfe_endpoint_plan* plan, const float* h_pcm, const
 int dspfe_endpoint_robust(dspfe_endpoint_plan* plan, const int16_t* d_pcm, int64_t total_samples, const int64_t* d_offsets,
                           int32_t n_utt, int32_t* d_lr, void* stream);
 int dspfe_endpoint_robust_host(dspfe_endpoint_plan* plan, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr);
+/* robust_endpoint_detection (endpoint.py:68-92) on float32 samples: the frame statistics of dspfe_endpoint_f32, then the gated
+ * rule with acr_rule evaluated in the reference's float64 arithmetic.  acr(frame, n) (sigproc.py:48-53) is NumPy's pairwise
+ * sum of the len - n exact products x[i] x[i+n] divided by len - n, every lag with its own split tree; the gate is
+ * max_n acr(n) / acr(0) > 0.55 over the lags rate//500 .. rate//50 below the frame length.  A frame holding a NaN or +-inf
+ * sample, and an all-zero frame, fail the gate, as in the reference.  Bit-exact against the reference for any float32 input.
+ * Frames longer than 1536 samples are not built: DSPFE_ERR_UNSUPPORTED.  d_pcm must be 16-byte aligned; validation and the
+ * other error codes as for dspfe_endpoint_f32.  The host form stages the batch once and computes its statistics once. */
+int dspfe_endpoint_robust_f32(dspfe_endpoint_plan* plan, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets,
+                              int32_t n_utt, int32_t* d_lr, void* stream);
+int dspfe_endpoint_robust_host_f32(dspfe_endpoint_plan* plan, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr);
 /* List form of amplitude_rule(use_acr=True) (endpoint.py:133): gate[n_frames] (0/1) is acr_rule of every frame, which
  * dspfe_acr_gate_rows_f64 computes on the device for a float64 frame matrix [n_rows, len]. */
 int dspfe_amplitude_rule_gated_host(const dspfe_endpoint_params* p, const double* amp, const int32_t* gate, int32_t n_frames, double mh,
