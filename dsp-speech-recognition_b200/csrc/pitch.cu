@@ -125,6 +125,24 @@ __global__ void __launch_bounds__(32 * kPitchWarps, MODE == 1 ? 3 : 4) pitch_fra
     else pitch_fft_pair<(MODE == 2 ? 1 : MODE)>(p, h0, g0, nvalid > 1, smem + kTabMod * 8 + w * kWarpSmemBytes, tws, tws + kTabW32);
 }
 
+// K4a-2 for cepstrum frames of 100..511 samples: the N-point DFTs by Bluestein's chirp (12 transforms per pair), a frame pair per
+// warp in the slot space of pitch_frame_kernel<0>
+__global__ void __launch_bounds__(32 * kPitchWarps, 3) pitch_cep_bluestein_kernel(const __grid_constant__ PitchParams p) {
+    extern __shared__ __align__(16) unsigned char smem[];
+    float2* tws = reinterpret_cast<float2*>(smem);                       // W512 twiddles + W32 (kTabMod float2)
+    const int64_t total = p.slot_off[p.n_utt];
+    if (2 * (int64_t)blockIdx.x * kPitchWarps >= total) return;         // surplus CTAs leave before touching the tables
+    for (int i = threadIdx.x; i < kTabMod; i += blockDim.x) tws[i] = p.tab[i];
+    __syncthreads();
+    const int w = threadIdx.x >> 5;
+    const int64_t h0 = 2 * ((int64_t)blockIdx.x * kPitchWarps + w);
+    if (h0 >= total) return;   // whole warp leaves; only warp-level syncs below
+    int nvalid; int64_t g0;
+    slot_unit_from_desc(p, h0, 2, g0, nvalid);
+    if (nvalid == 0) return;   // padding slots at the end of an utterance
+    pitch_cep_bluestein_pair(p, h0, g0, nvalid > 1, smem + kTabMod * 8 + w * kWarpSmemBytes, tws, tws + kTabW32);
+}
+
 __global__ void __launch_bounds__(kTrackThreads) pitch_track_kernel(const __grid_constant__ PitchParams p) {
     extern __shared__ __align__(16) unsigned char smem[];
     float* chunk = reinterpret_cast<float*>(smem);
@@ -259,13 +277,14 @@ int dspfe_pitch_create(const dspfe_pitch_params* q, dspfe_pitch_plan** plan) {
     std::string err;
     const int trc = build_pitch_tables(*q, b, tab, err);
     if (trc) { delete pl; return fail(trc, err); }
-    if (int rc = pl->d_tab.reserve(kTabTotal)) { delete pl; return rc; }
-    cudaError_t e = cudaMemcpy(pl->d_tab.get(), tab.data(), kTabTotal * sizeof(float2), cudaMemcpyHostToDevice);
+    if (int rc = pl->d_tab.reserve(kTabCepTotal)) { delete pl; return rc; }
+    cudaError_t e = cudaMemcpy(pl->d_tab.get(), tab.data(), kTabCepTotal * sizeof(float2), cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_clip_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kClipCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_clip_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kClipCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFrameCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kFrameCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_frame_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kQuadCtaSmem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_cep_bluestein_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFrameCtaSmem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(pitch_track_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, track_smem(kCepLen));
     if (e != cudaSuccess) { delete pl; return fail(DSPFE_ERR_CUDA, cudaGetErrorString(e)); }
     b.tab = pl->d_tab.get();
@@ -317,6 +336,8 @@ int dspfe_pitch(dspfe_pitch_plan* pl, const void* d_pcm, int32_t sample_dtype, i
     const int64_t bound = dspfe_pitch_frames_bound(pl, total_samples, n_utt);
     if ((d_pitch || d_lag || d_rows) && max_frames < bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_pitch_frames_bound()");
     if (d_feat && pl->base.mode != 0) return fail(DSPFE_ERR_UNSUPPORTED, "pitch_feature is defined on the cepstrum pitch (pitch.py:33)");
+    if (d_feat && pl->base.frame_len != kCepLen)
+        return fail(DSPFE_ERR_UNSUPPORTED, "pitch_feature is defined on 512-sample cepstrum frames (pitch.py:33 uses the default winlen)");
     int rc = ensure(pl, n_utt, bound);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
@@ -334,13 +355,15 @@ int dspfe_pitch(dspfe_pitch_plan* pl, const void* d_pcm, int32_t sample_dtype, i
     if (clip_i16_keys(p)) pitch_clip_kernel<true><<<cgrid, 32 * kPitchWarps, kClipCtaSmem, st>>>(p);
     else pitch_clip_kernel<false><<<cgrid, 32 * kPitchWarps, kClipCtaSmem, st>>>(p);
     LAUNCH_CHECK("pitch_clip_kernel", st);
-    const int fmode = p.mode == 0 ? 0 : (acr_short_frames(p.frame_len, p.row_len) ? 2 : 1);
+    // 3: cepstrum frames other than 512 samples (pitch_cep_bluestein_kernel)
+    const int fmode = p.mode == 0 ? (p.frame_len == kCepLen ? 0 : 3) : (acr_short_frames(p.frame_len, p.row_len) ? 2 : 1);
     const int per = (fmode == 2 ? 4 : 2) * kPitchWarps;
     const unsigned fgrid = (unsigned)((slots + per - 1) / per);
     if (fmode == 0) pitch_frame_kernel<0><<<fgrid, 32 * kPitchWarps, kFrameCtaSmem, st>>>(p);
+    else if (fmode == 3) pitch_cep_bluestein_kernel<<<fgrid, 32 * kPitchWarps, kFrameCtaSmem, st>>>(p);
     else if (fmode == 2) pitch_frame_kernel<2><<<fgrid, 32 * kPitchWarps, kQuadCtaSmem, st>>>(p);
     else pitch_frame_kernel<1><<<fgrid, 32 * kPitchWarps, kFrameCtaSmem, st>>>(p);
-    LAUNCH_CHECK(fmode == 0 ? "pitch_frame_kernel<0>" : fmode == 2 ? "pitch_frame_kernel<2>" : "pitch_frame_kernel<1>", st);
+    LAUNCH_CHECK(fmode == 0 ? "pitch_frame_kernel<0>" : fmode == 3 ? "pitch_cep_bluestein_kernel" : fmode == 2 ? "pitch_frame_kernel<2>" : "pitch_frame_kernel<1>", st);
     if (d_pitch || d_lag || d_feat) {
         pitch_track_kernel<<<(unsigned)n_utt, kTrackThreads, track_smem(p.row_len), st>>>(p);
         LAUNCH_CHECK("pitch_track_kernel", st);

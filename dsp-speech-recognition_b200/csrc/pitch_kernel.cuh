@@ -9,6 +9,7 @@
 //            the reference), centre-clip at the median of its non-negative samples (exact bitwise selection),
 //            apply the one-sided (complex) FIR band-pass as a 1024-point FFT product, then
 //              cepstrum:        FFT512 -> log|.| -> IFFT512 -> |.|            -> row of row_len (<= 512) columns
+//                               (frames of 100..511 samples: N-point DFTs by Bluestein's chirp, pitch_cep_bluestein_pair)
 //              autocorrelation: |y| -> FFT1024 -> |.|^2 -> IFFT1024 -> /(L-n) -> row of 180 lags (20..199)
 //   K4b/K5b  one CTA per utterance walks its frames in order, 16 at a time: the reference's in-place running
 //            mean (a recurrence over already-smoothed rows, one column per thread), then peak scoring / argmax
@@ -48,6 +49,9 @@ constexpr int kWarpSmemBytes = kWarpScr * 8 + 512 * 16;              // transfor
 // table blob offsets, in float2
 constexpr int kTabTw = 0, kTabW32 = kTabTw + 512, kTabMod = kTabW32 + 32, kTabHe = kTabMod + 512, kTabHo = kTabHe + 512,
               kTabTotal = kTabHo + 512;
+// the Bluestein tables of pitch_cep_bluestein_pair follow the blob above (filled for cepstrum frames other than 512 samples):
+// the chirp w_n = exp(-i pi n^2 / N) for n < N (zero beyond) and the even / odd bins of the 1024-point spectrum of conj(w) wrapped
+constexpr int kTabChirp = kTabTotal, kTabBe = kTabChirp + 512, kTabBo = kTabBe + 512, kTabCepTotal = kTabBo + 512;
 constexpr int kFrameCtaSmem = (kTabMod * 8) + kPitchWarps * kWarpSmemBytes;                      // shared tables | per-warp areas
 constexpr int kClipRun = 8;         // frames per warp of K4a-1, and the padding unit of the slot space (even: pairs never straddle two runs)
 constexpr int kTrackThreads = 256;
@@ -70,7 +74,7 @@ struct PitchParams {
     int frame_len, frame_step;           // at the decimated rate: 512/100 (or 300/100 for the autocorrelation variant)
     int do_clip;                         // center_clip(frame, False) before the band-pass (pitch.py:88,103)
     int no_smooth;                       // taps only: K4b/K5b score the rows as given (peak_score on its own)
-    const float2* tab;                   // table blob (kTab* offsets): W512 twiddles, W32, W1024^n, He, Ho
+    const float2* tab;                   // table blob (kTab* offsets): W512 twiddles, W32, W1024^n, He, Ho (+ chirp, Be, Bo)
     float pre_hi, pre_lo;                // preemph split into float32 head + tail
     int ds_q32, ds_r32;                  // 32 / ds_out, 32 % ds_out
     int mode;                            // 0 cepstrum, 1 autocorrelation
@@ -696,6 +700,109 @@ DEVFN void pitch_fft_pair(const PitchParams& p, int64_t h0, int64_t g0, bool has
                         const float inv_n = (n < L) ? 1.0f / (float)(L - n) : NAN;
                         rowa[j] = r.x * inv_n;
                         if (hasB) rowb[j] = r.y * inv_n;
+                    }
+                }
+            }
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// K4a-2 for cepstrum frames of 100 <= N < 512 samples (pitch.py:83 with winlen != 0.0512): a frame pair per warp, as
+// pitch_fft_pair<0>, but the cepstrum's transforms are N-point DFTs, taken by Bluestein's identity
+//     DFT_N(a)[k] = w_k sum_n (a_n w_n) conj(w_{k-n}),   w_n = exp(-i pi n^2 / N),
+// a 1024-point circular convolution of s = a w (zero from N on) with b = conj(w) wrapped (b[m] = b[1024 - m] = conj(w_m), m < N):
+// b reaches 2N - 1 <= 1023 points, so the first N outputs carry no wrap.  Only magnitudes leave either DFT -- |Y| goes into the
+// log, |ifft| into the row -- and |w_k| = 1 drops the post-multiplication; the inverse DFT of the real log|Y| is
+// conj(DFT_N(log|Y|)) / N, so it is the same forward chain.  Each 1024-point convolution of an s supported on [0, 512) takes
+// four 512-point transforms, as the FIR of pitch_fft_pair<1> does:
+//     (s (*) k)[n] = (IFFT512(S_e K_e)[n] + W1024^-n IFFT512(S_o K_o)[n]) / 1024,   S_e = FFT512(s), S_o = FFT512(s W1024^n)
+// Three convolutions, 12 transforms per pair:  x (*) h -> y[0..N)  (He, Ho);  (y w) (*) b -> |Y|  (Be, Bo);
+// (log|Y| w) (*) b -> |.| / N -> rows.  s is parked for its odd half while the even half runs, then the two swap places.
+// wsm: per-warp shared memory = scr[kWarpScr] float2 | park[512] float4 (as pitch_fft_pair).
+// ---------------------------------------------------------------------------------------------------------
+// h0: the pair's first slot (even); g0: global index of its first frame; hasB: the second frame exists
+DEVFN void pitch_cep_bluestein_pair(const PitchParams& p, int64_t h0, int64_t g0, bool hasB, unsigned char* wsm, const float2* tws, const float2* w32s) {
+    const int lane = simt::tid() & 31;
+    float2* scr = reinterpret_cast<float2*>(wsm);
+    float4* park = reinterpret_cast<float4*>(scr + kWarpScr);
+    const float2* xs = p.clip + (h0 >> 1) * 512;      // the clipped frame pair
+    const float2* modA = p.tab + kTabMod;             // W1024^n, n = 32 t + lane
+    const float2* chirp = p.tab + kTabChirp;          // w_n (zero from N on)
+    const int N = p.frame_len;
+    const float2 zero2 = make_float2(0.f, 0.f);
+    const float inv1024 = 1.0f / 1024.0f;
+    cpx2 x[16];
+#pragma unroll
+    for (int t = 0; t < 16; ++t) { x[t].re = xs[32 * t + lane]; x[t].im = zero2; }
+    // stage 4c + 0  F(s)      -> S_e K_e          (s parked first)      c = 0: FIR, K = H;  c = 1, 2: Bluestein, K = B
+    //       4c + 1  inverse   -> park <-> x: the even half in, s W1024^n out
+    //       4c + 2  forward   -> S_o K_o
+    //       4c + 3  inverse   -> v = (park + W1024^-n d) / 1024, then  c = 0: y w;  c = 1: log|v| w;  c = 2: |v| / N -> rows
+#pragma unroll 1
+    for (int st = 0; st < 12; ++st) {
+        const int c = st >> 2, k = st & 3;
+        const bool inv = k & 1;
+        if (k == 0) {
+#pragma unroll
+            for (int t = 0; t < 16; ++t) park[32 * t + lane] = make_float4(x[t].re.x, x[t].re.y, x[t].im.x, x[t].im.y);
+        }
+        if (inv) {                                           // inverse = conj . forward . conj
+#pragma unroll
+            for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
+        }
+        fft512<true>(x, scr, tws, w32s, lane);
+        if (inv) {
+#pragma unroll
+            for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
+        }
+        if (!inv) {                                          // even (k = 0) or odd (k = 2) bins of the kernel's 1024-point spectrum
+            const float2* T = p.tab + (c == 0 ? (k == 0 ? kTabHe : kTabHo) : (k == 0 ? kTabBe : kTabBo));
+#pragma unroll
+            for (int t = 0; t < 16; ++t) { const float2 h = ldg(T + 32 * t + lane); x[t] = cmuls(x[t], h.x, h.y); }
+        } else if (k == 1) {                                 // (every lane only ever touches its own park entries)
+#pragma unroll
+            for (int t = 0; t < 16; ++t) {
+                const float4 pk = park[32 * t + lane];
+                park[32 * t + lane] = make_float4(x[t].re.x, x[t].re.y, x[t].im.x, x[t].im.y);
+                const float2 m = ldg(modA + 32 * t + lane);
+                cpx2 s; s.re = make_float2(pk.x, pk.y); s.im = make_float2(pk.z, pk.w);
+                x[t] = cmuls(s, m.x, m.y);
+            }
+        } else {
+#pragma unroll
+            for (int t = 0; t < 16; ++t) {
+                const int n = 32 * t + lane;
+                const float4 pk = park[n];
+                const float2 m = ldg(modA + n);
+                const cpx2 d = cmuls(x[t], m.x, -m.y);
+                cpx2 v;
+                v.re = f2muls(f2add(d.re, make_float2(pk.x, pk.y)), inv1024);
+                v.im = f2muls(f2add(d.im, make_float2(pk.z, pk.w)), inv1024);
+                if (c == 2) {
+                    x[t] = v;
+                } else {
+                    const float2 w = ldg(chirp + n);        // zero from N on: the sequence ends with the frame
+                    if (c == 1) {                            // log|Y| (the chirp of the last DFT has modulus 1); 0 * -inf is a NaN
+                        const float2 s2 = f2fma(v.im, v.im, f2mul(v.re, v.re));
+                        const float2 lg = n < N ? make_float2(0.5f * dsp_fast_logf(s2.x), 0.5f * dsp_fast_logf(s2.y)) : zero2;
+                        x[t].re = f2muls(lg, w.x); x[t].im = f2muls(lg, w.y);
+                    } else {
+                        x[t] = cmuls(v, w.x, w.y);
+                    }
+                }
+            }
+            if (c == 2) {                                    // |ifft_N| = |DFT_N| / N -> rows
+                const float invN = 1.0f / (float)N;
+                float* rowa = p.rows + g0 * p.row_len;
+                float* rowb = rowa + p.row_len;
+#pragma unroll
+                for (int t = 0; t < 16; ++t) {
+                    const int n = 32 * t + lane;
+                    if (n < p.row_len) {
+                        const float2 s2 = f2fma(x[t].im, x[t].im, f2mul(x[t].re, x[t].re));
+                        rowa[n] = dsp_fast_sqrtf(s2.x) * invN;
+                        if (hasB) rowb[n] = dsp_fast_sqrtf(s2.y) * invN;
                     }
                 }
             }

@@ -1,5 +1,5 @@
 // Host-side constant tables of the pitch kernels (shared by libdspfe.so and the test emulator):
-// parameter validation, the decimator pattern, W1024^k and the 1024-point spectrum of the FIR taps.
+// parameter validation, the decimator pattern, W1024^k, the 1024-point spectrum of the FIR taps and the Bluestein chirp tables.
 #pragma once
 #include <cmath>
 #include <cstring>
@@ -40,12 +40,36 @@ inline void fill_fft512_twiddles(float2* tws, float2* w32) {
     }
 }
 
+// Bluestein tables of an N-point DFT, N <= 512, as a 1024-point circular convolution (pitch_cep_bluestein_pair), float64 rounded
+// once: chirp[n] = w_n = exp(-i pi n^2 / N) for n < N, zero beyond; be[k] / bo[k] = bins 2k / 2k + 1 of FFT1024(b) with
+// b[m] = b[1024 - m] = conj(w_m) for m < N, zero elsewhere.  n^2 is reduced mod 2N in integers, so every angle
+// pi (n^2 mod 2N) / N lies in [0, 2 pi) and keeps its float64 precision for any n.
+inline void fill_cep_bluestein_tables(int N, float2* chirp, float2* be, float2* bo) {
+    const double kPi = 3.14159265358979323846;
+    std::vector<double> wr(N), wi(N), cr(kPitchFft), ci(kPitchFft);
+    for (int n = 0; n < N; ++n) {
+        const double a = -kPi * (double)((long long)n * n % (2LL * N)) / N;
+        wr[n] = cos(a); wi[n] = sin(a);
+    }
+    for (int n = 0; n < 512; ++n) chirp[n] = n < N ? make_float2((float)wr[n], (float)wi[n]) : make_float2(0.f, 0.f);
+    for (int j = 0; j < kPitchFft; ++j) { cr[j] = cos(-2 * kPi * j / kPitchFft); ci[j] = sin(-2 * kPi * j / kPitchFft); }
+    for (int k = 0; k < kPitchFft; ++k) {
+        double sr = 0, si = 0;
+        for (int m = 1 - N; m < N; ++m) {                          // b[m mod 1024] = conj(w_|m|)
+            const int am = m < 0 ? -m : m, j = (int)(((long long)k * (m & (kPitchFft - 1))) & (kPitchFft - 1));
+            sr += wr[am] * cr[j] + wi[am] * ci[j]; si += wr[am] * ci[j] - wi[am] * cr[j];
+        }
+        (k & 1 ? bo : be)[k >> 1] = make_float2((float)sr, (float)si);
+    }
+}
+
 // Fills the scalar part of PitchParams and the two tables.  Returns 0 or a dspfe_status with `err` set.
 inline int build_pitch_tables(const dspfe_pitch_params& q, PitchParams& b, std::vector<float2>& tab, std::string& err) {
     std::memset(&b, 0, sizeof(b));
     if (q.samplerate <= 0 || q.dst_rate <= 0 || q.frame_step < 1) { err = "bad pitch parameters"; return DSPFE_ERR_INVALID_ARG; }
     if (q.method != 0 && q.method != 1) { err = "method must be 0 (cepstrum) or 1 (autocorrelation)"; return DSPFE_ERR_INVALID_ARG; }
-    if (q.method == 0 && q.frame_len != kCepLen) { err = "the cepstrum kernel is built for 512-sample frames"; return DSPFE_ERR_UNSUPPORTED; }
+    // peak_score (pitch.py:227-242) reads row columns 20..99: the reference raises on shorter cepstrum frames
+    if (q.method == 0 && (q.frame_len < kMinLag + kPeakLags || q.frame_len > kCepLen)) { err = "cepstrum frames must have 100..512 samples"; return DSPFE_ERR_UNSUPPORTED; }
     if (q.method == 1 && (q.frame_len <= kMinLag || q.frame_len > 512)) { err = "autocorrelation frames must have 21..512 samples"; return DSPFE_ERR_UNSUPPORTED; }
     if (q.frame_len + q.frame_step > kClipDecCap) { err = "frame_step too large: two frames must fit the clip kernel's sample buffer"; return DSPFE_ERR_UNSUPPORTED; }
     // decimator pattern (preprocess.py:21-28): the k-th kept sample (k >= 1) is floor((k-1)*src/dst) + 1
@@ -59,14 +83,16 @@ inline int build_pitch_tables(const dspfe_pitch_params& q, PitchParams& b, std::
     }
     b.frame_len = q.frame_len; b.frame_step = q.frame_step; b.do_clip = q.center_clip ? 1 : 0; b.mode = q.method;
     b.preemph = q.preemph;
-    b.row_len = q.method == 0 ? (q.row_len > 0 ? q.row_len : kCepCols) : kAcrLags;
-    if (q.method == 0 && (b.row_len < kPeakLags + kMinLag || b.row_len > kCepLen)) { err = "row_len must be in 100..512"; return DSPFE_ERR_INVALID_ARG; }
+    // cepstrum rows: columns 0..199 decide every peak score; a row shorter than that is the whole cepstrum (the right-hand
+    // scan of peak_score ends at the frame length)
+    b.row_len = q.method == 0 ? (q.row_len > 0 ? q.row_len : (q.frame_len < kCepCols ? q.frame_len : kCepCols)) : kAcrLags;
+    if (q.method == 0 && (b.row_len < kPeakLags + kMinLag || b.row_len > q.frame_len)) { err = "row_len must be in 100..frame_len"; return DSPFE_ERR_INVALID_ARG; }
     b.ds_q32 = 32 / b.ds_out; b.ds_r32 = 32 % b.ds_out;
     b.pre_hi = (float)q.preemph; b.pre_lo = (float)(q.preemph - (double)b.pre_hi);
     // tables, float64 on the host, rounded once: the FFT twiddles, W1024^n and the even / odd bins of the 1024-point
     // spectrum of the FIR taps, all in natural order
     const double kPi = 3.14159265358979323846;
-    tab.assign(kTabTotal, make_float2(0.f, 0.f));
+    tab.assign(kTabCepTotal, make_float2(0.f, 0.f));
     fill_fft512_twiddles(tab.data() + kTabTw, tab.data() + kTabW32);
     for (int n = 0; n < 512; ++n) tab[kTabMod + n] = make_float2((float)cos(-2 * kPi * n / 1024.0), (float)sin(-2 * kPi * n / 1024.0));
     std::vector<double> hr, hi;
@@ -81,6 +107,7 @@ inline int build_pitch_tables(const dspfe_pitch_params& q, PitchParams& b, std::
             }
             tab[(odd ? kTabHo : kTabHe) + k] = make_float2((float)sr, (float)si);
         }
+    if (q.method == 0 && q.frame_len != kCepLen) fill_cep_bluestein_tables(q.frame_len, tab.data() + kTabChirp, tab.data() + kTabBe, tab.data() + kTabBo);
     if (q.method == 1 && acr_short_frames(q.frame_len, b.row_len)) {
         // pitch_acr_quad's split FIR: H_lo = FFT512(taps 0..T), H_hi = FFT512(taps T+1..L-1 left in place), T = 512 - L;
         // kTabHe <- A = (H_lo - i H_hi) / 2, kTabHo <- B = (H_lo + i H_hi) / 2, both with the inverse transform's 1/512

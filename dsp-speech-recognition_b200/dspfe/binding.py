@@ -594,7 +594,10 @@ def _np_ptr(a):
 
 class PitchPlan:
     """dspfe_pitch_plan: batched pitch_detect (method 0) / pitch_detect_sr (method 1) / pitch_feature
-    (reference pitch.py:83, :96, :26)."""
+    (reference pitch.py:83, :96, :26).  frame_len = int(10000 * winlen): 100..512 for the cepstrum (512 = winlen 0.0512, the
+    reference default; other lengths take N-point transforms), 21..512 for the autocorrelation; other lengths raise
+    DspfeUnsupported.  row_len (cepstrum): 0 = min(frame_len, 200), else 100..frame_len.  want_feat needs method 0 at
+    frame_len 512."""
 
     def __init__(self, method=0, samplerate=16000, dst_rate=10000, frame_len=512, frame_step=100, center_clip=True,
                  row_len=0, band_lo=50.0, band_hi=None, preemph=0.0):

@@ -56,8 +56,11 @@ def _frame_geometry(winlen, step):
 
 def _detect(sig, rate, winlen, step, method, want_feat=False):
     frame_len, frame_step = _frame_geometry(winlen, step)
-    if method == 0 and frame_len != 512:
-        raise NotImplementedError("cepstrum pitch is built for winlen=0.0512 (512 samples at 10 kHz)")
+    if method == 0 and frame_len < 100:
+        # the reference's peak_score reads row[20..99] of every cepstrum row of frame_len values (pitch.py:232)
+        raise IndexError(f"index {max(frame_len, 20)} is out of bounds for axis 0 with size {frame_len}")
+    if method == 0 and frame_len > 512:
+        raise NotImplementedError("cepstrum pitch is built for frames of 100..512 samples at 10 kHz (winlen 0.01..0.0512)")
     if method == 1 and not (20 < frame_len <= 512):
         raise NotImplementedError("autocorrelation pitch is built for frames of 21..512 samples at 10 kHz")
     if frame_step < 1:
@@ -76,7 +79,7 @@ def _frames_of(sig, rate, frame_len, frame_step):
 def pitch_feature(sig, rate, gender='male'):
     """reference pitch.py:26-47: the five SVM inputs (slope1, slope2, quad1, quad2, median shift) of a signal that
     has been endpoint-trimmed (and pre-emphasised) by the caller.  The reference's two debugging prints are dropped."""
-    (pitch, lag, fo, feat), _ = _detect(sig, rate, 0.0512, 0.01, 0, want_feat=True)
+    (pitch, lag, fo, feat), _ = _detect(sig, rate, 0.0512, 0.01, 0, want_feat=True)   # always the default winlen (pitch.py:33)
     return tuple(np.float64(v) for v in feat[0])
 
 
@@ -102,7 +105,8 @@ def sub_endpoint_detect(frames):
 
 
 def pitch_detect(sig, rate, winlen=0.0512, step=0.01, gender='male'):
-    """reference pitch.py:83-94: cepstrum pitch.  Returns (list of Hz per frame, frames [F,512] float64)."""
+    """reference pitch.py:83-94: cepstrum pitch.  Returns (list of Hz per frame, frames [F,N] float64), N = int(10000 * winlen).
+    N from 100 to 512 samples is built; N < 100 raises IndexError as the reference's peak_score does, N > 512 NotImplementedError."""
     (pitch, lag, fo), (fl, fs) = _detect(sig, rate, winlen, step, 0)
     return [np.float64(v) for v in pitch], _frames_of(sig, rate, fl, fs)
 
@@ -137,10 +141,12 @@ def pitch_detect_frame_sr(frame, rate):
 
 
 def pitch_detect_frame(frame, rate, gender):
-    """reference pitch.py:135-143: |ifft(log|fft(window(frame, 50, 1000, 'hamming'))|)|, 512 values."""
-    if len(frame) != 512:
-        raise NotImplementedError("the cepstrum kernel is built for 512-sample frames")
-    return _frame_rows(frame, rate, 0, 512)
+    """reference pitch.py:135-143: |ifft(log|fft(window(frame, 50, 1000, 'hamming'))|)|, all N values of a 1-D frame of
+    N = 100..512 samples (N-point transforms, as the reference)."""
+    n = np.asarray(frame).shape[-1] if np.ndim(frame) else 0
+    if np.ndim(frame) != 1 or not (100 <= n <= 512):
+        raise NotImplementedError("the cepstrum kernel is built for 1-D frames of 100..512 samples")
+    return _frame_rows(frame, rate, 0, n)
 
 
 def center_clip(frame, binary=True):

@@ -237,11 +237,14 @@ typedef struct dspfe_pitch_plan dspfe_pitch_plan;
 typedef struct {
     int32_t samplerate;      /* rate of the packed samples, 16000 */
     int32_t dst_rate;        /* 10000: rate the pitch functions decimate to (pitch.py:84,100) */
-    int32_t frame_len;       /* int(dst_rate*winlen): 512 (pitch_detect), or 300 for pitch_detect_sr as model.py:92 calls it */
+    int32_t frame_len;       /* int(dst_rate*winlen): 512 (pitch_detect), or 300 for pitch_detect_sr as model.py:92 calls it.
+                              * Cepstrum: 100..512 (512 runs the 512-point chain, the others N-point DFTs by Bluestein's chirp);
+                              * autocorrelation: 21..512.  Others: DSPFE_ERR_UNSUPPORTED */
     int32_t frame_step;      /* int(step*dst_rate): 100 */
     int32_t method;          /* 0 cepstrum (pitch_detect), 1 autocorrelation (pitch_detect_sr) */
     int32_t center_clip;     /* 1: center_clip(frame, False) before the band-pass (pitch.py:88); 0 for the per-frame taps */
-    int32_t row_len;         /* cepstrum columns kept per frame; 0 = 200 (all peak_score can reach), 512 for the full-row tap */
+    int32_t row_len;         /* cepstrum columns kept per frame, 100..frame_len; 0 = min(frame_len, 200) (all peak_score can
+                              * reach: its right-hand scan ends at the frame length), frame_len for the full-row tap */
     int32_t reserved;
     double band_lo, band_hi; /* band-pass edges in Hz: 50..1000 (pitch.py:137) / 50..900 (pitch.py:124) */
     double preemph;          /* pre-emphasis over the whole utterance before trimming (pitch_model.py:39-41); 0 = none */
@@ -261,7 +264,8 @@ int64_t dspfe_pitch_num_frames_host(const dspfe_pitch_params* p, int64_t n_sampl
 /* Device path, asynchronous on `stream`.  sample_dtype: 0 = int16, 1 = float32 samples.  d_trim as for
  * dspfe_mfcc_delta (pitch runs on sig[left:right], pitch_model.py:41).  Outputs (each may be NULL):
  *   d_pitch [frames] float64 Hz (robust_max_pitch), d_lag [frames] int32 = 20 + argmax (before the octave repair),
- *   d_feat [n_utt,5] float64 = pitch_feature (cepstrum method only; NaN x5 where a half has < 3 usable frames),
+ *   d_feat [n_utt,5] float64 = pitch_feature (cepstrum method at frame_len 512 only, the default winlen pitch.py:33 uses;
+ *          other plans fail with DSPFE_ERR_UNSUPPORTED; NaN x5 where a half has < 3 usable frames),
  *   d_rows [frames,row_len] float32 = the per-frame cepstrum / autocorrelation rows before smoothing,
  *   d_frame_off [n_utt+1] int64.  max_frames = capacity in frames, >= dspfe_pitch_frames_bound(). */
 int dspfe_pitch(dspfe_pitch_plan* plan, const void* d_pcm, int32_t sample_dtype, int64_t total_samples, const int64_t* d_offsets,
