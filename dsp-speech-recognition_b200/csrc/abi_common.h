@@ -13,6 +13,29 @@
 namespace dspfe {
 inline thread_local std::string g_err;
 inline int fail(int code, const std::string& msg) { g_err = msg; return code; }
+
+// The argument check of every batched entry point on device samples, in one order: a null plan, offsets or required output
+// (`args_ok` false) or a negative count -> DSPFE_ERR_INVALID_ARG; a plan that cannot run this entry point (`unsupported`, the
+// message, or null) -> DSPFE_ERR_UNSUPPORTED; an empty batch -> DSPFE_OK, and the caller returns before it queues anything;
+// null samples with total_samples > 0, or samples not 16-byte aligned -> DSPFE_ERR_INVALID_ARG.
+inline int check_batch(bool args_ok, int64_t n_utt, int64_t total_samples, const void* d_pcm, const char* unsupported = nullptr) {
+    if (!args_ok || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (unsupported) return fail(DSPFE_ERR_UNSUPPORTED, unsupported);
+    if (n_utt == 0) return DSPFE_OK;
+    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
+    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
+    return DSPFE_OK;
+}
+
+// The same for the host-buffer forms: bad arguments, then `unsupported`, then every offset of the batch non-decreasing
+// (h_offsets[0 .. n_utt]); DSPFE_OK for an empty batch.
+inline int check_host_batch(bool args_ok, const int64_t* h_offsets, int32_t n_utt, const char* unsupported = nullptr) {
+    if (!args_ok || !h_offsets || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (unsupported) return fail(DSPFE_ERR_UNSUPPORTED, unsupported);
+    for (int32_t u = 0; u < n_utt; ++u)
+        if (h_offsets[u + 1] < h_offsets[u]) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
+    return DSPFE_OK;
+}
 }  // namespace dspfe
 
 // After a kernel launch: always check the launch status; with DSPFE_DEBUG_SYNC=1 in the environment also wait for
@@ -118,6 +141,45 @@ public:
     cudaEvent_t get() const { return e_; }
 private:
     cudaEvent_t e_ = nullptr;
+};
+
+// The staging of a plan's host-buffer forms: a stream, and on the device the samples of a host batch from h_offsets[0] on
+// and the offsets relative to the first.
+class HostBatch : NoCopy {
+public:
+    // Copies the batch on the stream.  frames(u, len) is the frame count of utterance u of len samples: their prefix sums go
+    // to h_frame_off (optional, [n_utt + 1]), and *total / *n_frames receive the batch's samples and frames.
+    template <class Frames>
+    int stage(const void* h_pcm, int64_t esz, const int64_t* h_offsets, int32_t n_utt, Frames frames, int64_t* h_frame_off,
+              int64_t* total, int64_t* n_frames) {
+        const int64_t base = h_offsets[0];
+        *total = h_offsets[n_utt] - base;
+        CUDA_TRY(stream_.ensure());
+        int rc = pcm_.reserve((*total + 8) * esz);
+        if (!rc) rc = off_.reserve(n_utt + 1);
+        if (rc) return rc;
+        std::vector<int64_t> rel(n_utt + 1);
+        int64_t f = 0;
+        for (int32_t u = 0; u < n_utt; ++u) {
+            rel[u] = h_offsets[u] - base;
+            if (h_frame_off) h_frame_off[u] = f;
+            f += frames(u, h_offsets[u + 1] - h_offsets[u]);
+        }
+        rel[n_utt] = *total;
+        if (h_frame_off) h_frame_off[n_utt] = f;
+        *n_frames = f;
+        const cudaStream_t st = stream_.get();
+        if (*total > 0) CUDA_TRY(cudaMemcpyAsync(pcm_.get(), (const char*)h_pcm + base * esz, *total * esz, cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaMemcpyAsync(off_.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        return DSPFE_OK;
+    }
+    cudaStream_t stream() const { return stream_.get(); }
+    template <class T = void> const T* pcm() const { return reinterpret_cast<const T*>(pcm_.get()); }
+    const int64_t* offsets() const { return off_.get(); }
+private:
+    Stream stream_;
+    DeviceArray<unsigned char> pcm_;
+    DeviceArray<int64_t> off_;
 };
 
 // A per-call temporary: alloc() takes it from the stream-ordered pool of `st`, and it goes back on the same stream when

@@ -206,6 +206,16 @@ int launch_mfcc(dspfe_plan* pl, Workspace& ws, const void* d_pcm, bool f32, int6
     return DSPFE_OK;
 }
 
+// the device forms: mode 0 MFCC + delta + delta-delta, 1 the filterbank tap, 2 the spectrum tap of the given kind
+int mfcc_device(dspfe_plan* pl, const void* d_pcm, bool f32, int64_t total_samples, const int64_t* d_offsets, const int32_t* d_trim,
+                int32_t n_utt, float* d_out, int64_t max_rows, int64_t* d_frame_off, void* stream, int mode = 0, int kind = 0) {
+    if (int rc = check_batch(pl && d_offsets && d_out && kind >= 0 && kind <= 2, n_utt, total_samples, d_pcm)) return rc;
+    if (n_utt == 0) return DSPFE_OK;
+    if (max_rows < dspfe_rows_bound(pl, total_samples, n_utt))
+        return fail(DSPFE_ERR_INVALID_ARG, "d_out capacity (max_rows) is below dspfe_rows_bound()");
+    return launch_mfcc(pl, pl->ws, d_pcm, f32, total_samples, d_offsets, d_trim, n_utt, d_out, d_frame_off, (cudaStream_t)stream, mode, kind);
+}
+
 }  // namespace
 
 extern "C" {
@@ -342,48 +352,28 @@ int64_t dspfe_rows_bound(const dspfe_plan* pl, int64_t total_samples, int64_t n_
 int dspfe_mfcc_delta(dspfe_plan* pl, const int16_t* d_pcm, int64_t total_samples, const int64_t* d_offsets,
                      const int32_t* d_trim, int32_t n_utt, float* d_out, int64_t max_rows, int64_t* d_frame_off,
                      void* stream) {
-    if (!pl || !d_offsets || !d_out || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    if (max_rows < dspfe_rows_bound(pl, total_samples, n_utt))
-        return fail(DSPFE_ERR_INVALID_ARG, "d_out capacity (max_rows) is below dspfe_rows_bound()");
-    return launch_mfcc(pl, pl->ws, d_pcm, false, total_samples, d_offsets, d_trim, n_utt, d_out, d_frame_off, (cudaStream_t)stream);
+    return mfcc_device(pl, d_pcm, false, total_samples, d_offsets, d_trim, n_utt, d_out, max_rows, d_frame_off, stream);
 }
 
 int dspfe_mfcc_delta_f32(dspfe_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets,
                          const int32_t* d_trim, int32_t n_utt, float* d_out, int64_t max_rows, int64_t* d_frame_off,
                          void* stream) {
-    if (!pl || !d_offsets || !d_out || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    if (max_rows < dspfe_rows_bound(pl, total_samples, n_utt))
-        return fail(DSPFE_ERR_INVALID_ARG, "d_out capacity (max_rows) is below dspfe_rows_bound()");
-    return launch_mfcc(pl, pl->ws, d_pcm, true, total_samples, d_offsets, d_trim, n_utt, d_out, d_frame_off, (cudaStream_t)stream);
+    return mfcc_device(pl, d_pcm, true, total_samples, d_offsets, d_trim, n_utt, d_out, max_rows, d_frame_off, stream);
 }
 
 int dspfe_fbank_f32(dspfe_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                     float* d_out, int64_t max_rows, int64_t* d_frame_off, void* stream) {
-    if (!pl || !d_offsets || !d_out || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    if (max_rows < dspfe_rows_bound(pl, total_samples, n_utt)) return fail(DSPFE_ERR_INVALID_ARG, "d_out capacity (max_rows) is below dspfe_rows_bound()");
-    return launch_mfcc(pl, pl->ws, d_pcm, true, total_samples, d_offsets, nullptr, n_utt, d_out, d_frame_off, (cudaStream_t)stream, 1, 0);
+    return mfcc_device(pl, d_pcm, true, total_samples, d_offsets, nullptr, n_utt, d_out, max_rows, d_frame_off, stream, 1);
 }
 
 int dspfe_spectrum_f32(dspfe_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                        int32_t kind, float* d_out, int64_t max_rows, int64_t* d_frame_off, void* stream) {
-    if (!pl || !d_offsets || !d_out || n_utt < 0 || total_samples < 0 || kind < 0 || kind > 2) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    if (max_rows < dspfe_rows_bound(pl, total_samples, n_utt)) return fail(DSPFE_ERR_INVALID_ARG, "d_out capacity (max_rows) is below dspfe_rows_bound()");
-    return launch_mfcc(pl, pl->ws, d_pcm, true, total_samples, d_offsets, nullptr, n_utt, d_out, d_frame_off, (cudaStream_t)stream, 2, kind);
+    return mfcc_device(pl, d_pcm, true, total_samples, d_offsets, nullptr, n_utt, d_out, max_rows, d_frame_off, stream, 2, kind);
 }
 
 int dspfe_mfcc_delta_host(dspfe_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, float* h_out,
                           int64_t* h_frame_off) {
-    if (!pl || !h_offsets || !h_out || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (int rc = check_host_batch(pl && h_out, h_offsets, n_utt)) return rc;
     if (n_utt == 0) return DSPFE_OK;
     const int flen = pl->cfg.count_len, fstep = pl->cfg.frame_step, width = pl->width;
     // slabs of consecutive utterances: <= kSlabSamples samples each (one oversized utterance = its own slab)
@@ -395,7 +385,6 @@ int dspfe_mfcc_delta_host(dspfe_plan* pl, const int16_t* h_pcm, const int64_t* h
         int32_t u_end = u; int64_t samples = 0, rows = 0;
         while (u_end < n_utt) {
             const int64_t len = h_offsets[u_end + 1] - h_offsets[u_end];
-            if (len < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
             if (u_end > u && samples + len > kSlabSamples) break;
             samples += len; rows += num_frames(len, flen, fstep);
             if (h_frame_off) h_frame_off[u_end] = row + rows - num_frames(len, flen, fstep);

@@ -69,4 +69,16 @@ int64_t num_frames(int64_t slen, int frame_len, int frame_step) {
     return 1 + (slen - frame_len + frame_step - 1) / frame_step;
 }
 
+// Python's slice sig[l:r] with l, r >= 0 of a signal of `len` samples: l and r clamped into [0, len]; returns the slice's
+// length and leaves its first sample in l.  (The prep kernels write the clamp out: through this call their SASS differs.)
+inline
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+long long trim_slice(long long len, long long& l, long long r) {
+    if (l < 0) l = 0; if (r < 0) r = 0;
+    if (l > len) l = len; if (r > len) r = len;
+    return r > l ? r - l : 0;
+}
+
 }  // namespace dspfe

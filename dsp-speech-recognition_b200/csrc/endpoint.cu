@@ -12,7 +12,8 @@ struct dspfe_endpoint_plan {
     dspfe_endpoint_params prm;
     EpRule rule;
     int frame_len, frame_step, q, rem;
-    Stream stream;              // host path
+    HostBatch host;             // host-path staging (int16 or float32 samples)
+    DeviceArray<int32_t> d_lr;
     // workspaces
     DeviceArray<int64_t> frame_off, block_off; DeviceArray<int32_t> order;
     DeviceArray<int32_t> blk, asum, zcr;
@@ -20,9 +21,6 @@ struct dspfe_endpoint_plan {
     // float-sample path: the split tree of the pairwise sum over one frame (np_pairwise_tree), uploaded on first use
     std::vector<int32_t> h_tree; int nleaf = 0;
     DeviceArray<int32_t> tree; bool tree_ready = false;
-    // host-path staging (int16 or float32 samples)
-    DeviceArray<unsigned char> d_pcm;
-    DeviceArray<int64_t> d_off; DeviceArray<int32_t> d_lr;
 };
 
 namespace {
@@ -49,6 +47,115 @@ int ensure(dspfe_endpoint_plan* pl, int64_t n_utt, int64_t blocks, int64_t frame
     if (!rc) rc = pl->zcr.reserve(frames);
     if (!rc) rc = pl->amp.reserve(frames);
     return rc;
+}
+
+// What differs between the sample types: the frame statistics (int16: sum |x| per frame from K2a + K2b; float32: K2f's
+// float64 amplitudes), the EpParams fields that carry the samples and the statistics, the decision kernel's amplitude source,
+// and the kernel names the timing reports show.
+template <class T> struct EpType;
+template <> struct EpType<int16_t> {
+    using Stat = int32_t;
+    using Amp = AmpFromSum;
+    static constexpr const char* kDecide = "ep_decide_kernel";
+    static constexpr const char* kRobust = "ep_decide_robust_kernel";
+    static const char* unsupported(const dspfe_endpoint_plan*) { return nullptr; }
+    static Stat* stat(dspfe_endpoint_plan* pl) { return pl->asum.get(); }
+    static void set(EpParams& p, const int16_t* x, Stat* stat) { p.pcm = x; p.asum = stat; }
+    static int stats(dspfe_endpoint_plan*, const EpParams& p, int64_t, cudaStream_t st) {
+        ep_block_kernel<<<(unsigned)((p.max_blocks + 127) / 128), 128, 0, st>>>(p);
+        LAUNCH_CHECK("ep_block_kernel", st);
+        ep_frame_kernel<<<(unsigned)((p.max_frames + 255) / 256), 256, 0, st>>>(p);
+        LAUNCH_CHECK("ep_frame_kernel", st);
+        return DSPFE_OK;
+    }
+};
+template <> struct EpType<float> {
+    using Stat = double;
+    using Amp = AmpFromF64;
+    static constexpr const char* kDecide = "ep_decide_kernel<f64>";
+    static constexpr const char* kRobust = "ep_decide_robust_kernel<f32>";
+    static const char* unsupported(const dspfe_endpoint_plan* pl) {
+        return pl && pl->frame_len > kEpF32MaxLen ? "float-sample endpoint frames longer than 8192 samples are not built" : nullptr;
+    }
+    static Stat* stat(dspfe_endpoint_plan* pl) { return pl->amp.get(); }
+    static void set(EpParams& p, const float* x, Stat* stat) { p.pcm_f32 = x; p.amp = stat; }
+    static int stats(dspfe_endpoint_plan* pl, const EpParams& p, int64_t total_samples, cudaStream_t st) {
+        if (!pl->tree_ready) {
+            int rc = pl->tree.reserve((int64_t)pl->h_tree.size());
+            if (rc) return rc;
+            CUDA_TRY(cudaMemcpyAsync(pl->tree.get(), pl->h_tree.data(), pl->h_tree.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+            pl->tree_ready = true;
+        }
+        EpF32Params f;
+        f.pcm = p.pcm_f32; f.total_samples = total_samples; f.offsets = p.offsets; f.frame_off = p.frame_off; f.n_utt = p.n_utt;
+        f.frame_len = p.frame_len; f.frame_step = p.frame_step; f.tree = pl->tree.get(); f.nleaf = pl->nleaf;
+        f.max_frames = p.max_frames; f.amp = const_cast<double*>(p.amp); f.zcr = p.zcr;
+        ep_f32_layout(f);
+        if (f.sm_total > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(ep_stats_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, f.sm_total));
+        ep_stats_f32_kernel<<<(unsigned)((p.max_frames + f.run - 1) / f.run), kEpF32Threads, f.sm_total, st>>>(f);
+        LAUNCH_CHECK("ep_stats_f32_kernel", st);
+        return DSPFE_OK;
+    }
+};
+
+const char* robust_unsupported(const dspfe_endpoint_plan* pl) {
+    return pl && pl->frame_len > kEpGateMaxLen ? "robust endpoint frames longer than 1536 samples are not built" : nullptr;
+}
+
+// K1 (prep), the frame statistics, K3 (decision); `robust` then runs K3r's gated rule over the same statistics, which
+// overwrites K3's decision.  Null d_stat / d_zcr / d_frame_off: the plan's workspaces.
+template <class T>
+int endpoint_device(dspfe_endpoint_plan* pl, const T* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt, int32_t* d_lr,
+                    typename EpType<T>::Stat* d_stat, int32_t* d_zcr, int64_t* d_frame_off, int64_t max_frames, void* stream, bool robust = false) {
+    const char* unsupported = robust ? robust_unsupported(pl) : EpType<T>::unsupported(pl);
+    if (int rc = check_batch(pl && d_offsets && d_lr, n_utt, total_samples, d_pcm, unsupported)) return rc;
+    if (n_utt == 0) return DSPFE_OK;
+    const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
+    if ((d_stat || d_zcr) && max_frames < frames_bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_endpoint_frames_bound()");
+    const int64_t blocks_bound = frames_bound + (int64_t)n_utt * (pl->q + 1);
+    int rc = ensure(pl, n_utt, blocks_bound, frames_bound);   // first: growing a workspace moves it
+    if (rc) return rc;
+    EpParams p;
+    std::memset(&p, 0, sizeof(p));
+    EpType<T>::set(p, d_pcm, d_stat ? d_stat : EpType<T>::stat(pl));
+    p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step; p.q = pl->q; p.rem = pl->rem;
+    p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.block_off = pl->block_off.get(); p.blk = pl->blk.get();
+    p.zcr = d_zcr ? d_zcr : pl->zcr.get(); p.lr = d_lr; p.rule = pl->rule; p.order = pl->order.get();
+    p.max_blocks = blocks_bound; p.max_frames = frames_bound;
+    cudaStream_t st = (cudaStream_t)stream;
+    ep_prep_kernel<<<1, kEpPrepThreads, 0, st>>>(p);
+    LAUNCH_CHECK("ep_prep_kernel", st);
+    rc = EpType<T>::stats(pl, p, total_samples, st);
+    if (rc) return rc;
+    ep_decide_kernel<typename EpType<T>::Amp><<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
+    LAUNCH_CHECK(EpType<T>::kDecide, st);
+    if (!robust) return DSPFE_OK;
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
+    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<T>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    ep_decide_robust_kernel<T><<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
+    LAUNCH_CHECK(EpType<T>::kRobust, st);
+    return DSPFE_OK;
+}
+
+// the host-buffer forms: the batch is staged once and the device form run once on the plan's stream
+template <class T>
+int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
+                  typename EpType<T>::Stat* h_stat, int32_t* h_zcr, int64_t* h_frame_off, bool robust = false) {
+    if (int rc = check_host_batch(pl && h_lr, h_offsets, n_utt, robust ? robust_unsupported(pl) : nullptr)) return rc;
+    if (n_utt == 0) return DSPFE_OK;
+    int64_t total = 0, frames = 0;
+    int rc = pl->d_lr.reserve((int64_t)n_utt * 2);
+    if (!rc) rc = pl->host.stage(h_pcm, sizeof(T), h_offsets, n_utt, [pl](int32_t, int64_t len) { return num_frames(len, pl->frame_len, pl->frame_step); },
+                                 h_frame_off, &total, &frames);
+    if (rc) return rc;
+    const cudaStream_t st = pl->host.stream();
+    rc = endpoint_device<T>(pl, pl->host.pcm<T>(), total, pl->host.offsets(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st, robust);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (h_stat) CUDA_TRY(cudaMemcpyAsync(h_stat, EpType<T>::stat(pl), frames * sizeof(*h_stat), cudaMemcpyDeviceToHost, st));
+    if (h_zcr) CUDA_TRY(cudaMemcpyAsync(h_zcr, pl->zcr.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return DSPFE_OK;
 }
 
 }  // namespace
@@ -156,190 +263,23 @@ int64_t dspfe_endpoint_frames_bound(const dspfe_endpoint_plan* pl, int64_t total
 
 int dspfe_endpoint(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                    int32_t* d_lr, int32_t* d_asum, int32_t* d_zcr, int64_t* d_frame_off, int64_t max_frames, void* stream) {
-    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
-    if ((d_asum || d_zcr) && max_frames < frames_bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_endpoint_frames_bound()");
-    const int64_t blocks_bound = frames_bound + (int64_t)n_utt * (pl->q + 1);
-    int rc = ensure(pl, n_utt, blocks_bound, frames_bound);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    EpParams p;
-    p.pcm = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.block_off = pl->block_off.get();
-    p.blk = pl->blk.get(); p.asum = d_asum ? d_asum : pl->asum.get(); p.zcr = d_zcr ? d_zcr : pl->zcr.get(); p.lr = d_lr;
-    p.max_blocks = blocks_bound; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order.get();
-    ep_prep_kernel<<<1, kEpPrepThreads, 0, st>>>(p);
-    LAUNCH_CHECK("ep_prep_kernel", st);
-    ep_block_kernel<<<(unsigned)((blocks_bound + 127) / 128), 128, 0, st>>>(p);
-    LAUNCH_CHECK("ep_block_kernel", st);
-    ep_frame_kernel<<<(unsigned)((frames_bound + 255) / 256), 256, 0, st>>>(p);
-    LAUNCH_CHECK("ep_frame_kernel", st);
-    ep_decide_kernel<AmpFromSum><<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
-    LAUNCH_CHECK("ep_decide_kernel", st);
-    return DSPFE_OK;
+    return endpoint_device(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, d_asum, d_zcr, d_frame_off, max_frames, stream);
 }
 
 int dspfe_endpoint_f32(dspfe_endpoint_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                        int32_t* d_lr, double* d_amp, int32_t* d_zcr, int64_t* d_frame_off, int64_t max_frames, void* stream) {
-    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (pl->frame_len > kEpF32MaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "float-sample endpoint frames longer than 8192 samples are not built");
-    if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
-    if ((d_amp || d_zcr) && max_frames < frames_bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_endpoint_frames_bound()");
-    const int64_t blocks_bound = frames_bound + (int64_t)n_utt * (pl->q + 1);
-    int rc = ensure(pl, n_utt, blocks_bound, frames_bound);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (!pl->tree_ready) {
-        rc = pl->tree.reserve((int64_t)pl->h_tree.size());
-        if (rc) return rc;
-        CUDA_TRY(cudaMemcpyAsync(pl->tree.get(), pl->h_tree.data(), pl->h_tree.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-        pl->tree_ready = true;
-    }
-    EpParams p;
-    p.pcm = nullptr; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = d_frame_off ? d_frame_off : pl->frame_off.get(); p.block_off = pl->block_off.get();
-    p.blk = pl->blk.get(); p.asum = nullptr; p.zcr = d_zcr ? d_zcr : pl->zcr.get(); p.lr = d_lr;
-    p.max_blocks = blocks_bound; p.max_frames = frames_bound; p.rule = pl->rule; p.order = pl->order.get();
-    p.amp = d_amp ? d_amp : pl->amp.get();
-    EpF32Params f;
-    f.pcm = d_pcm; f.total_samples = total_samples; f.offsets = d_offsets; f.frame_off = p.frame_off; f.n_utt = n_utt;
-    f.frame_len = pl->frame_len; f.frame_step = pl->frame_step; f.tree = pl->tree.get(); f.nleaf = pl->nleaf;
-    f.max_frames = frames_bound; f.amp = const_cast<double*>(p.amp); f.zcr = p.zcr;
-    ep_f32_layout(f);
-    ep_prep_kernel<<<1, kEpPrepThreads, 0, st>>>(p);
-    LAUNCH_CHECK("ep_prep_kernel", st);
-    if (f.sm_total > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(ep_stats_f32_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, f.sm_total));
-    ep_stats_f32_kernel<<<(unsigned)((frames_bound + f.run - 1) / f.run), kEpF32Threads, f.sm_total, st>>>(f);
-    LAUNCH_CHECK("ep_stats_f32_kernel", st);
-    ep_decide_kernel<AmpFromF64><<<(unsigned)((n_utt + kEpDecideWarps - 1) / kEpDecideWarps), 32 * kEpDecideWarps, 0, st>>>(p);
-    LAUNCH_CHECK("ep_decide_kernel<f64>", st);
-    return DSPFE_OK;
+    return endpoint_device(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, d_amp, d_zcr, d_frame_off, max_frames, stream);
 }
 
 int dspfe_endpoint_robust(dspfe_endpoint_plan* pl, const int16_t* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                           int32_t* d_lr, void* stream) {
-    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (pl->frame_len > kEpGateMaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "robust endpoint frames longer than 1536 samples are not built");
-    // frame statistics exactly as the basic path (its own decision is discarded), then the gated rule
-    int rc = dspfe_endpoint(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, nullptr, nullptr, nullptr, 0, stream);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int64_t frames_bound = dspfe_endpoint_frames_bound(pl, total_samples, n_utt);
-    EpParams p;
-    p.pcm = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off.get(); p.block_off = pl->block_off.get(); p.blk = pl->blk.get();
-    p.asum = pl->asum.get(); p.zcr = pl->zcr.get(); p.lr = d_lr; p.max_blocks = 0; p.max_frames = frames_bound; p.rule = pl->rule;
-    p.order = pl->order.get();
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<int16_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<int16_t>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    ep_decide_robust_kernel<int16_t><<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
-    LAUNCH_CHECK("ep_decide_robust_kernel", st);
-    return DSPFE_OK;
+    return endpoint_device(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, nullptr, nullptr, nullptr, 0, stream, true);
 }
 
 int dspfe_endpoint_robust_f32(dspfe_endpoint_plan* pl, const float* d_pcm, int64_t total_samples, const int64_t* d_offsets, int32_t n_utt,
                               int32_t* d_lr, void* stream) {
-    if (!pl || !d_offsets || !d_lr || n_utt < 0 || total_samples < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (pl->frame_len > kEpGateMaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "robust endpoint frames longer than 1536 samples are not built");
-    if (n_utt == 0) return DSPFE_OK;
-    // K2f's frame statistics exactly as the basic float path (its own decision is discarded), then the gated rule
-    int rc = dspfe_endpoint_f32(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, nullptr, nullptr, nullptr, 0, stream);
-    if (rc) return rc;
-    cudaStream_t st = (cudaStream_t)stream;
-    EpParams p;
-    std::memset(&p, 0, sizeof(p));
-    p.pcm_f32 = d_pcm; p.offsets = d_offsets; p.n_utt = n_utt; p.frame_len = pl->frame_len; p.frame_step = pl->frame_step;
-    p.q = pl->q; p.rem = pl->rem; p.frame_off = pl->frame_off.get(); p.amp = pl->amp.get(); p.zcr = pl->zcr.get(); p.lr = d_lr;
-    p.max_frames = dspfe_endpoint_frames_bound(pl, total_samples, n_utt); p.rule = pl->rule; p.order = pl->order.get();
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, kEpRobustSmem));
-    CUDA_TRY(cudaFuncSetAttribute(ep_decide_robust_kernel<float>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    ep_decide_robust_kernel<float><<<(unsigned)n_utt, 32 * kEpRobustWarps, kEpRobustSmem, st>>>(p);
-    LAUNCH_CHECK("ep_decide_robust_kernel<f32>", st);
-    return DSPFE_OK;
+    return endpoint_device(pl, d_pcm, total_samples, d_offsets, n_utt, d_lr, nullptr, nullptr, nullptr, 0, stream, true);
 }
-
-int dspfe_endpoint_robust_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr) {
-    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    // stage through the basic host path's buffers (it leaves pcm / offsets on the device), then re-decide with the gate
-    int rc = dspfe_endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, nullptr, nullptr, nullptr);
-    if (rc) return rc;
-    const int64_t total = h_offsets[n_utt] - h_offsets[0];
-    const cudaStream_t st = pl->stream.get();
-    rc = dspfe_endpoint_robust(pl, reinterpret_cast<const int16_t*>(pl->d_pcm.get()), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return DSPFE_OK;
-}
-
-}  // extern "C"
-
-namespace {
-
-// stages a host batch on the plan's stream: the samples into d_pcm, the offsets relative to the first into d_off; *total = the
-// sample count, h_frame_off (optional) = the frame prefix sums
-template <class T>
-int stage_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int64_t* h_frame_off, int64_t* total_out,
-               int64_t* frames_out) {
-    const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
-    if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-    CUDA_TRY(pl->stream.ensure());
-    int rc = pl->d_pcm.reserve((total + 8) * (int64_t)sizeof(T));
-    if (!rc) rc = pl->d_off.reserve(n_utt + 1);
-    if (!rc) rc = pl->d_lr.reserve((int64_t)n_utt * 2);
-    if (rc) return rc;
-    std::vector<int64_t> rel(n_utt + 1);
-    int64_t frames = 0;
-    for (int32_t u = 0; u <= n_utt; ++u) {
-        rel[u] = h_offsets[u] - base;
-        if (u < n_utt) {
-            if (h_frame_off) h_frame_off[u] = frames;
-            frames += num_frames(h_offsets[u + 1] - h_offsets[u], pl->frame_len, pl->frame_step);
-        }
-    }
-    if (h_frame_off) h_frame_off[n_utt] = frames;
-    cudaStream_t st = pl->stream.get();
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), h_pcm + base, total * sizeof(T), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    *total_out = total;
-    if (frames_out) *frames_out = frames;
-    return DSPFE_OK;
-}
-
-// the host-buffer path of either sample type: int16 samples give sum|x| per frame (Stat = int32_t), float32 samples the
-// float64 amplitude (Stat = double)
-template <class T, class Stat>
-int endpoint_host(dspfe_endpoint_plan* pl, const T* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
-                  Stat* h_stat, int32_t* h_zcr, int64_t* h_frame_off) {
-    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (n_utt == 0) return DSPFE_OK;
-    int64_t total = 0, frames = 0;
-    int rc = stage_host(pl, h_pcm, h_offsets, n_utt, h_frame_off, &total, &frames);
-    if (rc) return rc;
-    cudaStream_t st = pl->stream.get();
-    const T* d_pcm = reinterpret_cast<const T*>(pl->d_pcm.get());
-    if constexpr (sizeof(T) == 2) rc = dspfe_endpoint(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
-    else rc = dspfe_endpoint_f32(pl, d_pcm, total, pl->d_off.get(), n_utt, pl->d_lr.get(), nullptr, nullptr, nullptr, 0, st);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    if (h_stat) CUDA_TRY(cudaMemcpyAsync(h_stat, sizeof(T) == 2 ? (void*)pl->asum.get() : (void*)pl->amp.get(), frames * sizeof(Stat), cudaMemcpyDeviceToHost, st));
-    if (h_zcr) CUDA_TRY(cudaMemcpyAsync(h_zcr, pl->zcr.get(), frames * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return DSPFE_OK;
-}
-
-}  // namespace
-
-extern "C" {
 
 int dspfe_endpoint_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr,
                         int32_t* h_asum, int32_t* h_zcr, int64_t* h_frame_off) {
@@ -351,20 +291,12 @@ int dspfe_endpoint_host_f32(dspfe_endpoint_plan* pl, const float* h_pcm, const i
     return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, h_amp, h_zcr, h_frame_off);
 }
 
+int dspfe_endpoint_robust_host(dspfe_endpoint_plan* pl, const int16_t* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr) {
+    return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, nullptr, nullptr, nullptr, true);
+}
+
 int dspfe_endpoint_robust_host_f32(dspfe_endpoint_plan* pl, const float* h_pcm, const int64_t* h_offsets, int32_t n_utt, int32_t* h_lr) {
-    if (!pl || !h_offsets || !h_lr || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
-    if (pl->frame_len > kEpGateMaxLen) return fail(DSPFE_ERR_UNSUPPORTED, "robust endpoint frames longer than 1536 samples are not built");
-    if (n_utt == 0) return DSPFE_OK;
-    // the batch is staged once; the device form computes the frame statistics once and then runs the gated rule
-    int64_t total = 0;
-    int rc = stage_host(pl, h_pcm, h_offsets, n_utt, nullptr, &total, nullptr);
-    if (rc) return rc;
-    const cudaStream_t st = pl->stream.get();
-    rc = dspfe_endpoint_robust_f32(pl, reinterpret_cast<const float*>(pl->d_pcm.get()), total, pl->d_off.get(), n_utt, pl->d_lr.get(), st);
-    if (rc) return rc;
-    CUDA_TRY(cudaMemcpyAsync(h_lr, pl->d_lr.get(), (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    return DSPFE_OK;
+    return endpoint_host(pl, h_pcm, h_offsets, n_utt, h_lr, nullptr, nullptr, nullptr, true);
 }
 
 }  // extern "C"

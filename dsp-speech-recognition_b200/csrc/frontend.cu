@@ -238,12 +238,11 @@ template <class T>
 int frontend_device(dspfe_frontend_plan* pl, const T* d_pcm, const int64_t* d_offsets, const int64_t* h_off, int32_t n_utt,
                     const dspfe_frontend_out* o, int64_t* totals, void* stream) {
     constexpr int64_t kAlign = FeSamples<T>::kAlign;
-    if (!pl || !d_offsets || !h_off || !o || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     if (totals) totals[0] = totals[1] = totals[2] = 0;
+    const int64_t total_samples = h_off && n_utt > 0 ? h_off[n_utt] - h_off[0] : 0;
+    if (int rc = check_batch(pl && d_offsets && h_off && o, n_utt, total_samples, d_pcm)) return rc;
+    if (int rc = check_host_batch(true, h_off, n_utt)) return rc;
     if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && h_off[n_utt] > h_off[0]) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
-    for (int32_t u = 0; u < n_utt; ++u) if (h_off[u + 1] < h_off[u]) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
     cudaStream_t st = (cudaStream_t)stream;
     int64_t base[3] = {0, 0, 0};
     for (int32_t u0 = 0; u0 < n_utt;) {
@@ -284,11 +283,10 @@ template <class T>
 int frontend_host(dspfe_frontend_plan* pl, const T* h_pcm, const int64_t* h_off, int32_t n_utt, const dspfe_frontend_out* o,
                   int64_t* totals) {
     constexpr int64_t kAlign = FeSamples<T>::kAlign;
-    if (!pl || !h_off || !o || n_utt < 0) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
     if (totals) totals[0] = totals[1] = totals[2] = 0;
+    if (int rc = check_host_batch(pl && o, h_off, n_utt)) return rc;
     if (n_utt == 0) return DSPFE_OK;
     if (!h_pcm && h_off[n_utt] > h_off[0]) return fail(DSPFE_ERR_INVALID_ARG, "h_pcm is null");
-    for (int32_t u = 0; u < n_utt; ++u) if (h_off[u + 1] < h_off[u]) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
     CUDA_TRY(pl->s_copy.ensure());
     for (auto& ln : pl->lanes) {
         if (!ln.ep) { int rc = create_lane(ln, pl->prm); if (rc) return rc; }

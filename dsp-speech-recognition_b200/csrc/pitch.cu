@@ -219,16 +219,14 @@ __global__ void center_clip_kernel(const float* in, int64_t n_rows, int len, int
 struct dspfe_pitch_plan {
     dspfe_pitch_params prm;
     PitchParams base;          // scalars + table pointers; per-call pointers filled in launch
-    Stream stream;             // host path
+    HostBatch host;            // host-path staging
+    DeviceArray<int32_t> d_trim; DeviceArray<double> d_feat;
     DeviceArray<float2> d_tab;
     // workspaces
     DeviceArray<int64_t> seg_start; DeviceArray<int32_t> seg_len, ds_len; DeviceArray<int64_t> frame_off, slot_off;
     DeviceArray<int32_t> order;
     DeviceArray<float2> clip; DeviceArray<int4> run_desc; DeviceArray<float> rows; DeviceArray<double> frame_amp, pitch;
     DeviceArray<int32_t> lag; DeviceArray<double> scratch;
-    // host-path staging
-    DeviceArray<unsigned char> d_pcm;
-    DeviceArray<int64_t> d_off; DeviceArray<int32_t> d_trim; DeviceArray<double> d_feat;
 };
 
 namespace {
@@ -328,11 +326,8 @@ int64_t dspfe_pitch_num_frames(const dspfe_pitch_plan* pl, int64_t n_samples) {
 int dspfe_pitch(dspfe_pitch_plan* pl, const void* d_pcm, int32_t sample_dtype, int64_t total_samples, const int64_t* d_offsets,
                 const int32_t* d_trim, int32_t n_utt, double* d_pitch, int32_t* d_lag, double* d_feat, float* d_rows,
                 int64_t* d_frame_off, int64_t max_frames, void* stream) {
-    if (!pl || !d_offsets || n_utt < 0 || total_samples < 0 || (sample_dtype != 0 && sample_dtype != 1))
-        return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (int rc = check_batch(pl && d_offsets && (sample_dtype == 0 || sample_dtype == 1), n_utt, total_samples, d_pcm)) return rc;
     if (n_utt == 0) return DSPFE_OK;
-    if (!d_pcm && total_samples > 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm is null");
-    if (((uintptr_t)d_pcm & 15) != 0) return fail(DSPFE_ERR_INVALID_ARG, "d_pcm must be 16-byte aligned");
     const int64_t bound = dspfe_pitch_frames_bound(pl, total_samples, n_utt);
     if ((d_pitch || d_lag || d_rows) && max_frames < bound) return fail(DSPFE_ERR_INVALID_ARG, "max_frames is below dspfe_pitch_frames_bound()");
     if (d_feat && pl->base.mode != 0) return fail(DSPFE_ERR_UNSUPPORTED, "pitch_feature is defined on the cepstrum pitch (pitch.py:33)");
@@ -377,43 +372,24 @@ int dspfe_pitch(dspfe_pitch_plan* pl, const void* d_pcm, int32_t sample_dtype, i
 
 int dspfe_pitch_host(dspfe_pitch_plan* pl, const void* h_pcm, int32_t sample_dtype, const int64_t* h_offsets, const int32_t* h_trim,
                      int32_t n_utt, double* h_pitch, int32_t* h_lag, double* h_feat, int64_t* h_frame_off) {
-    if (!pl || !h_offsets || n_utt < 0 || (sample_dtype != 0 && sample_dtype != 1)) return fail(DSPFE_ERR_INVALID_ARG, "bad argument");
+    if (int rc = check_host_batch(pl && (sample_dtype == 0 || sample_dtype == 1), h_offsets, n_utt)) return rc;
     if (n_utt == 0) return DSPFE_OK;
-    const int esz = sample_dtype ? 4 : 2;
-    const int64_t base = h_offsets[0], total = h_offsets[n_utt] - base;
-    if (total < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-    CUDA_TRY(pl->stream.ensure());
-    int rc = pl->d_pcm.reserve((total + 8) * esz);
-    if (!rc) rc = pl->d_off.reserve(n_utt + 1);
-    if (!rc) rc = pl->d_trim.reserve((int64_t)n_utt * 2);
+    int rc = pl->d_trim.reserve((int64_t)n_utt * 2);
     if (!rc) rc = pl->d_feat.reserve((int64_t)n_utt * 5);
     if (rc) return rc;
-    std::vector<int64_t> rel(n_utt + 1);
-    int64_t frames = 0;
-    for (int32_t u = 0; u <= n_utt; ++u) {
-        rel[u] = h_offsets[u] - base;
-        if (u < n_utt) {
-            int64_t len = h_offsets[u + 1] - h_offsets[u];
-            if (len < 0) return fail(DSPFE_ERR_INVALID_ARG, "offsets must be non-decreasing");
-            if (h_trim) {
-                int64_t l = h_trim[2 * u], r = h_trim[2 * u + 1];
-                if (l < 0) l = 0; if (r < 0) r = 0;
-                if (l > len) l = len; if (r > len) r = len;
-                len = r > l ? r - l : 0;
-            }
-            if (h_frame_off) h_frame_off[u] = frames;
-            frames += dspfe_pitch_num_frames(pl, len);
-        }
-    }
-    if (h_frame_off) h_frame_off[n_utt] = frames;
-    cudaStream_t st = pl->stream.get();
-    if (total > 0) CUDA_TRY(cudaMemcpyAsync(pl->d_pcm.get(), (const char*)h_pcm + base * esz, total * esz, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemcpyAsync(pl->d_off.get(), rel.data(), (n_utt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+    auto frames_of = [&](int32_t u, int64_t len) {
+        if (h_trim) { long long l = h_trim[2 * u]; len = trim_slice(len, l, h_trim[2 * u + 1]); }
+        return dspfe_pitch_num_frames(pl, len);
+    };
+    int64_t total = 0, frames = 0;
+    rc = pl->host.stage(h_pcm, sample_dtype ? 4 : 2, h_offsets, n_utt, frames_of, h_frame_off, &total, &frames);
+    if (rc) return rc;
+    const cudaStream_t st = pl->host.stream();
     if (h_trim) CUDA_TRY(cudaMemcpyAsync(pl->d_trim.get(), h_trim, (int64_t)n_utt * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     const int64_t bound = dspfe_pitch_frames_bound(pl, total, n_utt);
     rc = ensure(pl, n_utt, bound);   // size the workspaces first: their pointers are the outputs of the device call
     if (rc) return rc;
-    rc = dspfe_pitch(pl, pl->d_pcm.get(), sample_dtype, total, pl->d_off.get(), h_trim ? pl->d_trim.get() : nullptr, n_utt, pl->pitch.get(),
+    rc = dspfe_pitch(pl, pl->host.pcm(), sample_dtype, total, pl->host.offsets(), h_trim ? pl->d_trim.get() : nullptr, n_utt, pl->pitch.get(),
                      pl->lag.get(), h_feat ? pl->d_feat.get() : nullptr, nullptr, nullptr, bound, st);
     if (rc) return rc;
     if (h_pitch) CUDA_TRY(cudaMemcpyAsync(h_pitch, pl->pitch.get(), frames * sizeof(double), cudaMemcpyDeviceToHost, st));
