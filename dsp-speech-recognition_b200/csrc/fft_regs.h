@@ -53,11 +53,11 @@ DEVFN void dft16(cpx2 (&x)[16]) {
 
 // 512-point complex FFT of a packed frame pair, one warp, 16 complex values per lane, 512 = 16 x 2 x 16:
 //   element n = 32*n1 + 16*q + n2'  ->  lane 16*q + n2', register n1   (natural order: n = 32*register + lane)
-// radix-16 in registers over n1, radix-2 across the two half-warps (one shuffle), twiddle, a 16x16 transpose inside each
-// half-warp through shared memory, radix-16 in registers over n2'.  With the radix-2 stage in the middle the output
-// lands in the SAME layout (k = k1 + 16*kq + 32*k2' -> lane 16*kq + k1, register k2'), so one routine serves every
-// transform of the chain and all pointwise tables are in natural order.  Forward DFT sum x[n] W512^{nk}; the
-// unnormalised inverse is the same routine between two conjugations.
+// radix-16 in registers over n1, radix-2 across the two half-warps, twiddle, a 32x16 transpose over the warp through shared
+// memory, radix-16 in registers over n2'.  With the radix-2 stage in the middle the output lands in the SAME layout
+// (k = k1 + 16*kq + 32*k2' -> lane 16*kq + k1, register k2'), so one routine serves every transform of the chain and all
+// pointwise tables are in natural order.  Forward DFT sum x[n] W512^{nk}; the unnormalised inverse is the same routine
+// between two conjugations.
 DEVFN cpx2 shfl_xor_c(cpx2 a, int m) {
     cpx2 r;
     r.re.x = simt::shfl32_xor(a.re.x, m); r.re.y = simt::shfl32_xor(a.re.y, m);
@@ -65,37 +65,45 @@ DEVFN cpx2 shfl_xor_c(cpx2 a, int m) {
     return r;
 }
 
-// tws: W512^{n2' (k1 + 16 kq)} at [k1*32 + lane]; w32s: [2*k1 + q] = W32^{q k1}; scr: kWarpScr float2 owned by the warp
-// W32IMM: take W32^k1 from immediates selected by the half-warp instead of the w32s table (one shared-memory load less per
-// k1; worth it only where registers are not the constraint: the pitch frame kernels at 3 CTAs/SM)
-template <bool W32IMM = false>
-DEVFN void fft512(cpx2 (&x)[16], float2* scr, const float2* tws, const float2* w32s, int lane) {
+// The radix-2 stage exchanges half the registers: b[kq][k1] = a0[k1] + (-1)^kq W32^k1 a1[k1] needs both half-warps' a at
+// k1, so lane (q, n2') takes the butterflies of k1 = 8q + j, j < 8, and receives one value per j from lane (1 - q, n2'):
+// q = 0 keeps a0[j] and sends a0[8 + j], q = 1 keeps W32^{8+j} a1[8 + j] and sends W32^j a1[j].  Each output is the same
+// single rounding of the same two operands as a full exchange would give; q = 1 forms kp - r = -b[1] exactly and its
+// twiddle carries the sign.  Afterwards register r of lane (q, n2') holds (kq, k1) = (r >> 3, 8q + (r & 7)).
+// W32^k1 comes from immediates.  tws: [r*32 + lane] = W512^{n2' (k1 + 16 kq)} of that (kq, k1), negated for q = kq = 1
+// (fill_fft512_twiddles).
+// scr: kWarpScr float2 owned by the warp: the 32 x 16 tile, row 16 kq + k1 at a pitch of 17 float2.  Writes put a half-warp
+// on 16 consecutive float2 of one row, reads a lane on its own row at column n2: row * 17 + n2 = row + n2 (mod 16) is
+// distinct over each half-warp, so both 64-bit phases run without bank conflicts.
+DEVFN void fft512(cpx2 (&x)[16], float2* scr, const float2* tws, int lane) {
     dft16(x);                                                   // over n1 -> k1
-    const int q = lane >> 4, ll = lane & 15;
-    const float sg = q ? -1.f : 1.f;
+    const int q = lane >> 4;
+    const float kC[16] = {1.0f, 0.98078528f, 0.923879533f, 0.831469612f, 0.707106781f, 0.555570233f, 0.382683432f, 0.195090322f, 6.123234e-17f, -0.195090322f, -0.382683432f, -0.555570233f, -0.707106781f, -0.831469612f, -0.923879533f, -0.98078528f};
+    const float kS[16] = {-0.0f, -0.195090322f, -0.382683432f, -0.555570233f, -0.707106781f, -0.831469612f, -0.923879533f, -0.98078528f, -1.0f, -0.98078528f, -0.923879533f, -0.831469612f, -0.707106781f, -0.555570233f, -0.382683432f, -0.195090322f};
 #pragma unroll
-    for (int k1 = 0; k1 < 16; ++k1) {                           // b[kq] = a[q=0] + (-1)^kq W32^k1 a[q=1]
-        const float kC[16] = {1.0f, 0.98078528f, 0.923879533f, 0.831469612f, 0.707106781f, 0.555570233f, 0.382683432f, 0.195090322f, 6.123234e-17f, -0.195090322f, -0.382683432f, -0.555570233f, -0.707106781f, -0.831469612f, -0.923879533f, -0.98078528f};
-        const float kS[16] = {-0.0f, -0.195090322f, -0.382683432f, -0.555570233f, -0.707106781f, -0.831469612f, -0.923879533f, -0.98078528f, -1.0f, -0.98078528f, -0.923879533f, -0.831469612f, -0.707106781f, -0.555570233f, -0.382683432f, -0.195090322f};
-        const float2 w = W32IMM ? make_float2(q ? kC[k1] : 1.f, q ? kS[k1] : 0.f) : w32s[2 * k1 + q];
-        const cpx2 u = cmuls(x[k1], w.x, w.y);
-        const cpx2 v = shfl_xor_c(u, 16);
-        cpx2 d; d.re = f2fmas(u.re, sg, v.re); d.im = f2fmas(u.im, sg, v.im);
-        const float2 t = tws[k1 * 32 + lane];
-        x[k1] = cmuls(d, t.x, t.y);
+    for (int j = 0; j < 8; ++j) {
+        const cpx2 us = cmuls(x[j], kC[j], kS[j]), uk = cmuls(x[8 + j], kC[8 + j], kS[8 + j]);   // W32^k1 a1[k1], taken on q = 1 only
+        cpx2 snd, kp;
+        snd.re = q ? us.re : x[8 + j].re; snd.im = q ? us.im : x[8 + j].im;
+        kp.re = q ? uk.re : x[j].re; kp.im = q ? uk.im : x[j].im;
+        const cpx2 r = shfl_xor_c(snd, 16);
+        const float2 t0 = tws[j * 32 + lane], t1 = tws[(8 + j) * 32 + lane];
+        x[j] = cmuls(cadd(kp, r), t0.x, t0.y);
+        x[8 + j] = cmuls(csub(kp, r), t1.x, t1.y);
     }
-    float2* tile = scr + q * (16 * 17);                         // (k1, n2') -> (n2', k1) inside the half-warp
+    float2* wr = scr + 8 * q * 17 + (lane & 15);                // row 16 (r >> 3) + 8q + (r & 7), column n2'
+    const float2* rd = scr + lane * 17;                         // row 16 kq + k1 = lane
 #pragma unroll
-    for (int k1 = 0; k1 < 16; ++k1) tile[k1 * 17 + ll] = x[k1].re;
+    for (int r = 0; r < 16; ++r) wr[(16 * (r >> 3) + (r & 7)) * 17] = x[r].re;
     simt::warp_sync();
 #pragma unroll
-    for (int n2 = 0; n2 < 16; ++n2) x[n2].re = tile[ll * 17 + n2];
+    for (int n2 = 0; n2 < 16; ++n2) x[n2].re = rd[n2];
     simt::warp_sync();
 #pragma unroll
-    for (int k1 = 0; k1 < 16; ++k1) tile[k1 * 17 + ll] = x[k1].im;
+    for (int r = 0; r < 16; ++r) wr[(16 * (r >> 3) + (r & 7)) * 17] = x[r].im;
     simt::warp_sync();
 #pragma unroll
-    for (int n2 = 0; n2 < 16; ++n2) x[n2].im = tile[ll * 17 + n2];
+    for (int n2 = 0; n2 < 16; ++n2) x[n2].im = rd[n2];
     simt::warp_sync();
     dft16(x);                                                   // over n2' -> k2'
 }

@@ -30,12 +30,12 @@ constexpr int kLongNfft = 1536;                  // the size with the decimation
 constexpr int kLongBins = kLongNfft / 2 + 1;     // 769
 constexpr int kLongMaxNfft = 2048;
 constexpr int kLongWarps = 4;
-constexpr int kLongScr = 2 * 16 * 17;            // fft512's transpose tiles (float2)
-// float blob offsets (in floats): fft twiddles | W1536^k | window | mel tables | dct
+constexpr int kLongScr = 32 * 17;                // fft512's transpose tile (float2)
+// float blob offsets (in floats): fft twiddles | W32 (read by no kernel, as kTabW32) | W1536^k | window | mel tables | dct
 constexpr int kLtTw = 0, kLtW32 = kLtTw + 1024, kLtW1536 = kLtW32 + 64, kLtWin = kLtW1536 + 2 * kLongMaxNfft,
               kLtEdge = kLtWin + kLongMaxNfft, kLtInvUp = kLtEdge + 48, kLtInvDn = kLtInvUp + 48, kLtDct = kLtInvDn + 48,
               kLtTotal = kLtDct + 16 * 48;
-// per-warp shared memory: transpose tiles | X / power per bin | log-mel pair.  The accumulators need nfft/2 + 1 float4 slots; the
+// per-warp shared memory: transpose tile | X / power per bin | log-mel pair.  The accumulators need nfft/2 + 1 float4 slots; the
 // decimation-in-frequency path of nfft = 1536 parks 512 float2 behind 769 + 7 float2 power values, which fits the same area.
 #ifdef __CUDACC__
 #define LONG_HD __host__ __device__
@@ -115,7 +115,7 @@ DEVFN float long_sample(const MfccLongParams& p, const LongFrame& f, int n, floa
 // wsm: per-warp shared memory = scr[kLongScr] float2 | acc[kLongBins] float4 | lmel[64] float2
 // NFFT: the transform size when known at compile time (1536: the trainer's), else 0
 template <int NFFT = 0>
-DEVFN void mfcc_long_pair(const MfccLongParams& p, int64_t g0, int64_t total, unsigned char* wsm, const float2* tws, const float2* w32s) {
+DEVFN void mfcc_long_pair(const MfccLongParams& p, int64_t g0, int64_t total, unsigned char* wsm, const float2* tws, const float2* /*w32s*/) {
     const int lane = simt::tid() & 31;
     float2* scr = reinterpret_cast<float2*>(wsm);
     float4* acc = reinterpret_cast<float4*>(scr + kLongScr);
@@ -168,7 +168,7 @@ DEVFN void mfcc_long_pair(const MfccLongParams& p, int64_t g0, int64_t total, un
                 }
                 x[t].re = f2muls(v, m.x); x[t].im = f2muls(v, m.y);
             }
-            fft512(x, scr, tws, w32s, lane);
+            fft512(x, scr, tws, lane);
 #pragma unroll
             for (int t = 0; t < 16; ++t) {
                 const int q = 32 * t + lane;
@@ -191,7 +191,7 @@ DEVFN void mfcc_long_pair(const MfccLongParams& p, int64_t g0, int64_t total, un
             x[t].re = make_float2(long_sample(p, fa, n, w), long_sample(p, fb, n, w));
             x[t].im = zero2;
         }
-        fft512(x, scr, tws, w32s, lane);
+        fft512(x, scr, tws, lane);
         // X[k] += W_nfft^{r k} Z_r[k mod 512] for every bin k = j + 512 c <= nfft / 2, j = 32 t + lane (nfft >= 512);
         // X[k] = Z_0[D k] for the short transforms
 #pragma unroll

@@ -44,9 +44,10 @@ constexpr int kMinLag = 20;
 constexpr int kPeakLags = 80;       // peak_score evaluates lags 20..99 (pitch.py:232)
 constexpr int kMaxDsOut = 256;      // decimator pattern length limit
 constexpr int kPitchWarps = 4;      // warps per CTA in K4a/K5a, each carrying a pair of frames
-constexpr int kWarpScr = 2 * 16 * 17;   // two padded 16x16 transpose tiles (float2), one per half-warp
+constexpr int kWarpScr = 32 * 17;       // fft512's padded 32x16 transpose tile (float2)
 constexpr int kWarpSmemBytes = kWarpScr * 8 + 512 * 16;              // transform kernel: transpose tile | parked spectrum
-// table blob offsets, in float2
+// table blob offsets, in float2.  The W32 slot is read by no kernel since fft512 takes W32 from immediates; the frame pair
+// bodies and the emulator entry points that call them still pass a pointer to it.
 constexpr int kTabTw = 0, kTabW32 = kTabTw + 512, kTabMod = kTabW32 + 32, kTabHe = kTabMod + 512, kTabHo = kTabHe + 512,
               kTabTotal = kTabHo + 512;
 // the Bluestein tables of pitch_cep_bluestein_pair follow the blob above (filled for cepstrum frames other than 512 samples):
@@ -584,7 +585,7 @@ DEVFN void pitch_clip_run(const PitchParams& p, int64_t h0, unsigned char* wsm, 
 // wsm: per-warp shared memory = scr[kWarpScr] float2 | park[512] float4.
 template <int MODE>
 // h0: the pair's first slot (even); g0: global index of its first frame; hasB: the second frame exists
-DEVFN void pitch_fft_pair(const PitchParams& p, int64_t h0, int64_t g0, bool hasB, unsigned char* wsm, const float2* tws, const float2* w32s) {
+DEVFN void pitch_fft_pair(const PitchParams& p, int64_t h0, int64_t g0, bool hasB, unsigned char* wsm, const float2* tws, const float2* /*w32s*/) {
     const int lane = simt::tid() & 31;
     float2* scr = reinterpret_cast<float2*>(wsm);
     float4* park = reinterpret_cast<float4*>(scr + kWarpScr);
@@ -622,7 +623,7 @@ DEVFN void pitch_fft_pair(const PitchParams& p, int64_t h0, int64_t g0, bool has
 #pragma unroll
             for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
         }
-        fft512<true>(x, scr, tws, w32s, lane);
+        fft512(x, scr, tws, lane);
         if (inv) {
 #pragma unroll
             for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
@@ -722,7 +723,7 @@ DEVFN void pitch_fft_pair(const PitchParams& p, int64_t h0, int64_t g0, bool has
 // wsm: per-warp shared memory = scr[kWarpScr] float2 | park[512] float4 (as pitch_fft_pair).
 // ---------------------------------------------------------------------------------------------------------
 // h0: the pair's first slot (even); g0: global index of its first frame; hasB: the second frame exists
-DEVFN void pitch_cep_bluestein_pair(const PitchParams& p, int64_t h0, int64_t g0, bool hasB, unsigned char* wsm, const float2* tws, const float2* w32s) {
+DEVFN void pitch_cep_bluestein_pair(const PitchParams& p, int64_t h0, int64_t g0, bool hasB, unsigned char* wsm, const float2* tws, const float2* /*w32s*/) {
     const int lane = simt::tid() & 31;
     float2* scr = reinterpret_cast<float2*>(wsm);
     float4* park = reinterpret_cast<float4*>(scr + kWarpScr);
@@ -751,7 +752,7 @@ DEVFN void pitch_cep_bluestein_pair(const PitchParams& p, int64_t h0, int64_t g0
 #pragma unroll
             for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
         }
-        fft512<true>(x, scr, tws, w32s, lane);
+        fft512(x, scr, tws, lane);
         if (inv) {
 #pragma unroll
             for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
@@ -824,7 +825,8 @@ DEVFN void pitch_cep_bluestein_pair(const PitchParams& p, int64_t h0, int64_t g0
 //     |V1|^2 = |Z + Zr*|^2 / 4 and |V2|^2 = |Z - Zr*|^2 / 4; both power spectra are real and even, so the inverse transform
 //     of |V1|^2 + i |V2|^2 has r1 in its real part and r2 in its imaginary part: one forward + one inverse per quad.
 // The partner bins Zr come from the lane 32 - lane (register 15 - t) by shuffles; lane 0 holds the bins 32 t, whose partners
-// 32 (16 - t) are its own registers, fetched with a one-register look-behind so that the update can run in place.
+// 32 (16 - t) are its own registers.  So that the update can run in place, the FIR split keeps a one-register look-behind;
+// the power spectra are even, so there lane 0 copies bin 32 (16 - t), finished one step earlier, into bin 32 t.
 // wsm: per-warp shared memory = scr[kWarpScr] float2 | vpark[32 * kQuadT] float2.
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kQuadT = 10;                                            // registers that hold samples of a frame of <= 320 samples
@@ -841,15 +843,15 @@ template <int KIND>
 DEVFN void split_pairs(cpx2 (&x)[16], const float2* A, const float2* B, int lane) {
     const int src = (32 - lane) & 31;
     const bool l0 = lane == 0;
-    cpx2 saved = x[0];
+    cpx2 saved = x[0];                                  // KIND 0: lane 0's x[16 - t] before step t - 1 overwrote it
 #pragma unroll
     for (int t = 0; t < 8; ++t) {
         const int a = t, b = 15 - t;
         cpx2 sa = shfl_c(x[b], src), sb = shfl_c(x[a], src);
-        if (l0) { sa = saved; sb = x[a + 1]; }
-        saved = x[b];
         const cpx2 za = x[a], zb = x[b];
+        if (l0) { sa = KIND == 0 ? saved : za; sb = x[a + 1]; }   // (KIND 1 uses this sa at t = 0 only: bin 0 is its own partner)
         if (KIND == 0) {
+            saved = zb;
             const float2 Aa = ldg(A + 32 * a + lane), Ba = ldg(B + 32 * a + lane), Ab = ldg(A + 32 * b + lane), Bb = ldg(B + 32 * b + lane);
             // z A + conj(s) B:  re = z.re A.x - z.im A.y + s.re B.x + s.im B.y;  im = z.re A.y + z.im A.x + s.re B.y - s.im B.x
             x[a].re = f2fmas(sa.im, Ba.y, f2fmas(sa.re, Ba.x, f2fmas(za.im, -Aa.y, f2muls(za.re, Aa.x))));
@@ -861,11 +863,12 @@ DEVFN void split_pairs(cpx2 (&x)[16], const float2* A, const float2* B, int lane
             const float2 pb_r = f2add(zb.re, sb.re), pb_i = f2sub(zb.im, sb.im), mb_r = f2sub(zb.re, sb.re), mb_i = f2add(zb.im, sb.im);
             x[a].re = f2muls(f2fma(pa_i, pa_i, f2mul(pa_r, pa_r)), 0.25f); x[a].im = f2muls(f2fma(ma_i, ma_i, f2mul(ma_r, ma_r)), 0.25f);
             x[b].re = f2muls(f2fma(pb_i, pb_i, f2mul(pb_r, pb_r)), 0.25f); x[b].im = f2muls(f2fma(mb_i, mb_i, f2mul(mb_r, mb_r)), 0.25f);
+            if (l0 && t > 0) x[a] = x[16 - t];             // |.|^2 of bin 32 t = that of bin 32 (16 - t), set at step t - 1
         }
     }
 }
 // h0: the quad's first slot (a multiple of 4); g0: global index of its first frame; nvalid: how many of its frames exist (1..4)
-DEVFN void pitch_acr_quad(const PitchParams& p, int64_t h0, int64_t g0, int nvalid, unsigned char* wsm, const float2* tws, const float2* w32s) {
+DEVFN void pitch_acr_quad(const PitchParams& p, int64_t h0, int64_t g0, int nvalid, unsigned char* wsm, const float2* tws, const float2* /*w32s*/) {
     const int lane = simt::tid() & 31;
     float2* scr = reinterpret_cast<float2*>(wsm);
     float2* vpark = scr + kWarpScr;
@@ -898,7 +901,7 @@ DEVFN void pitch_acr_quad(const PitchParams& p, int64_t h0, int64_t g0, int nval
 #pragma unroll
             for (int t = 0; t < 16; ++t) x[t].im = f2neg(x[t].im);
         }
-        fft512<true>(x, scr, tws, w32s, lane);
+        fft512(x, scr, tws, lane);
         if (st == 0 || st == 2) {
             split_pairs<0>(x, tabA, tabB, lane);
         } else if (st == 1 || st == 3) {                     // v = |y| on the frame, zero beyond it (the conjugation does not change |.|)
@@ -938,22 +941,23 @@ DEVFN void pitch_acr_quad(const PitchParams& p, int64_t h0, int64_t g0, int nval
             }
         } else if (st == 4) {
             split_pairs<1>(x, tabA, tabB, lane);
-        } else {                                             // st == 5: r[n] / 512, unbiased normalisation (sigproc.py:48-53), rows
-            const float inv512 = 1.0f / 512.0f;
-            float* row = p.rows + g0 * p.row_len;
-            const int RL = p.row_len;
-            const bool f1 = nvalid > 1, f2 = nvalid > 2, f3 = nvalid > 3;
+        }
+    }
+    // r[n] / 512, unbiased normalisation (sigproc.py:48-53), rows (after the loop: the loop-invariant divisions would otherwise
+    // be hoisted out of it and held in registers through every stage)
+    const float inv512 = 1.0f / 512.0f;
+    float* row = p.rows + g0 * p.row_len;
+    const int RL = p.row_len;
+    const bool f1 = nvalid > 1, f2 = nvalid > 2, f3 = nvalid > 3;
 #pragma unroll
-            for (int t = 0; t < 7; ++t) {
-                const int n = 32 * t + lane, j = n - kMinLag;
-                if (j >= 0 && j < RL) {
-                    const float sc = (n < L) ? inv512 / (float)(L - n) : NAN;
-                    row[j] = x[t].re.x * sc;
-                    if (f1) row[RL + j] = x[t].re.y * sc;
-                    if (f2) row[2 * RL + j] = -x[t].im.x * unscale.x * sc;   // the inverse is conj . forward . conj: its imaginary part is
-                    if (f3) row[3 * RL + j] = -x[t].im.y * unscale.y * sc;   // minus the imaginary part left in the registers
-                }
-            }
+    for (int t = 0; t < 7; ++t) {
+        const int n = 32 * t + lane, j = n - kMinLag;
+        if (j >= 0 && j < RL) {
+            const float sc = (n < L) ? inv512 / (float)(L - n) : NAN;
+            row[j] = x[t].re.x * sc;
+            if (f1) row[RL + j] = x[t].re.y * sc;
+            if (f2) row[2 * RL + j] = -x[t].im.x * unscale.x * sc;   // the inverse is conj . forward . conj: its imaginary part is
+            if (f3) row[3 * RL + j] = -x[t].im.y * unscale.y * sc;   // minus the imaginary part left in the registers
         }
     }
 }

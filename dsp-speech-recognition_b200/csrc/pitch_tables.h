@@ -26,15 +26,18 @@ inline void fir_taps(int N, double rate, double lo, double hi, bool hamming, std
     }
 }
 
-// twiddles of fft512 (fft_regs.h): tws[k1*32 + lane] = W512^{n2' (k1 + 16 kq)} with lane = 16 kq + n2', w32[2*k1 + q] = W32^{q k1}
+// twiddles of fft512 (fft_regs.h): tws[r*32 + lane] = W512^{n2' (k1 + 16 kq)} for register r of lane 16 q + n2' after the
+// radix-2 stage, (kq, k1) = (r >> 3, 8 q + (r & 7)), negated for q = kq = 1; w32[2*k1 + q] = W32^{q k1}
 inline void fill_fft512_twiddles(float2* tws, float2* w32) {
     const double kPi = 3.14159265358979323846;
-    for (int k1 = 0; k1 < 16; ++k1) {
+    for (int r = 0; r < 16; ++r)
         for (int lane = 0; lane < 32; ++lane) {
-            const int kq = lane >> 4, n2 = lane & 15;
+            const int q = lane >> 4, n2 = lane & 15, kq = r >> 3, k1 = 8 * q + (r & 7);
             const double a = -2 * kPi * (double)(n2 * (k1 + 16 * kq)) / 512.0;
-            tws[k1 * 32 + lane] = make_float2((float)cos(a), (float)sin(a));
+            const float sg = q && kq ? -1.f : 1.f;
+            tws[r * 32 + lane] = make_float2(sg * (float)cos(a), sg * (float)sin(a));
         }
+    for (int k1 = 0; k1 < 16; ++k1) {
         w32[2 * k1] = make_float2(1.f, 0.f);
         w32[2 * k1 + 1] = make_float2((float)cos(-2 * kPi * k1 / 32.0), (float)sin(-2 * kPi * k1 / 32.0));
     }
